@@ -26,6 +26,9 @@ prefill + 36 frame steps + windowed codec decode to PCM.
 
 Multi-GPU: request-parallel replicas (SURVEY.md §8e) — one process per GPU (torchrun), each with its own shard of utterances (weak
 scaling on the headline line); NCCL carries only the barrier, the max-over-ranks time, the sums, and the result gather.
+
+`--dump-outputs DIR` writes what the last timed step returned to its caller as DIR/*.npy (see dump_outputs).  Every step's requests
+are drawn from its index, so the same arguments give the same inputs on every run and two builds can be compared output for output.
 """
 from __future__ import annotations
 
@@ -112,6 +115,24 @@ def peaks():
         j = json.load(open(p))
         return j.get("hbm_gbs", 6650.0), j.get("bf16_tflops_sustained", 1400.0), "measured"
     return 6650.0, 1590.0, "fallback"
+
+
+def dump_outputs(out_dir, pcm, frames, n_samples, suffix="", budget=63 << 20):
+    """--dump-outputs: what the last timed q3tts_generate_pcm_batch call returned -- every utterance's PCM (float32, zero-padded to
+    `n_samples`), its length in samples and its frame count -- as .npy files, so two builds can be compared output for output on
+    identical inputs.  Above `budget` bytes of PCM (64 MB in all with the small per-utterance arrays) a fixed seeded sample of
+    utterances is written; `utterance.npy` names the rows."""
+    rows = np.arange(len(pcm))
+    keep = max(1, budget // (4 * max(1, n_samples)))
+    if keep < len(pcm):
+        rows = np.sort(np.random.default_rng(0).choice(len(pcm), keep, replace=False))
+    block = np.zeros((len(rows), n_samples), dtype=np.float32)
+    for j, i in enumerate(rows):
+        block[j, :pcm[i].size] = pcm[i]
+    os.makedirs(out_dir, exist_ok=True)
+    for name, arr in (("pcm", block[:, :budget // 4]), ("pcm_samples", [pcm[i].size for i in rows]), ("frames", [frames[i] for i in rows]),
+                      ("utterance", rows)):
+        np.save(os.path.join(out_dir, f"{name}{suffix}.npy"), np.asarray(arr, dtype=np.float32 if name == "pcm" else np.float64))
 
 
 def workload_config(a, world):
@@ -346,7 +367,13 @@ def main():
     ap.add_argument("--config4-clips", type=int, default=128)
     ap.add_argument("--packed-gemm", type=int, default=0, choices=[0, 1, 2],
                     help="q3tts_options.packed_gemm of the measured handle: 1 = packed weights dequantised inside the tcgen05 GEMM, 2 / 0 = fp16 operand copies")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one returned (PCM, samples and frames per utterance) as DIR/<name>.npy")
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the CUDA engine (--impl b200)")
 
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -421,7 +448,8 @@ def main():
         samples = int(sum(p.size for p in pcm))
         return {"wall": wall, "dev": (tm.talker_ms + tm.decode_ms) * 1e-3, "talker": tm.talker_ms * 1e-3, "decode": tm.decode_ms * 1e-3,
                 "samples": samples, "frames": int(tm.frames), "launches": int(tm.kernel_launches), "h2d": int(tm.h2d_bytes), "d2h": int(tm.d2h_bytes),
-                "codec_flops": int(tm.codec_flops), "bytes_frame": int(tm.weight_bytes_per_frame), "prefill": tm.prefill_ms * 1e-3}
+                "codec_flops": int(tm.codec_flops), "bytes_frame": int(tm.weight_bytes_per_frame), "prefill": tm.prefill_ms * 1e-3,
+                "out": (pcm, frames)}
 
     # nvidia-smi is started BEFORE the warm-up steps: its start-up (NVML init takes driver locks for tens to hundreds of ms on a
     # box without persistence mode) would otherwise stall kernel submission inside the first timed step; it keeps sampling
@@ -442,6 +470,8 @@ def main():
     t_total = time.perf_counter() - t_begin
     clocks = sampler.snapshot()
     n_clock_rows = len(sampler.rows)
+    if a.dump_outputs:  # before the extra blocks below reuse out_bufs
+        dump_outputs(a.dump_outputs, *res[-1]["out"], a.frames * up, f"_rank{rank}" if world > 1 else "")
 
     dev = sum(r["dev"] for r in res)
     wall = sum(r["wall"] for r in res)

@@ -3,11 +3,10 @@
 Tolerances (BASELINE.json north_star): dequantised weights bit-exact; teacher-forced logits max-abs <= 1e-2;
 greedy ids identical wherever the oracle's top-2 margin exceeds 2e-2 (a first divergence is accepted only at a
 near-tie, and is reported)."""
-import os
 import numpy as np
 import pytest
 
-from conftest import ROOT, TEXT_IDS, ckpt
+from conftest import TEXT_IDS, ckpt
 
 pytestmark = pytest.mark.gpu
 
@@ -636,44 +635,6 @@ def test_fp16_kv_rings_long_window(tiny8, oracles, monkeypatch):
     d0 = np.abs(l16["code0_logits"] - l32["code0_logits"]).max()
     print(f"[tiny8, 230 steps] fp16 KV rings: max-abs logit error vs oracle code0 {e0:.3e}, code predictor {ec:.3e}; fp16 vs fp32 rings {d0:.3e}")
     assert e0 <= LOGIT_TOL and ec <= LOGIT_TOL and d0 <= 5e-3
-
-
-def test_trapped_kernel_surfaces_as_cuda_error_and_poisons_the_handle(tiny8):
-    """VERDICT r1 item 11: a wait on an mbarrier nobody arrives at (a broken TMA / tcgen05 protocol) must end as a trapped kernel and
-    Q3TTS_ERR_CUDA on the host -- never a hung GPU -- and the handle must fail deterministically afterwards (a kernel fault is sticky for
-    the process's CUDA context, so this runs in its own process)."""
-    import subprocess
-    import sys
-    import textwrap
-
-    code = textwrap.dedent(f"""
-        import sys, time
-        sys.path.insert(0, {os.path.join(ROOT, "mlx-swift-qwen3-tts_b200")!r})
-        import numpy as np
-        import qwen3tts_b200 as q
-        from qwen3tts_b200 import _abi as A
-        eng = q.Engine({tiny8!r}, max_frames=64)
-        req = q.GenRequest(text_ids={TEXT_IDS!r}, temperature=0.0, max_tokens=4)
-        assert len(eng.generate_codes(req)) > 0              # healthy before
-        t0 = time.time()
-        st = A.lib().q3tts_debug_trap(eng._h)
-        dt = time.time() - t0
-        msg1 = A.lib().q3tts_last_error(eng._h).decode()
-        assert st == A.ERR_CUDA, st
-        assert "poisoned" in msg1, msg1
-        assert dt < 30.0, dt                                 # bounded: 2^22 polls, not a hang
-        for _ in range(2):                                   # deterministic afterwards: same status, same text
-            try:
-                eng.generate_codes(req)
-                raise SystemExit("a poisoned handle accepted work")
-            except q.Q3Error as e:
-                assert e.status == A.ERR_CUDA and e.message == msg1, (e.status, e.message)
-        eng.close()                                          # destroy still works
-        print("TRAP-OK %.3f s" % dt)
-    """)
-    r = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True, timeout=300)
-    assert r.returncode == 0 and "TRAP-OK" in r.stdout, r.stdout + r.stderr
-    print(r.stdout.strip())
 
 
 def test_two_handles_served_from_two_threads_equal_one_handle(tiny8):
