@@ -58,7 +58,8 @@ typedef struct q3tts_options {
   int32_t device;           /* CUDA ordinal */
   void* cuda_stream;        /* cudaStream_t to run on, or NULL: the library creates its own */
   int32_t max_batch;        /* concurrent utterances the handle can hold (1 = the reference's behaviour) */
-  int32_t kv_capacity;      /* KV ring capacity per utterance in positions (>= prefill + 16, >= 208); 0 = 512 */
+  int32_t kv_capacity;      /* KV ring capacity per utterance in positions (>= prefill + 16); 0 = 512; values below 208 (a
+                               192-key window + 16) are raised to 208; above 512 a 1-2 slot handle runs the CUDA-graph step */
   int32_t max_frames;       /* per-utterance frame buffer (>= max_tokens); 0 = 2400 (Qwen3TTSPipeline.swift:42) */
   int32_t use_cuda_graph;   /* 1: frame step replayed as a CUDA graph (the reference's analogue is MLX compile{}) */
   int32_t load_codec;       /* 0: talker only */
@@ -309,6 +310,20 @@ q3tts_status q3tts_conv_probe(int32_t device, const float* x, int32_t B, int32_t
                               int32_t N, int32_t ntap, int32_t dil, int32_t act, int32_t swiglu, const float* res,
                               const float* scale, const float* snake_ea, const float* snake_ieb, int32_t snake_ch,
                               int32_t use_tensor_cores, float* y32, float* y16);
+
+/* One talker attention launch as the engine issues it (head_dim 128, scale 1/sqrt(128)), on host buffers:
+ * kernel: 0 = rope_attention (decode: one row per slot, appends that row's k/v), 1 = qk_norm_rope_append + attention (prefill),
+ *         2 = cp_pass0_attention (rows 2s, 2s+1 at positions 0, 1; fp16 out, fp32 cache).
+ * qkv [m][(heads + 2*kv_heads)*128]; row_slot / row_pos [m]; win_start [n_slots] or NULL (= 0);
+ * k_ring / v_ring [n_slots][kv_heads][capacity][128] fp32, in/out (rounded to fp16 on upload when kv_f16, widened back);
+ * out [m][heads*128] fp32 (fp16 values widened when out_f16).
+ * Everything is validated before the launch: heads / kv_heads in {1, 2, 4}, slots in range, 0 <= win_start <= pos,
+ * pos - win_start + 1 <= capacity, one row per slot for kernel 0, rows (2s, 2s+1) of slot s at positions (0, 1) with an fp32
+ * cache and fp16 output for kernel 2.  Anything else returns Q3TTS_ERR_INVALID_ARG without touching the device. */
+q3tts_status q3tts_attention_probe(int32_t device, int32_t kernel, int32_t kv_f16, int32_t out_f16, const float* qkv, int32_t m,
+                                   int32_t heads, int32_t kv_heads, const float* q_norm, const float* k_norm, float eps,
+                                   const float* inv_freq, const int32_t* row_slot, const int32_t* row_pos, const int32_t* win_start,
+                                   int32_t n_slots, int32_t capacity, float* k_ring, float* v_ring, float* out);
 
 /* ------------------------------------------------------------------------------------------------------
  * measurement hook (bench.py roofline): runs the dequant-fused linear launches of ONE talker decode step

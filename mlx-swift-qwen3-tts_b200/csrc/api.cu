@@ -1287,6 +1287,116 @@ q3tts_status q3tts_conv_probe(int32_t device, const float* x, int32_t B, int32_t
   }
 }
 
+q3tts_status q3tts_attention_probe(int32_t device, int32_t kernel, int32_t kv_f16, int32_t out_f16, const float* qkv, int32_t m,
+                                   int32_t heads, int32_t kv_heads, const float* q_norm, const float* k_norm, float eps,
+                                   const float* inv_freq, const int32_t* row_slot, const int32_t* row_pos, const int32_t* win_start,
+                                   int32_t n_slots, int32_t capacity, float* k_ring, float* v_ring, float* out) {
+  std::vector<void*> allocs;
+  try {
+    // every index a kernel derives from these arguments is checked here, so no input can make a launch read or write outside
+    // its buffers
+    Q3_CHECK(qkv && q_norm && k_norm && inv_freq && row_slot && row_pos && k_ring && v_ring && out, Q3TTS_ERR_INVALID_ARG, "NULL argument");
+    Q3_CHECK(kernel >= 0 && kernel <= 2, Q3TTS_ERR_INVALID_ARG, "kernel must be 0, 1 or 2");
+    Q3_CHECK(m > 0 && n_slots > 0 && capacity > 0 && kv_heads > 0 && heads > 0 && heads % kv_heads == 0, Q3TTS_ERR_INVALID_ARG,
+             "bad sizes (m %d, n_slots %d, capacity %d, heads %d, kv_heads %d)", m, n_slots, capacity, heads, kv_heads);
+    const int G = heads / kv_heads;
+    Q3_CHECK(G == 1 || G == 2 || G == 4, Q3TTS_ERR_INVALID_ARG, "GQA group %d not in {1, 2, 4}", G);
+    const size_t ring_elems = (size_t)n_slots * kv_heads * capacity * 128;
+    Q3_CHECK(ring_elems < ((size_t)1 << 31) && (size_t)m * (heads + 2 * kv_heads) * 128 < ((size_t)1 << 31), Q3TTS_ERR_INVALID_ARG, "buffers too large");
+    std::vector<int> rows_of_slot(n_slots, 0);
+    for (int r = 0; r < m; ++r) {
+      const int s = row_slot[r], p = row_pos[r];
+      Q3_CHECK(s >= 0 && s < n_slots, Q3TTS_ERR_INVALID_ARG, "row %d: slot %d out of range", r, s);
+      const int w = win_start ? win_start[s] : 0;
+      Q3_CHECK(w >= 0 && w <= p && p - w + 1 <= capacity, Q3TTS_ERR_INVALID_ARG, "row %d: window [%d, %d] does not fit a ring of %d", r, w, p, capacity);
+      ++rows_of_slot[s];
+    }
+    if (kernel == 0)
+      for (int s = 0; s < n_slots; ++s) Q3_CHECK(rows_of_slot[s] <= 1, Q3TTS_ERR_INVALID_ARG, "kernel 0 takes at most one row per slot");
+    if (kernel == 1)  // rows of one slot append at distinct ring indices (their windows fit the ring, so distinct positions suffice)
+      for (int a = 0; a < m; ++a)
+        for (int b = a + 1; b < m; ++b)
+          Q3_CHECK(row_slot[a] != row_slot[b] || row_pos[a] != row_pos[b], Q3TTS_ERR_INVALID_ARG, "rows %d and %d share slot and position", a, b);
+    if (kernel == 2) {
+      Q3_CHECK(m == 2 * n_slots && !kv_f16 && out_f16 && capacity >= 2, Q3TTS_ERR_INVALID_ARG,
+               "kernel 2 takes rows (2s, 2s+1) of every slot, an fp32 cache of >= 2 positions and fp16 output");
+      for (int r = 0; r < m; ++r)
+        Q3_CHECK(row_slot[r] == r / 2 && row_pos[r] == r % 2 && (!win_start || win_start[r / 2] == 0), Q3TTS_ERR_INVALID_ARG,
+                 "kernel 2: row %d must be slot %d at position %d", r, r / 2, r % 2);
+    }
+    require_device(device);
+    init_talker_kernels();
+    auto dev = [&](const void* src, size_t bytes) -> void* {
+      void* d = nullptr;
+      Q3_CUDA(cudaMalloc(&d, std::max<size_t>(bytes, 16)));
+      allocs.push_back(d);
+      if (src) Q3_CUDA(cudaMemcpy(d, src, bytes, cudaMemcpyHostToDevice));
+      return d;
+    };
+    const int ld = (heads + 2 * kv_heads) * 128, ldo = heads * 128;
+    float* dqkv = (float*)dev(qkv, (size_t)m * ld * 4);
+    const float* dqn = (const float*)dev(q_norm, 128 * 4);
+    const float* dkn = (const float*)dev(k_norm, 128 * 4);
+    const float* dfreq = (const float*)dev(inv_freq, 64 * 4);
+    const int* dslot = (const int*)dev(row_slot, (size_t)m * 4);
+    const int* dpos = (const int*)dev(row_pos, (size_t)m * 4);
+    const int* dwin = win_start ? (const int*)dev(win_start, (size_t)n_slots * 4) : nullptr;
+    KVLayout kv;
+    kv.slot_stride = (size_t)kv_heads * capacity * 128;
+    kv.capacity = capacity;
+    kv.f16 = kv_f16 ? 1 : 0;
+    std::vector<__half> h16;
+    if (kv.f16) {
+      h16.resize(ring_elems);
+      for (size_t i = 0; i < ring_elems; ++i) h16[i] = __float2half_rn(k_ring[i]);
+      kv.k = dev(h16.data(), ring_elems * 2);
+      for (size_t i = 0; i < ring_elems; ++i) h16[i] = __float2half_rn(v_ring[i]);
+      kv.v = dev(h16.data(), ring_elems * 2);
+    } else {
+      kv.k = dev(k_ring, ring_elems * 4);
+      kv.v = dev(v_ring, ring_elems * 4);
+    }
+    void* dout = dev(nullptr, (size_t)m * ldo * (out_f16 ? 2 : 4));
+    Q3_CUDA(cudaMemset(dout, 0, (size_t)m * ldo * (out_f16 ? 2 : 4)));
+    LaunchCtx c{nullptr, nullptr};
+    if (kernel == 0) {
+      if (out_f16) launch_rope_attention_f16(c, dqkv, ld, m, heads, kv_heads, dqn, dkn, eps, dfreq, dslot, dpos, dwin, kv, (__half*)dout, ldo);
+      else launch_rope_attention(c, dqkv, ld, m, heads, kv_heads, dqn, dkn, eps, dfreq, dslot, dpos, dwin, kv, (float*)dout, ldo);
+    } else if (kernel == 1) {
+      launch_qk_norm_rope_append(c, dqkv, ld, m, heads, kv_heads, 128, dqn, dkn, eps, dfreq, dslot, dpos, kv);
+      if (out_f16) launch_attention_f16(c, dqkv, ld, m, heads, kv_heads, 128, dslot, dpos, dwin, kv, (__half*)dout, ldo);
+      else launch_attention(c, dqkv, ld, m, heads, kv_heads, 128, dslot, dpos, dwin, kv, (float*)dout, ldo);
+    } else {
+      launch_cp_pass0_attention_f16(c, dqkv, ld, n_slots, heads, kv_heads, dqn, dkn, eps, dfreq, kv, (__half*)dout, ldo);
+    }
+    Q3_CUDA(cudaGetLastError());
+    Q3_CUDA(cudaDeviceSynchronize());
+    if (kv.f16) {
+      Q3_CUDA(cudaMemcpy(h16.data(), kv.k, ring_elems * 2, cudaMemcpyDeviceToHost));
+      for (size_t i = 0; i < ring_elems; ++i) k_ring[i] = __half2float(h16[i]);
+      Q3_CUDA(cudaMemcpy(h16.data(), kv.v, ring_elems * 2, cudaMemcpyDeviceToHost));
+      for (size_t i = 0; i < ring_elems; ++i) v_ring[i] = __half2float(h16[i]);
+    } else {
+      Q3_CUDA(cudaMemcpy(k_ring, kv.k, ring_elems * 4, cudaMemcpyDeviceToHost));
+      Q3_CUDA(cudaMemcpy(v_ring, kv.v, ring_elems * 4, cudaMemcpyDeviceToHost));
+    }
+    if (out_f16) {
+      std::vector<__half> o((size_t)m * ldo);
+      Q3_CUDA(cudaMemcpy(o.data(), dout, o.size() * 2, cudaMemcpyDeviceToHost));
+      for (size_t i = 0; i < o.size(); ++i) out[i] = __half2float(o[i]);
+    } else {
+      Q3_CUDA(cudaMemcpy(out, dout, (size_t)m * ldo * 4, cudaMemcpyDeviceToHost));
+    }
+    for (void* d : allocs) cudaFree(d);
+    return Q3TTS_OK;
+  } catch (const Error& e) {
+    for (void* d : allocs) cudaFree(d);
+    g_create_error = e.what();
+    cudaGetLastError();
+    return e.status;
+  }
+}
+
 static q3tts_status skinny_trace_impl(int32_t device, int32_t M, int32_t N, int32_t K, int32_t bits, int32_t swiglu, int32_t residual, int32_t iters,
                                       uint64_t* stamps_out, int32_t capacity_ctas, int32_t* tiles_out, int32_t* split_out, int32_t* stages_out,
                                       double* avg_us_out) {

@@ -453,3 +453,23 @@ def conv_probe(x, w, bias=None, ntap=1, dil=1, act=0, swiglu=False, res=None, sc
     A.check(A.lib().q3tts_conv_probe(device, p(x), B, T, cin, p(w), p(keep[0]), N, ntap, dil, act, 1 if swiglu else 0, p(keep[1]), p(keep[2]),
                                      p(ea), p(ieb), sch, 1 if use_tensor_cores else 0, p(y32), p(y16)), None)
     return y32, y16
+
+
+def attention_probe(kernel, qkv, heads, kv_heads, q_norm, k_norm, eps, inv_freq, row_slot, row_pos, win_start, k_ring, v_ring,
+                    kv_f16=False, out_f16=False, device=0):
+    """`q3tts_attention_probe`: one talker attention launch.  qkv [m, (heads + 2*kv_heads)*128]; k_ring / v_ring
+    [n_slots, kv_heads, capacity, 128] (not modified); win_start [n_slots] or None.  -> (out [m, heads*128], k_ring, v_ring after
+    the launch), fp32 numpy (fp16 values widened)."""
+    f = lambda a: np.ascontiguousarray(a, dtype=np.float32)
+    i = lambda a: np.ascontiguousarray(a, dtype=np.int32)
+    qkv, q_norm, k_norm, inv_freq = f(qkv), f(q_norm), f(k_norm), f(inv_freq)
+    row_slot, row_pos = i(row_slot), i(row_pos)
+    win = None if win_start is None else i(win_start)
+    k_out, v_out = f(k_ring).copy(), f(v_ring).copy()
+    n_slots, _, capacity, _ = k_out.shape
+    m = qkv.shape[0]
+    out = np.zeros((m, heads * 128), dtype=np.float32)
+    pf, pi = (lambda a: a.ctypes.data_as(A.p_f32)), (lambda a: None if a is None else a.ctypes.data_as(A.p_i32))
+    A.check(A.lib().q3tts_attention_probe(device, kernel, int(bool(kv_f16)), int(bool(out_f16)), pf(qkv), m, heads, kv_heads, pf(q_norm), pf(k_norm),
+                                          eps, pf(inv_freq), pi(row_slot), pi(row_pos), pi(win), n_slots, capacity, pf(k_out), pf(v_out), pf(out)), None)
+    return out, k_out, v_out
