@@ -325,6 +325,44 @@ q3tts_status q3tts_attention_probe(int32_t device, int32_t kernel, int32_t kv_f1
                                    const float* inv_freq, const int32_t* row_slot, const int32_t* row_pos, const int32_t* win_start,
                                    int32_t n_slots, int32_t capacity, float* k_ring, float* v_ring, float* out);
 
+/* Codec-decoder kernels one launch at a time, through the engine's own launchers, on host buffers.  Every argument is validated on
+ * the host first: anything out of range returns Q3TTS_ERR_INVALID_ARG without touching the device.  Outputs no launch writes read
+ * as 3.4e38 (fp32) or NaN (fp16).
+ *
+ * Codec-transformer attention (head_dim 64, scale 1/sqrt(64)).  kernel: 0 = the tcgen05 pipeline's fp16-output launch on the
+ * mma.sync kernel (whatever Q3TTS_CODEC_ATT_MMA says), 1 = the SIMT pipeline's fp32 kernel (causal), 2 = its bidirectional form (ICL
+ * encoder), 3 = the fp16-output SIMT kernel (the fallback of kernel 0's launcher).  qkv [B][T][(nh + 2*nkv)*64] fp32, in/out: when
+ * inv_freq [32] is given the codec RoPE runs on it first, in place (positions t = row % T), and the roped rows come back.
+ * out [B][T][nh*64] fp32 (fp16 values widened for kernels 0 and 3).  1 <= B <= 64, 1 <= T <= 2400, nh <= 64, nh % nkv == 0. */
+q3tts_status q3tts_codec_attention_probe(int32_t device, int32_t kernel, float* qkv, int32_t B, int32_t T, int32_t nh, int32_t nkv,
+                                         const float* inv_freq, float* out);
+
+/* One DecoderResidualUnit of the vocoder (Vocoder/SpeechTokenizer.swift:696-718) on fp16 operands:
+ *   x' = res + conv1x1(snake2(conv7_dil(a) + b7)) + b1,   out = snake3(x')
+ * form: 1 = the fused kernel (codec_unit), 0 = the two tensor-core GEMM launches the decoder uses when the fused kernel does not take
+ * the shape.  a = snake1(x) and res = x [B][T][C] fp32 (rounded to fp16 on upload); w7 [7][C][C] (tap 6 reads row t, tap 0 row
+ * t - 6*dil), w1 [C][C] ([out][in]); b7 / b1 [C] or NULL; SnakeBeta parameters ea / ieb [C] (v + ieb * sin^2(v * ea)).
+ * weight_reps (1..32): copies of each fp16 weight laid out as the decoder stores them.  emit_residual: x' is stored (fp16) and
+ * returned in x_out (NULL otherwise); in_place: x' overwrites the residual buffer.  snake_out = out (fp16 widened).
+ * C % 32 == 0, 32 <= C <= 1536; form 1 also needs C <= 192, 128 + 6*dil <= 192 and B * ceil(T / 128) >= 32. */
+q3tts_status q3tts_codec_unit_probe(int32_t device, int32_t form, int32_t B, int32_t T, int32_t C, int32_t dil, const float* a,
+                                    const float* w7, const float* b7, const float* ea2, const float* ieb2, const float* w1, const float* b1,
+                                    const float* res, const float* ea3, const float* ieb3, int32_t in_place, int32_t emit_residual,
+                                    int32_t weight_reps, float* x_out, float* snake_out);
+
+/* DecoderOutputConv (causal 7 taps, C -> 1, then clip(-1, 1), NaN -> 0): y[b][t] from x [B][T][C], w [7][C] (tap 6 reads row t),
+ * bias [1].  kernel: 0 = the streaming fp16 kernel (C in {32, 64, 96, 128}; strip = outputs per warp, a multiple of 32, 0 = the
+ * default), 1 = the SIMT kernel on fp32 input, 2 = the SIMT kernel on fp16 input (C <= 256 for both), 3 = the tcgen05 GEMM's pcm
+ * epilogue (C % 8 == 0).  fp16 kernels round x on upload. */
+q3tts_status q3tts_codec_out_conv_probe(int32_t device, int32_t kernel, const float* x, int32_t B, int32_t T, int32_t C, const float* w,
+                                        const float* bias, int32_t strip, float* y);
+
+/* Row-wise codec ops on x [rows][ldx] -> y [rows][C]:  op 0 = causal depthwise conv k7 (w [7][C], b [C]; rows = B * T, tap 6 reads
+ * row t), 1 = LayerNorm (w, b [C], eps; fp32 out), 2 = LayerNorm with fp16 out, 3 = RMSNorm with fp16 out (w [C] or NULL, ldx >= C),
+ * 4 = SnakeBeta (w = ea, b = ieb), 5 = silu(x[:, :C]) * x[:, C:] (ldx = 2C).  Other ops take ldx = C. */
+q3tts_status q3tts_codec_rowop_probe(int32_t device, int32_t op, const float* x, int32_t rows, int32_t ldx, int32_t C, int32_t T,
+                                     const float* w, const float* b, float eps, float* y);
+
 /* ------------------------------------------------------------------------------------------------------
  * measurement hook (bench.py roofline): runs the dequant-fused linear launches of ONE talker decode step
  * (which = 0: 28 x {qkv, o, gate|up, down} + codec_head) or ONE code-predictor pass (which = 1) for `m` activation

@@ -10,6 +10,7 @@
 #include "speaker_encoder.h"
 #include "codec.h"
 #include "codec_kernels.h"
+#include "codec_unit.h"
 #include "engine.h"
 #include "gemm_tc.h"
 #include "tc_ptx.cuh"
@@ -1160,13 +1161,13 @@ q3tts_status q3tts_quantized_matmul(int32_t device, const float* x, int32_t m, c
 q3tts_status q3tts_quantized_matmul_tc(int32_t device, const float* x, int32_t m, const uint32_t* packed, const void* scales, const void* biases,
                                        int32_t scale_dtype, int32_t out_f, int32_t in_f, int32_t group, int32_t bits, const float* fold,
                                        int32_t swiglu_halves, const float* residual, float* y) {
+  std::vector<void*> allocs;
   try {
     Q3_CHECK(x && packed && scales && biases && y && m > 0 && m <= 128, Q3TTS_ERR_INVALID_ARG, "bad arguments (1 <= m <= 128)");
     require_device(device);
     init_tc_gemm();
     const int n_out = swiglu_halves ? out_f / 2 : out_f;
     const size_t wbytes = (size_t)out_f * in_f * bits / 8, sbytes = (size_t)out_f * (in_f / group) * dtype_size(scale_dtype);
-    std::vector<void*> allocs;
     auto dev = [&](const void* src, size_t bytes) -> void* {
       void* d = nullptr;
       Q3_CUDA(cudaMalloc(&d, std::max<size_t>(bytes, 16)));
@@ -1197,6 +1198,7 @@ q3tts_status q3tts_quantized_matmul_tc(int32_t device, const float* x, int32_t m
     for (void* d : allocs) cudaFree(d);
     return Q3TTS_OK;
   } catch (const Error& e) {
+    for (void* d : allocs) cudaFree(d);
     g_create_error = e.what();
     cudaGetLastError();
     return e.status;
@@ -1224,11 +1226,11 @@ q3tts_status q3tts_safetensors_check(const char* path, int32_t* n_tensors_out, i
 q3tts_status q3tts_conv_probe(int32_t device, const float* x, int32_t B, int32_t T, int32_t cin, const float* w, const float* bias, int32_t N,
                               int32_t ntap, int32_t dil, int32_t act, int32_t swiglu, const float* res, const float* scale,
                               const float* snake_ea, const float* snake_ieb, int32_t snake_ch, int32_t use_tc, float* y32, float* y16) {
+  std::vector<void*> allocs;
   try {
     Q3_CHECK(x && w && B > 0 && T > 0 && cin > 0 && N > 0 && ntap > 0 && dil > 0, Q3TTS_ERR_INVALID_ARG, "bad arguments");
     require_device(device);
     const size_t M = (size_t)B * T, nx = M * cin, nw = (size_t)ntap * N * cin, n_out = swiglu ? N / 2 : N, ny = M * n_out;
-    std::vector<void*> allocs;
     auto dev = [&](const void* src, size_t bytes) -> void* {
       void* d = nullptr;
       Q3_CUDA(cudaMalloc(&d, std::max<size_t>(bytes, 16)));
@@ -1281,6 +1283,7 @@ q3tts_status q3tts_conv_probe(int32_t device, const float* x, int32_t B, int32_t
     for (void* d : allocs) cudaFree(d);
     return Q3TTS_OK;
   } catch (const Error& e) {
+    for (void* d : allocs) cudaFree(d);
     g_create_error = e.what();
     cudaGetLastError();
     return e.status;
@@ -1394,6 +1397,247 @@ q3tts_status q3tts_attention_probe(int32_t device, int32_t kernel, int32_t kv_f1
     g_create_error = e.what();
     cudaGetLastError();
     return e.status;
+  }
+}
+
+// ------------------------------------------------------------------------------------------------ codec kernel probes
+namespace {
+// device copies of a probe's host buffers; every allocation is freed when the probe returns, on every path
+struct ProbeBuffers {
+  std::vector<void*> allocs;
+  ProbeBuffers() = default;
+  ProbeBuffers(const ProbeBuffers&) = delete;
+  ProbeBuffers& operator=(const ProbeBuffers&) = delete;
+  ~ProbeBuffers() { for (void* d : allocs) cudaFree(d); }
+  void* alloc(size_t bytes) {
+    void* d = nullptr;
+    Q3_CUDA(cudaMalloc(&d, std::max<size_t>(bytes, 16)));
+    allocs.push_back(d);
+    return d;
+  }
+  float* f32(const float* src, size_t n) {  // src == null: uninitialised
+    float* d = (float*)alloc(n * 4);
+    if (src) Q3_CUDA(cudaMemcpy(d, src, n * 4, cudaMemcpyHostToDevice));
+    return d;
+  }
+  // fp16 copy (round to nearest) of n values, `reps` times, f16_rep_stride_bytes(n) apart: the layout of CodecDecoder::upload_f16
+  __half* f16(const float* src, size_t n, int reps = 1) {
+    std::vector<__half> h(n);
+    for (size_t i = 0; i < n; ++i) h[i] = __float2half_rn(src[i]);
+    const size_t stride = f16_rep_stride_bytes(n);
+    uint8_t* d = (uint8_t*)alloc(stride * (size_t)reps);
+    for (int r = 0; r < reps; ++r) Q3_CUDA(cudaMemcpy(d + (size_t)r * stride, h.data(), n * 2, cudaMemcpyHostToDevice));
+    return (__half*)d;
+  }
+};
+
+void widen_f16(const __half* d, size_t n, float* out) {
+  std::vector<__half> h(n);
+  Q3_CUDA(cudaMemcpy(h.data(), d, n * 2, cudaMemcpyDeviceToHost));
+  for (size_t i = 0; i < n; ++i) out[i] = __half2float(h[i]);
+}
+
+q3tts_status probe_failed(const Error& e) {
+  g_create_error = e.what();
+  cudaGetLastError();
+  return e.status;
+}
+
+constexpr size_t kProbeMaxElems = (size_t)1 << 31;  // every buffer of a probe stays below 2^31 elements (the kernels' int row math)
+}  // namespace
+
+q3tts_status q3tts_codec_attention_probe(int32_t device, int32_t kernel, float* qkv, int32_t B, int32_t T, int32_t nh, int32_t nkv,
+                                         const float* inv_freq, float* out) {
+  ProbeBuffers buf;
+  try {
+    Q3_CHECK(qkv && out, Q3TTS_ERR_INVALID_ARG, "NULL argument");
+    Q3_CHECK(kernel >= 0 && kernel <= 3, Q3TTS_ERR_INVALID_ARG, "kernel must be 0, 1, 2 or 3");
+    Q3_CHECK(B >= 1 && B <= 64 && T >= 1 && T <= 2400, Q3TTS_ERR_INVALID_ARG, "B %d / T %d outside 1..64 / 1..2400", B, T);
+    Q3_CHECK(nkv >= 1 && nh >= 1 && nh <= 64 && nh % nkv == 0, Q3TTS_ERR_INVALID_ARG, "heads %d / kv heads %d (nh <= 64, nh %% nkv == 0)", nh, nkv);
+    const int ld = (nh + 2 * nkv) * 64, ldo = nh * 64;
+    const size_t M = (size_t)B * T;
+    Q3_CHECK(M * ld < kProbeMaxElems, Q3TTS_ERR_INVALID_ARG, "qkv too large");
+    require_device(device);
+    LaunchCtx c{nullptr, nullptr};
+    float* dqkv = buf.f32(qkv, M * ld);
+    if (inv_freq) launch_codec_rope(c, dqkv, ld, (int)M, T, nh + nkv, buf.f32(inv_freq, 32));  // q and k heads, in place (decode_pass_*)
+    if (kernel == 1 || kernel == 2) {
+      float* dout = buf.f32(nullptr, M * ldo);
+      Q3_CUDA(cudaMemset(dout, 0x7f, M * ldo * 4));  // an output no launch writes reads as 3.4e38
+      if (kernel == 1) launch_codec_attention(c, dqkv, ld, B, T, nh, nkv, dout, ldo);
+      else launch_codec_attention_bidir(c, dqkv, ld, B, T, nh, nkv, dout, ldo);
+      Q3_CUDA(cudaGetLastError());
+      Q3_CUDA(cudaDeviceSynchronize());
+      Q3_CUDA(cudaMemcpy(out, dout, M * ldo * 4, cudaMemcpyDeviceToHost));
+    } else {
+      __half* dout = (__half*)buf.alloc(M * ldo * 2);
+      Q3_CUDA(cudaMemset(dout, 0x7f, M * ldo * 2));  // fp16 NaN
+      launch_codec_attention_f16(c, dqkv, ld, B, T, nh, nkv, dout, ldo, kernel == 0);
+      Q3_CUDA(cudaGetLastError());
+      Q3_CUDA(cudaDeviceSynchronize());
+      widen_f16(dout, M * ldo, out);
+    }
+    if (inv_freq) Q3_CUDA(cudaMemcpy(qkv, dqkv, M * ld * 4, cudaMemcpyDeviceToHost));
+    return Q3TTS_OK;
+  } catch (const Error& e) {
+    return probe_failed(e);
+  }
+}
+
+q3tts_status q3tts_codec_unit_probe(int32_t device, int32_t form, int32_t B, int32_t T, int32_t C, int32_t dil, const float* a,
+                                    const float* w7, const float* b7, const float* ea2, const float* ieb2, const float* w1, const float* b1,
+                                    const float* res, const float* ea3, const float* ieb3, int32_t in_place, int32_t emit_residual,
+                                    int32_t weight_reps, float* x_out, float* snake_out) {
+  ProbeBuffers buf;
+  try {
+    Q3_CHECK(a && w7 && ea2 && ieb2 && w1 && res && ea3 && ieb3 && snake_out, Q3TTS_ERR_INVALID_ARG, "NULL argument");
+    Q3_CHECK(form == 0 || form == 1, Q3TTS_ERR_INVALID_ARG, "form must be 0 (two GEMM launches) or 1 (fused unit)");
+    Q3_CHECK(!in_place || emit_residual, Q3TTS_ERR_INVALID_ARG, "in_place needs emit_residual");
+    Q3_CHECK(!emit_residual == !x_out, Q3TTS_ERR_INVALID_ARG, "x_out must be given exactly when emit_residual is set");
+    Q3_CHECK(weight_reps >= 1 && weight_reps <= 32, Q3TTS_ERR_INVALID_ARG, "weight_reps %d outside 1..32", weight_reps);
+    Q3_CHECK(B >= 1 && T >= 1 && dil >= 1 && dil <= 64 && C >= 32 && C <= 1536 && C % 32 == 0, Q3TTS_ERR_INVALID_ARG,
+             "bad shape (B %d, T %d, C %d, dilation %d)", B, T, C, dil);
+    const size_t M = (size_t)B * T;
+    Q3_CHECK(M * C < kProbeMaxElems, Q3TTS_ERR_INVALID_ARG, "activations too large");
+    Q3_CHECK(form == 0 || codec_unit_shape_supported(B, T, C, dil), Q3TTS_ERR_INVALID_ARG,
+             "the fused unit does not run C %d, dilation %d, %d x %d rows", C, dil, B, T);
+    require_device(device);
+    const size_t n7 = (size_t)7 * C * C, n1 = (size_t)C * C;
+    const __half* da = buf.f16(a, M * C);
+    const __half* dw7 = buf.f16(w7, n7, weight_reps);
+    const __half* dw1 = buf.f16(w1, n1, weight_reps);
+    const float* db7 = b7 ? buf.f32(b7, C) : nullptr;
+    const float* db1 = b1 ? buf.f32(b1, C) : nullptr;
+    const float *dea2 = buf.f32(ea2, C), *dieb2 = buf.f32(ieb2, C), *dea3 = buf.f32(ea3, C), *dieb3 = buf.f32(ieb3, C);
+    __half* dres = buf.f16(res, M * C);
+    __half* doutr = !emit_residual ? nullptr : in_place ? dres : (__half*)buf.alloc(M * C * 2);
+    __half* dout = (__half*)buf.alloc(M * C * 2);
+    if (doutr && !in_place) Q3_CUDA(cudaMemset(doutr, 0x7f, M * C * 2));  // fp16 NaN where nothing is written
+    Q3_CUDA(cudaMemset(dout, 0x7f, M * C * 2));
+    LaunchCtx c{nullptr, nullptr};
+    if (form == 1) {
+      init_codec_unit();
+      CodecUnit u;
+      u.Bt = B; u.T = T; u.C = C; u.dil = dil;
+      u.a = da; u.w7 = dw7; u.b7 = db7; u.snake2_ea = dea2; u.snake2_ieb = dieb2; u.w1 = dw1; u.b1 = db1;
+      u.w7_reps = u.w1_reps = weight_reps;
+      u.w7_rep_stride = f16_rep_stride_bytes(n7) / 2; u.w1_rep_stride = f16_rep_stride_bytes(n1) / 2;
+      u.res16 = dres; u.outr16 = doutr; u.out16 = dout; u.next_ea = dea3; u.next_ieb = dieb3;
+      launch_codec_unit(c, u);
+    } else {  // what decode_pass_tc launches for a unit the fused kernel does not take
+      init_tc_gemm();
+      __half* dh = (__half*)buf.alloc(M * C * 2);
+      TcGemm g;
+      g.a = da; g.w = dw7; g.w_reps = weight_reps; g.w_rep_stride = f16_rep_stride_bytes(n7) / 2;
+      g.Bt = B; g.T = T; g.cin = C; g.N = C; g.ntap = 7; g.dil = dil; g.bias = db7;
+      g.out16 = dh; g.ld16 = C; g.snake_ea = dea2; g.snake_ieb = dieb2; g.snake_ch = C;
+      launch_tc_gemm(c, g);
+      TcGemm g2;
+      g2.a = dh; g2.w = dw1; g2.w_reps = weight_reps; g2.w_rep_stride = f16_rep_stride_bytes(n1) / 2;
+      g2.Bt = B; g2.T = T; g2.cin = C; g2.N = C; g2.bias = db1;
+      g2.ld_res = C; g2.ld32 = C; g2.res16 = dres; g2.allow_skinny = 0; g2.outr16 = doutr;
+      g2.out16 = dout; g2.ld16 = C; g2.snake_ea = dea3; g2.snake_ieb = dieb3; g2.snake_ch = C;
+      launch_tc_gemm(c, g2);
+    }
+    Q3_CUDA(cudaGetLastError());
+    Q3_CUDA(cudaDeviceSynchronize());
+    widen_f16(dout, M * C, snake_out);
+    if (doutr) widen_f16(doutr, M * C, x_out);
+    return Q3TTS_OK;
+  } catch (const Error& e) {
+    return probe_failed(e);
+  }
+}
+
+q3tts_status q3tts_codec_out_conv_probe(int32_t device, int32_t kernel, const float* x, int32_t B, int32_t T, int32_t C, const float* w,
+                                        const float* bias, int32_t strip, float* y) {
+  ProbeBuffers buf;
+  try {
+    Q3_CHECK(x && w && bias && y, Q3TTS_ERR_INVALID_ARG, "NULL argument");
+    Q3_CHECK(kernel >= 0 && kernel <= 3, Q3TTS_ERR_INVALID_ARG, "kernel must be 0, 1, 2 or 3");
+    Q3_CHECK(B >= 1 && T >= 1 && C >= 1, Q3TTS_ERR_INVALID_ARG, "bad shape (B %d, T %d, C %d)", B, T, C);
+    const size_t M = (size_t)B * T;
+    Q3_CHECK(M * C < kProbeMaxElems, Q3TTS_ERR_INVALID_ARG, "activations too large");
+    Q3_CHECK(kernel == 0 || strip == 0, Q3TTS_ERR_INVALID_ARG, "strip applies to kernel 0 only");
+    if (kernel == 0)
+      Q3_CHECK(out_conv_stream_supported(C) && (strip == 0 || (strip >= 32 && strip <= 65536 && strip % 32 == 0)), Q3TTS_ERR_INVALID_ARG,
+               "streaming kernel: C %d not in {32, 64, 96, 128} or strip %d not 0 / a multiple of 32 in 32..65536", C, strip);
+    if (kernel == 1 || kernel == 2) Q3_CHECK(C <= 256, Q3TTS_ERR_INVALID_ARG, "C %d > 256 (the tile of 134 rows x C lives in shared memory)", C);
+    if (kernel == 3) Q3_CHECK(C % 8 == 0 && C <= 1536, Q3TTS_ERR_INVALID_ARG, "tensor-core form: C %d not a multiple of 8 up to 1536", C);
+    require_device(device);
+    LaunchCtx c{nullptr, nullptr};
+    float* dy = buf.f32(nullptr, M);
+    Q3_CUDA(cudaMemset(dy, 0x7f, M * 4));  // an output no launch writes reads as 3.4e38, outside the clip range
+    if (kernel == 3) {  // the engine's out_tc_: the one output channel padded to 32 columns, [7][32][C] fp16, 8 copies, bias [32]
+      init_tc_gemm();
+      std::vector<float> wp((size_t)7 * 32 * C, 0.f), bp(32, 0.f);
+      for (int k = 0; k < 7; ++k)
+        for (int ch = 0; ch < C; ++ch) wp[(size_t)k * 32 * C + ch] = w[(size_t)k * C + ch];
+      bp[0] = bias[0];
+      const int reps = 8;
+      TcGemm g;
+      g.a = buf.f16(x, M * C); g.w = buf.f16(wp.data(), wp.size(), reps); g.w_reps = reps; g.w_rep_stride = f16_rep_stride_bytes(wp.size()) / 2;
+      g.Bt = B; g.T = T; g.cin = C; g.N = 32; g.ntap = 7; g.dil = 1; g.bias = buf.f32(bp.data(), 32);
+      g.pcm = dy;
+      launch_tc_gemm(c, g);
+    } else {
+      init_codec_kernels();
+      const float* dw = buf.f32(w, (size_t)7 * C);
+      const float* db = buf.f32(bias, 1);
+      if (kernel == 0) launch_out_conv_stream_f16(c, buf.f16(x, M * C), dw, db, C, B, T, dy, strip);
+      else if (kernel == 1) launch_out_conv(c, buf.f32(x, M * C), dw, db, C, B, T, dy);
+      else launch_out_conv_f16(c, buf.f16(x, M * C), dw, db, C, B, T, dy);
+    }
+    Q3_CUDA(cudaGetLastError());
+    Q3_CUDA(cudaDeviceSynchronize());
+    Q3_CUDA(cudaMemcpy(y, dy, M * 4, cudaMemcpyDeviceToHost));
+    return Q3TTS_OK;
+  } catch (const Error& e) {
+    return probe_failed(e);
+  }
+}
+
+q3tts_status q3tts_codec_rowop_probe(int32_t device, int32_t op, const float* x, int32_t rows, int32_t ldx, int32_t C, int32_t T,
+                                     const float* w, const float* b, float eps, float* y) {
+  ProbeBuffers buf;
+  try {
+    Q3_CHECK(x && y, Q3TTS_ERR_INVALID_ARG, "NULL argument");
+    Q3_CHECK(op >= 0 && op <= 5, Q3TTS_ERR_INVALID_ARG, "op must be 0..5");
+    Q3_CHECK(rows >= 1 && C >= 1 && C <= 65536, Q3TTS_ERR_INVALID_ARG, "bad shape (rows %d, C %d)", rows, C);
+    Q3_CHECK(op == 3 || op == 5 || w, Q3TTS_ERR_INVALID_ARG, "op %d needs w", op);
+    Q3_CHECK(op == 3 || op == 5 || b, Q3TTS_ERR_INVALID_ARG, "op %d needs b", op);
+    const int want_ld = op == 5 ? 2 * C : C;
+    Q3_CHECK(op == 3 ? ldx >= C : ldx == want_ld, Q3TTS_ERR_INVALID_ARG, "ldx %d (op %d wants %s %d)", ldx, op, op == 3 ? ">=" : "==", want_ld);
+    Q3_CHECK(op != 0 || (T >= 1 && rows % T == 0), Q3TTS_ERR_INVALID_ARG, "dwconv7: rows %d not a multiple of T %d", rows, T);
+    Q3_CHECK((size_t)rows * ldx < kProbeMaxElems, Q3TTS_ERR_INVALID_ARG, "input too large");
+    require_device(device);
+    LaunchCtx c{nullptr, nullptr};
+    const size_t ny = (size_t)rows * C;
+    const float* dx = buf.f32(x, (size_t)rows * ldx);
+    const float* dw = w ? buf.f32(w, (size_t)(op == 0 ? 7 : 1) * C) : nullptr;
+    const float* db = b ? buf.f32(b, C) : nullptr;
+    if (op == 2 || op == 3) {
+      __half* dy = (__half*)buf.alloc(ny * 2);
+      Q3_CUDA(cudaMemset(dy, 0x7f, ny * 2));
+      if (op == 2) launch_layernorm_f16(c, dx, rows, C, dw, db, eps, dy);
+      else launch_rmsnorm_f16(c, dx, ldx, rows, C, dw, eps, dy, C);
+      Q3_CUDA(cudaGetLastError());
+      Q3_CUDA(cudaDeviceSynchronize());
+      widen_f16(dy, ny, y);
+    } else {
+      float* dy = buf.f32(nullptr, ny);
+      Q3_CUDA(cudaMemset(dy, 0x7f, ny * 4));
+      if (op == 0) launch_dwconv7(c, dx, dw, db, C, T, rows, dy);
+      else if (op == 1) launch_layernorm(c, dx, rows, C, dw, db, eps, dy);
+      else if (op == 4) { SnakeW s; s.alpha = dw; s.beta = db; s.ch = C; launch_snake(c, dx, s, rows, dy); }
+      else launch_silu_mul(c, dx, rows, C, dy);
+      Q3_CUDA(cudaGetLastError());
+      Q3_CUDA(cudaDeviceSynchronize());
+      Q3_CUDA(cudaMemcpy(y, dy, ny * 4, cudaMemcpyDeviceToHost));
+    }
+    return Q3TTS_OK;
+  } catch (const Error& e) {
+    return probe_failed(e);
   }
 }
 

@@ -52,7 +52,7 @@ const STensor& need(const std::map<std::string, STensor>& t, const std::string& 
 const __half* CodecDecoder::upload_f16(const std::vector<float>& h, int reps, size_t* rep_stride) {
   std::vector<__half> r(h.size());
   for (size_t i = 0; i < h.size(); ++i) r[i] = __float2half_rn(h[i]);
-  const size_t stride = (r.size() * sizeof(__half) + 255) / 256 * 256;  // bytes between copies
+  const size_t stride = f16_rep_stride_bytes(r.size());  // bytes between copies
   __half* d = (__half*)arena_.alloc(stride * (size_t)reps);
   for (int i = 0; i < reps; ++i)
     Q3_CUDA(cudaMemcpy(reinterpret_cast<uint8_t*>(d) + (size_t)i * stride, r.data(), r.size() * sizeof(__half), cudaMemcpyHostToDevice));

@@ -48,6 +48,9 @@ enum ConvEpilogue { CE_STORE = 0, CE_GELU = 1, CE_RES_SCALE = 2 };
 
 struct SnakeW { const float *alpha = nullptr, *beta = nullptr; int ch = 0; };
 
+// bytes between the copies of an fp16 weight of `halves` elements (ConvW::w16_reps): each copy starts 256-byte aligned
+inline size_t f16_rep_stride_bytes(size_t halves) { return (halves * sizeof(__half) + 255) / 256 * 256; }
+
 class CodecDecoder {
  public:
   CodecDecoder(const std::string& dir, cudaStream_t stream, LaunchCounter* counter, int pass_frames);

@@ -399,14 +399,22 @@ codec_unit_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant
 
 }  // namespace
 
+bool codec_unit_shape_supported(int Bt, int T, int C, int dil) {
+  if (C % 32 != 0 || C < 32 || C > kMaxC) return false;             // one CTA owns all C columns; 2.5 * C tensor-memory columns
+  if (dil < 1 || kTileM + (kTaps - 1) * dil > kHaloRowsMax) return false;  // the halo tile is one 192-row stage
+  if (Bt < 1 || T < 1 || (long long)Bt * ((T + kTileM - 1) / kTileM) < 32) return false;  // a few tiles: the two-kernel form (its <= 128-row variants) is fine
+  return true;
+}
+
+static bool codec_unit_launchable(const CodecUnit& u) {
+  if (!u.res16 || !u.out16 || !u.a || !u.w7 || !u.w1 || !u.snake2_ea || !u.next_ea) return false;
+  return codec_unit_shape_supported(u.Bt, u.T, u.C, u.dil);
+}
+
 bool codec_unit_supported(const CodecUnit& u) {
   const char* e = getenv("Q3TTS_CODEC_UNIT");  // read per call: the A/B test flips it between two handles of one process
   if (e && atoi(e) == 0) return false;
-  if (u.C % 32 != 0 || u.C < 32 || u.C > kMaxC) return false;       // one CTA owns all C columns; 2.5 * C tensor-memory columns
-  if (kTileM + (kTaps - 1) * u.dil > kHaloRowsMax) return false;     // the halo tile is one 192-row stage
-  if (!u.res16 || !u.out16 || !u.a || !u.w7 || !u.w1 || !u.snake2_ea || !u.next_ea) return false;
-  if ((long long)u.Bt * ((u.T + kTileM - 1) / kTileM) < 32) return false;  // a few tiles: the two-kernel form (its <= 128-row variants) is fine
-  return true;
+  return codec_unit_launchable(u);
 }
 
 void init_codec_unit() {
@@ -415,7 +423,7 @@ void init_codec_unit() {
 }
 
 void launch_codec_unit(const LaunchCtx& c, const CodecUnit& u) {
-  Q3_CHECK(codec_unit_supported(u), Q3TTS_ERR_INVALID_ARG, "codec_unit: unsupported shape (C %d, dilation %d, %d x %d rows)", u.C, u.dil, u.Bt, u.T);
+  Q3_CHECK(codec_unit_launchable(u), Q3TTS_ERR_INVALID_ARG, "codec_unit: unsupported shape (C %d, dilation %d, %d x %d rows)", u.C, u.dil, u.Bt, u.T);
   UnitParams p{};
   p.Bt = u.Bt; p.T = u.T; p.C = u.C; p.dil = u.dil;
   p.tiles_per_batch = (u.T + kTileM - 1) / kTileM;

@@ -24,7 +24,12 @@ struct CodecUnit {
   const float* next_ieb = nullptr;
 };
 
+// the shapes the fused kernel runs (C % 32 == 0, C <= 192, 128 + 6 * dil <= 192 halo rows, >= 32 row tiles)
+bool codec_unit_shape_supported(int Bt, int T, int C, int dil);
+// the shape is supported, every required operand is set and Q3TTS_CODEC_UNIT is not 0
 bool codec_unit_supported(const CodecUnit& u);
+// runs any supported shape with its operands set, whatever Q3TTS_CODEC_UNIT says: the decoder picks between this and the two-kernel
+// form with codec_unit_supported
 void launch_codec_unit(const LaunchCtx& c, const CodecUnit& u);
 void init_codec_unit();
 

@@ -85,6 +85,11 @@ SYMBOLS = {
     "q3tts_conv_probe": (i32, [i32, p_f32, i32, i32, i32, p_f32, p_f32, i32, i32, i32, i32, i32, p_f32, p_f32, p_f32, p_f32, i32, i32, p_f32, p_f32]),
     "q3tts_attention_probe": (i32, [i32, i32, i32, i32, p_f32, i32, i32, i32, p_f32, p_f32, f32, p_f32, p_i32, p_i32, p_i32, i32, i32, p_f32, p_f32,
                                     p_f32]),
+    "q3tts_codec_attention_probe": (i32, [i32, i32, p_f32, i32, i32, i32, i32, p_f32, p_f32]),
+    "q3tts_codec_unit_probe": (i32, [i32, i32, i32, i32, i32, i32, p_f32, p_f32, p_f32, p_f32, p_f32, p_f32, p_f32, p_f32, p_f32, p_f32, i32, i32,
+                                     i32, p_f32, p_f32]),
+    "q3tts_codec_out_conv_probe": (i32, [i32, i32, p_f32, i32, i32, i32, p_f32, p_f32, i32, p_f32]),
+    "q3tts_codec_rowop_probe": (i32, [i32, i32, p_f32, i32, i32, i32, i32, p_f32, p_f32, f32, p_f32]),
     "q3tts_profile_linear": (i32, [C.c_void_p, i32, i32, i32, C.POINTER(C.c_double), C.POINTER(i64), C.POINTER(i64)]),
     "q3tts_skinny_trace": (i32, [i32, i32, i32, i32, i32, i32, i32, C.POINTER(C.c_uint64), i32, C.POINTER(i32), C.POINTER(i32), C.POINTER(i32),
                                  C.POINTER(C.c_double)]),

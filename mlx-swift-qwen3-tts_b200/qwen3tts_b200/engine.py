@@ -473,3 +473,57 @@ def attention_probe(kernel, qkv, heads, kv_heads, q_norm, k_norm, eps, inv_freq,
     A.check(A.lib().q3tts_attention_probe(device, kernel, int(bool(kv_f16)), int(bool(out_f16)), pf(qkv), m, heads, kv_heads, pf(q_norm), pf(k_norm),
                                           eps, pf(inv_freq), pi(row_slot), pi(row_pos), pi(win), n_slots, capacity, pf(k_out), pf(v_out), pf(out)), None)
     return out, k_out, v_out
+
+
+def _f32(a):
+    return None if a is None else np.ascontiguousarray(a, dtype=np.float32)
+
+
+def _pf(a):
+    return None if a is None else a.ctypes.data_as(A.p_f32)
+
+
+def codec_attention_probe(kernel, qkv, nh, nkv, inv_freq=None, device=0):
+    """`q3tts_codec_attention_probe`: qkv [B, T, (nh + 2*nkv)*64]; inv_freq [32] or None (no RoPE).
+    -> (out [B, T, nh*64], qkv after the in-place RoPE), fp32 numpy (fp16 outputs widened)."""
+    q = _f32(qkv).copy()
+    B, T, _ = q.shape
+    f = _f32(inv_freq)
+    out = np.zeros((B, T, nh * 64), dtype=np.float32)
+    A.check(A.lib().q3tts_codec_attention_probe(device, kernel, _pf(q), B, T, nh, nkv, _pf(f), _pf(out)), None)
+    return out, q
+
+
+def codec_unit_probe(form, a, w7, b7, ea2, ieb2, w1, b1, res, ea3, ieb3, dil, in_place=False, emit_residual=True, weight_reps=1, device=0):
+    """`q3tts_codec_unit_probe`: one vocoder residual unit.  a, res [B, T, C]; w7 [7, C, C]; w1 [C, C]; b7 / b1 [C] or None.
+    -> (x' [B, T, C] or None when not emitted, snake3(x') [B, T, C]), fp16 values widened to fp32."""
+    a, res = _f32(a), _f32(res)
+    B, T, C = a.shape
+    keep = [_f32(v) for v in (w7, b7, ea2, ieb2, w1, b1, ea3, ieb3)]
+    x_out = np.zeros((B, T, C), dtype=np.float32) if emit_residual else None
+    out = np.zeros((B, T, C), dtype=np.float32)
+    A.check(A.lib().q3tts_codec_unit_probe(device, form, B, T, C, dil, _pf(a), *[_pf(v) for v in keep[:6]], _pf(res), _pf(keep[6]), _pf(keep[7]),
+                                           int(bool(in_place)), int(bool(emit_residual)), weight_reps, _pf(x_out), _pf(out)), None)
+    return x_out, out
+
+
+def codec_out_conv_probe(kernel, x, w, bias, strip=0, device=0):
+    """`q3tts_codec_out_conv_probe`: x [B, T, C], w [7, C], bias [1] -> pcm [B, T] (clipped, NaN -> 0)."""
+    x, w, b = _f32(x), _f32(w), _f32(np.reshape(bias, (1,)))
+    B, T, C = x.shape
+    y = np.zeros((B, T), dtype=np.float32)
+    A.check(A.lib().q3tts_codec_out_conv_probe(device, kernel, _pf(x), B, T, C, _pf(w), _pf(b), strip, _pf(y)), None)
+    return y
+
+
+CODEC_ROWOPS = {"dwconv7": 0, "layernorm": 1, "layernorm_f16": 2, "rmsnorm_f16": 3, "snake": 4, "silu_mul": 5}
+
+
+def codec_rowop_probe(op, x, C, w=None, b=None, eps=1e-6, T=0, device=0):
+    """`q3tts_codec_rowop_probe`: x [rows, ldx] -> y [rows, C] (fp16 outputs widened).  op is a key of CODEC_ROWOPS."""
+    x = _f32(x)
+    rows, ldx = x.shape
+    w, b = _f32(w), _f32(b)
+    y = np.zeros((rows, C), dtype=np.float32)
+    A.check(A.lib().q3tts_codec_rowop_probe(device, CODEC_ROWOPS[op], _pf(x), rows, ldx, C, T, _pf(w), _pf(b), eps, _pf(y)), None)
+    return y
