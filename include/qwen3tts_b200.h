@@ -72,7 +72,9 @@ typedef struct q3tts_options {
                                today 2; env Q3TTS_SKINNY_Q=1 flips it).  Same bits either way (the copies ARE the dequantised values). */
   int32_t runtime_quantization; /* Qwen3TTSPipelineConfiguration.applyRuntimeQuantization (Qwen3TTSPipeline.swift:25, 184, 961-980): a checkpoint
                                without a `quantization` block is MLX-quantised at load, group 64, 6 bits for embeddings / q,k,v projections /
-                               heads, 4 bits for the rest (codes held in an 8-bit container).  0 = run the checkpoint as stored */
+                               heads, 4 bits for the rest (codes held in an 8-bit container).  0 = run the checkpoint as stored.
+                               Checkpoints with a `quantization` block are never re-quantised; MLX affine checkpoints of 2, 3, 4, 5, 6
+                               and 8 bits with group_size 32, 64 or 128 load as stored (q3tts_info.checkpoint_quant_bits) */
   int32_t lanes;            /* > 1: q3tts_generate_pcm_batch / q3tts_generate_codes_batch calls with more than max_batch requests are split over
                                `lanes` handles (this one + lazily created q3tts_clone()s sharing its weights), each served by a worker thread
                                of the call: several latency-bound launch chains overlap on the device (see q3tts_clone).  The threads live
@@ -96,7 +98,10 @@ typedef struct q3tts_info {
   int32_t audio_encoder_hidden; /* width of the quantiser input (q3tts_encode_reference_audio latent_out) */
   int32_t has_speaker_encoder;   /* model.safetensors carries `speaker_encoder.*` (Qwen3TTSPipeline.swift:82-84, 155-169) */
   int32_t speaker_embedding_dim; /* enc_dim of the ECAPA-TDNN (1024 in the reference) */
-  int32_t reserved[4];
+  int32_t checkpoint_quant_bits; /* width of the MLX-packed leaves on disk (2, 3, 4, 5, 6 or 8); 0 = dense checkpoint, runtime-quantised
+                                    or not.  quant_bits is the width the kernels stream: 2 / 3-bit codes are held in 4-bit words and 5 / 6-bit
+                                    codes in 8-bit words, unchanged (DESIGN.md §1) */
+  int32_t reserved[3];
 } q3tts_info;
 
 /* ---- one utterance; replaces the argument list of Qwen3Talker.generateCodes / generateStream
@@ -147,7 +152,8 @@ typedef struct q3tts_timing {
   int64_t graph_replays;
   int64_t frames;          /* talker frames produced (before the validity filter) */
   int64_t h2d_bytes, d2h_bytes;
-  int64_t weight_bytes_per_frame; /* algorithmic bytes streamed per 12.5 Hz frame (SURVEY.md §8d) */
+  int64_t weight_bytes_per_frame; /* algorithmic bytes streamed per 12.5 Hz frame (SURVEY.md §8d): weights counted in the 4 / 8-bit
+                                     words the kernels read, so a 3-bit checkpoint counts as 4-bit and a 5 / 6-bit one as 8-bit */
   double talker_ms;               /* CUDA-event time of prompt assembly + prefill + all frame steps of the last call */
   int64_t codec_flops;            /* algorithmic flops of the codec passes of the last call (SURVEY.md §8d) */
   int64_t persistent_launches;    /* launches of the persistent frame kernel in the last call (0 = CUDA-graph / eager path) */
@@ -258,7 +264,11 @@ q3tts_status q3tts_generate_pcm_batch(q3tts_handle* h, const q3tts_request* reqs
  * ---------------------------------------------------------------------------------------------------- */
 /* MLX `dequantized(w, scales:, biases:, groupSize:, bits:, dtype:)` as called at Model/Qwen3Talker.swift:156.
  * packed [out][in*bits/32] uint32, scales/biases [out][in/group] of `scale_dtype`; out [out][in] of `out_dtype`.
- * Contract: deq32 = fp32(scale)*q (rounded) + fp32(bias) (rounded); result = round_to_nearest_even(deq32). */
+ * Contract: deq32 = fp32(scale)*q (rounded) + fp32(bias) (rounded); result = round_to_nearest_even(deq32).
+ * bits 2, 3, 4, 5, 6 or 8: a row is one little-endian LSB-first bit stream, code j at bits [j*bits, (j+1)*bits) (for 2 / 4 / 8 bits:
+ * element j of a word at bit offset j*bits).  Bits 2 / 3 / 5 / 6 need group_size 32, 64 or 128 and in % 32 == 0; they are widened on
+ * the device into the 4 / 8-bit words the loader keeps, then run the same kernel.  The same widths and rules hold for
+ * q3tts_quantized_matmul and q3tts_quantized_matmul_tc; arguments are checked before any device is touched. */
 /* MLX `quantize(w, group_size: 64, bits)` (affine) on the device -- the quantiser behind q3tts_options.runtime_quantization
  * (Qwen3TTSPipeline.applyMixedQuantization, Qwen3TTSPipeline.swift:961-980; bits 4, 6 or 8).  w: [out_f][in_f] of w_dtype (host);
  * codes8_out: [out_f][in_f] bytes, one code per byte (the 8-bit container, = MLX-packed 8-bit words); scales_out / biases_out:

@@ -568,6 +568,7 @@ q3tts_status q3tts_get_info(const q3tts_handle* hc, q3tts_info* out) {
     out->cp_hidden_size = c.cp.hidden_size; out->cp_num_layers = c.cp.num_hidden_layers; out->cp_vocab_size = c.cp.vocab_size;
     out->num_code_groups = c.cp.num_code_groups;
     out->quant_bits = hc->talker->quant_bits(); out->quant_group_size = hc->talker->quant_group();
+    out->checkpoint_quant_bits = hc->talker->checkpoint_quant_bits();
     out->weight_dtype = hc->talker->weight_dtype();
     out->num_speakers = (int32_t)c.spk_id.size();
     out->model_type = c.tts_model_type == "voice_design" ? 1 : (c.tts_model_type == "custom_voice" ? 2 : 0);
@@ -1066,27 +1067,64 @@ q3tts_status q3tts_generate_pcm_batch(q3tts_handle* h, const q3tts_request* reqs
 }
 
 // =================================================================================================== parity probes
+namespace {
+
+// The widths and groups the packed probes take, checked on the host before any device is touched.  The container's words must not
+// straddle a group (group % codes-per-word); 2 / 3 / 5 / 6-bit rows must be whole words (in % 32) and use MLX's groups.
+void check_packed_args(int out_f, int in_f, int group, int bits) {
+  const int cbits = container_bits(bits);
+  Q3_CHECK(cbits != 0, Q3TTS_ERR_INVALID_ARG, "bits %d: 2, 3, 4, 5, 6 or 8 are supported", bits);
+  Q3_CHECK(out_f > 0 && in_f > 0 && group > 0 && in_f % group == 0 && group % (32 / cbits) == 0, Q3TTS_ERR_INVALID_ARG,
+           "unsupported bits/group/shape (%d/%d, %d x %d)", bits, group, out_f, in_f);
+  if (cbits != bits)
+    Q3_CHECK((group == 32 || group == 64 || group == 128) && in_f % 32 == 0, Q3TTS_ERR_INVALID_ARG,
+             "%d-bit rows need group_size 32, 64 or 128 and in_features %% 32 == 0 (group %d, in %d)", bits, group, in_f);
+}
+
+// `packed` ([out_f][in_f * bits / 32] uint32 on the host) on the device in the container_bits(bits) word layout the kernels read.
+const uint32_t* upload_packed(const uint32_t* packed, int out_f, int in_f, int bits, std::vector<void*>& allocs) {
+  auto dev = [&](size_t bytes) -> void* {
+    void* d = nullptr;
+    Q3_CUDA(cudaMalloc(&d, bytes));
+    allocs.push_back(d);
+    return d;
+  };
+  const int cbits = container_bits(bits);
+  void* raw = dev((size_t)out_f * in_f * bits / 8);
+  Q3_CUDA(cudaMemcpy(raw, packed, (size_t)out_f * in_f * bits / 8, cudaMemcpyHostToDevice));
+  if (cbits == bits) return (const uint32_t*)raw;
+  uint32_t* wide = (uint32_t*)dev((size_t)out_f * in_f * cbits / 8);
+  LaunchCtx c{nullptr, nullptr};
+  launch_widen_bits(c, (const uint32_t*)raw, out_f, in_f, bits, wide);
+  return wide;
+}
+
+}  // namespace
+
 q3tts_status q3tts_dequantize(int32_t device, const uint32_t* packed, const void* scales, const void* biases, int32_t scale_dtype,
                               int32_t out_f, int32_t in_f, int32_t group, int32_t bits, int32_t out_dtype, void* out) {
+  std::vector<void*> allocs;
   try {
     Q3_CHECK(packed && scales && biases && out, Q3TTS_ERR_INVALID_ARG, "NULL argument");
-    Q3_CHECK((bits == 4 || bits == 8) && group > 0 && in_f % group == 0 && group % (32 / bits) == 0, Q3TTS_ERR_INVALID_ARG,
-             "unsupported bits/group (%d/%d)", bits, group);
+    check_packed_args(out_f, in_f, group, bits);
     require_device(device);
-    const size_t wbytes = (size_t)out_f * in_f * bits / 8, sbytes = (size_t)out_f * (in_f / group) * dtype_size(scale_dtype);
+    const size_t sbytes = (size_t)out_f * (in_f / group) * dtype_size(scale_dtype);
     const size_t obytes = (size_t)out_f * in_f * dtype_size(out_dtype);
-    void *dw = nullptr, *ds = nullptr, *db = nullptr, *dout = nullptr;
-    Q3_CUDA(cudaMalloc(&dw, wbytes)); Q3_CUDA(cudaMalloc(&ds, sbytes)); Q3_CUDA(cudaMalloc(&db, sbytes)); Q3_CUDA(cudaMalloc(&dout, obytes));
-    Q3_CUDA(cudaMemcpy(dw, packed, wbytes, cudaMemcpyHostToDevice));
+    const uint32_t* dw = upload_packed(packed, out_f, in_f, bits, allocs);
+    void *ds = nullptr, *db = nullptr, *dout = nullptr;
+    Q3_CUDA(cudaMalloc(&ds, sbytes)); allocs.push_back(ds);
+    Q3_CUDA(cudaMalloc(&db, sbytes)); allocs.push_back(db);
+    Q3_CUDA(cudaMalloc(&dout, obytes)); allocs.push_back(dout);
     Q3_CUDA(cudaMemcpy(ds, scales, sbytes, cudaMemcpyHostToDevice));
     Q3_CUDA(cudaMemcpy(db, biases, sbytes, cudaMemcpyHostToDevice));
     LaunchCtx c{nullptr, nullptr};
-    launch_dequantize(c, (const uint32_t*)dw, ds, db, scale_dtype, out_f, in_f, group, bits, out_dtype, dout);
+    launch_dequantize(c, dw, ds, db, scale_dtype, out_f, in_f, group, container_bits(bits), out_dtype, dout);
     Q3_CUDA(cudaDeviceSynchronize());
     Q3_CUDA(cudaMemcpy(out, dout, obytes, cudaMemcpyDeviceToHost));
-    cudaFree(dw); cudaFree(ds); cudaFree(db); cudaFree(dout);
+    for (void* d : allocs) cudaFree(d);
     return Q3TTS_OK;
   } catch (const Error& e) {
+    for (void* d : allocs) cudaFree(d);
     g_create_error = e.what();
     cudaGetLastError();
     return e.status;
@@ -1122,36 +1160,40 @@ q3tts_status q3tts_mlx_quantize(int32_t device, const void* w, int32_t w_dtype, 
 q3tts_status q3tts_quantized_matmul(int32_t device, const float* x, int32_t m, const uint32_t* packed, const void* scales,
                                     const void* biases, int32_t scale_dtype, int32_t out_f, int32_t in_f, int32_t group,
                                     int32_t bits, float* y) {
+  std::vector<void*> allocs;
   try {
     Q3_CHECK(x && packed && y && m > 0, Q3TTS_ERR_INVALID_ARG, "NULL argument");
+    if (bits) {
+      Q3_CHECK(scales && biases, Q3TTS_ERR_INVALID_ARG, "NULL scales/biases");
+      check_packed_args(out_f, in_f, group, bits);
+    }
     require_device(device);
     q3::init_talker_kernels();
     Linear L;
-    L.out = out_f; L.in = in_f; L.bits = bits; L.group = group; L.sdt = scale_dtype;
-    const size_t wbytes = bits ? (size_t)out_f * in_f * bits / 8 : (size_t)out_f * in_f * dtype_size(scale_dtype);
-    const size_t sbytes = bits ? (size_t)out_f * (in_f / group) * dtype_size(scale_dtype) : 0;
-    void *dw = nullptr, *ds = nullptr, *db = nullptr;
-    float *dx = nullptr, *dy = nullptr;
-    Q3_CUDA(cudaMalloc(&dw, wbytes));
-    Q3_CUDA(cudaMemcpy(dw, packed, wbytes, cudaMemcpyHostToDevice));
+    L.out = out_f; L.in = in_f; L.bits = container_bits(bits); L.group = group; L.sdt = scale_dtype;
+    auto dev = [&](const void* src, size_t bytes) -> void* {
+      void* d = nullptr;
+      Q3_CUDA(cudaMalloc(&d, bytes));
+      allocs.push_back(d);
+      if (src) Q3_CUDA(cudaMemcpy(d, src, bytes, cudaMemcpyHostToDevice));
+      return d;
+    };
     if (bits) {
-      Q3_CHECK(scales && biases, Q3TTS_ERR_INVALID_ARG, "NULL scales/biases");
-      Q3_CUDA(cudaMalloc(&ds, sbytes)); Q3_CUDA(cudaMalloc(&db, sbytes));
-      Q3_CUDA(cudaMemcpy(ds, scales, sbytes, cudaMemcpyHostToDevice));
-      Q3_CUDA(cudaMemcpy(db, biases, sbytes, cudaMemcpyHostToDevice));
-      L.qw = (const uint32_t*)dw; L.scales = ds; L.biases = db;
+      const size_t sbytes = (size_t)out_f * (in_f / group) * dtype_size(scale_dtype);
+      L.qw = upload_packed(packed, out_f, in_f, bits, allocs); L.scales = dev(scales, sbytes); L.biases = dev(biases, sbytes);
     } else {
-      L.w = dw;
+      L.w = dev(packed, (size_t)out_f * in_f * dtype_size(scale_dtype));
     }
-    Q3_CUDA(cudaMalloc(&dx, (size_t)m * in_f * 4)); Q3_CUDA(cudaMalloc(&dy, (size_t)m * out_f * 4));
-    Q3_CUDA(cudaMemcpy(dx, x, (size_t)m * in_f * 4, cudaMemcpyHostToDevice));
+    float* dx = (float*)dev(x, (size_t)m * in_f * 4);
+    float* dy = (float*)dev(nullptr, (size_t)m * out_f * 4);
     LaunchCtx c{nullptr, nullptr};
     launch_linear(c, L, dx, in_f, m, dy, out_f, nullptr, 0.f, EPI_STORE);
     Q3_CUDA(cudaDeviceSynchronize());
     Q3_CUDA(cudaMemcpy(y, dy, (size_t)m * out_f * 4, cudaMemcpyDeviceToHost));
-    cudaFree(dw); cudaFree(ds); cudaFree(db); cudaFree(dx); cudaFree(dy);
+    for (void* d : allocs) cudaFree(d);
     return Q3TTS_OK;
   } catch (const Error& e) {
+    for (void* d : allocs) cudaFree(d);
     g_create_error = e.what();
     cudaGetLastError();
     return e.status;
@@ -1164,10 +1206,11 @@ q3tts_status q3tts_quantized_matmul_tc(int32_t device, const float* x, int32_t m
   std::vector<void*> allocs;
   try {
     Q3_CHECK(x && packed && scales && biases && y && m > 0 && m <= 128, Q3TTS_ERR_INVALID_ARG, "bad arguments (1 <= m <= 128)");
+    check_packed_args(out_f, in_f, group, bits);
     require_device(device);
     init_tc_gemm();
     const int n_out = swiglu_halves ? out_f / 2 : out_f;
-    const size_t wbytes = (size_t)out_f * in_f * bits / 8, sbytes = (size_t)out_f * (in_f / group) * dtype_size(scale_dtype);
+    const size_t sbytes = (size_t)out_f * (in_f / group) * dtype_size(scale_dtype);
     auto dev = [&](const void* src, size_t bytes) -> void* {
       void* d = nullptr;
       Q3_CUDA(cudaMalloc(&d, std::max<size_t>(bytes, 16)));
@@ -1175,7 +1218,8 @@ q3tts_status q3tts_quantized_matmul_tc(int32_t device, const float* x, int32_t m
       if (src) Q3_CUDA(cudaMemcpy(d, src, bytes, cudaMemcpyHostToDevice));
       return d;
     };
-    void *dw = dev(packed, wbytes), *ds = dev(scales, sbytes), *db = dev(biases, sbytes);
+    const void* dw = upload_packed(packed, out_f, in_f, bits, allocs);
+    void *ds = dev(scales, sbytes), *db = dev(biases, sbytes);
     float* dx = (float*)dev(x, (size_t)m * in_f * 4);
     float* dfold = fold ? (float*)dev(fold, (size_t)in_f * 4) : nullptr;
     float* dy = (float*)dev(residual, (size_t)m * n_out * 4);
@@ -1187,7 +1231,8 @@ q3tts_status q3tts_quantized_matmul_tc(int32_t device, const float* x, int32_t m
     Q3_CUDA(cudaDeviceSynchronize());
     TcGemm g;
     g.a = dx16; g.Bt = 1; g.T = m; g.cin = in_f; g.N = out_f; g.swiglu = swiglu_halves ? 1 : 0;
-    g.q_w = (const uint32_t*)dw; g.q_scales = ds; g.q_biases = db; g.q_fold = dfold; g.q_bits = bits; g.q_group = group; g.q_sdt = scale_dtype;
+    g.q_w = (const uint32_t*)dw; g.q_scales = ds; g.q_biases = db; g.q_fold = dfold; g.q_bits = container_bits(bits); g.q_group = group;
+    g.q_sdt = scale_dtype;
     g.q_halves = swiglu_halves ? 1 : 0;
     g.out32 = dy; g.ld32 = n_out;
     if (residual) { g.res = dy; g.ld_res = n_out; }

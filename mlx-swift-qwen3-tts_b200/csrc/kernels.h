@@ -33,6 +33,15 @@ void launch_mlx_quantize(const LaunchCtx& c, const void* w, int wdt, int out, in
 void launch_dequantize(const LaunchCtx& c, const uint32_t* qw, const void* scales, const void* biases, int sdt, int out,
                        int in, int group, int bits, int out_dt, void* dst);
 
+// The word width the kernels read a b-bit MLX checkpoint in: 2 / 3 / 4 bits -> 4-bit words, 5 / 6 / 8 bits -> 8-bit words, 0 = a width
+// MLX does not write.  Codes are copied unchanged, so dequantised values do not depend on the container.
+inline int container_bits(int bits) {
+  return (bits == 2 || bits == 3 || bits == 4) ? 4 : ((bits == 5 || bits == 6 || bits == 8) ? 8 : 0);
+}
+// src: [rows][in * bits / 32] uint32 of MLX's b-bit bit stream (bits 2, 3, 5, 6; in % 32 == 0) -> dst: [rows][in * cb / 32] uint32 in the
+// container_bits(bits) = cb word layout of launch_dequantize / launch_linear.  Scales and biases are untouched.
+void launch_widen_bits(const LaunchCtx& c, const uint32_t* src, int rows, int in, int bits, uint32_t* dst);
+
 // y[m][*] (op)= epilogue( rmsnorm?(x[m][:]) . W^T + bias ).   x, y fp32 with row strides ldx / ldy.
 // norm_w != null fuses Qwen3RMSNorm (Model/Qwen3Layers.swift:18-25) into the prologue.
 // EPI_SWIGLU: W rows are [gate ; up]; y[m][r] = silu(gate_r) * up_r, r < out/2 (Model/Qwen3Layers.swift:236).

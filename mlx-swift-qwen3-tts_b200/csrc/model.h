@@ -104,6 +104,7 @@ struct TalkerWeights {
   std::vector<TcLinear> lm_head_tc;
   bool has_tc = false;
   size_t talker_step_bytes = 0, cp_pass_bytes = 0;  // algorithmic weight bytes per invocation
+  int checkpoint_bits = 0;  // width of the packed leaves on disk (2..8), 0 = dense; the kernels read 4 / 8-bit words (Linear::bits)
 };
 
 // Loads `model.safetensors` with the key remap of Qwen3Talker.load (Model/Qwen3Talker.swift:117-137).

@@ -49,6 +49,40 @@ void launch_dequantize(const LaunchCtx& c, const uint32_t* qw, const void* scale
   c.tick();
 }
 
+// ------------------------------------------------------------------------------------------------ b-bit rows -> 4/8-bit container
+// MLX stores a row of b-bit codes as one little-endian, LSB-first bit stream: code j at bits [j*b, (j+1)*b) of the row.  One thread
+// builds one container word (8 codes of 4 bits or 4 codes of 8 bits); their source bits span at most 24 bits starting anywhere in a
+// word, so two consecutive source words always hold them.  The second word is read only while it is inside the row, so the last word
+// of the last row never reads past the allocation.
+__global__ void widen_bits_kernel(const uint32_t* __restrict__ src, size_t rows, int in, int bits, int cbits, uint32_t* __restrict__ dst) {
+  const int per = 32 / cbits;
+  const int src_words = in / 32 * bits, dst_words = in / per;
+  const uint32_t mask = (1u << bits) - 1u;
+  const size_t total = rows * (size_t)dst_words;
+  for (size_t wi = (size_t)blockIdx.x * blockDim.x + threadIdx.x; wi < total; wi += (size_t)gridDim.x * blockDim.x) {
+    const size_t row = wi / dst_words;
+    const int col0 = (int)(wi - row * dst_words) * per;
+    const uint32_t* s = src + row * src_words;
+    const int bit0 = col0 * bits, w0 = bit0 >> 5;
+    uint64_t v = s[w0];
+    if (w0 + 1 < src_words) v |= (uint64_t)s[w0 + 1] << 32;
+    v >>= bit0 & 31;
+    uint32_t out = 0;
+    for (int j = 0; j < per; ++j) out |= (uint32_t)((v >> (j * bits)) & mask) << (j * cbits);
+    dst[wi] = out;
+  }
+}
+
+void launch_widen_bits(const LaunchCtx& c, const uint32_t* src, int rows, int in, int bits, uint32_t* dst) {
+  const int cbits = container_bits(bits);
+  Q3_CHECK((bits == 2 || bits == 3 || bits == 5 || bits == 6) && in > 0 && in % 32 == 0 && rows > 0, Q3TTS_ERR_INVALID_ARG,
+           "widen_bits: bits %d / in %d unsupported (bits 2, 3, 5 or 6, in a multiple of 32)", bits, in);
+  const size_t words = (size_t)rows * in * cbits / 32;
+  const int blocks = (int)std::max<size_t>(1, std::min<size_t>((words + 255) / 256, 148 * 16));
+  widen_bits_kernel<<<blocks, 256, 0, c.stream>>>(src, (size_t)rows, in, bits, cbits, dst);
+  c.tick();
+}
+
 // ------------------------------------------------------------------------------------------------ runtime quantisation
 // MLX `quantize(w, group_size: 64, bits)` (affine), one thread per group of 64 weights, restated operation for operation from
 // oracle/mlx_quant.py:quantize (every fp32 step rounded on its own: no FMA contraction, IEEE division, round-half-even):

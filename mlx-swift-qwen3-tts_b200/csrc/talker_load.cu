@@ -132,6 +132,7 @@ struct Loader {
   // embeddings, q/k/v projections and the heads, 4 bits for the rest; the codes live in an 8-bit container (launch_mlx_quantize)
   bool runtime_quant = false;
   int weight_dtype = -1;
+  int ckpt_bits = 0;  // width of the packed leaves on disk (q3tts_info.checkpoint_quant_bits)
   static bool six_bit(const std::string& path) {
     std::string p = path;
     for (char& ch : p) ch = (char)tolower((unsigned char)ch);
@@ -192,13 +193,30 @@ struct Loader {
     const STensor& w0 = get(prefixes[0] + ".weight");
     const bool is_packed = (w0.dtype == "U32" || w0.dtype == "I32") && has(prefixes[0] + ".scales");
     if (is_packed) {
-      Q3_CHECK(bits == 4 || bits == 8, Q3TTS_ERR_BAD_CONFIG,
-               "packed weights with bits=%d: only MLX affine 4/8-bit are in scope", bits);
+      const int cbits = container_bits(bits);
+      Q3_CHECK(cbits != 0, Q3TTS_ERR_BAD_CONFIG, "packed weights with bits=%d: MLX affine checkpoints of 2, 3, 4, 5, 6 or 8 bits are supported", bits);
+      const bool widen = cbits != bits;  // 2/3/5/6-bit rows are re-laid into the 4/8-bit words every kernel reads
+      if (widen) {
+        Q3_CHECK(group == 32 || group == 64 || group == 128, Q3TTS_ERR_BAD_CONFIG, "%d-bit checkpoint with group_size %d: 32, 64 or 128 are supported",
+                 bits, group);
+        Q3_CHECK(in % group == 0 && in % 32 == 0, Q3TTS_ERR_BAD_CONFIG, "%d-bit checkpoint: in_features %d must be a multiple of 32 and of group_size %d",
+                 bits, in, group);
+      }
       Q3_CHECK(in % group == 0, Q3TTS_ERR_BAD_WEIGHTS, "in_features %d not a multiple of group_size %d", in, group);
+      ckpt_bits = bits;
       const size_t row_words = (size_t)in * bits / 32, row_groups = (size_t)in / group;
       const int sdt = get(prefixes[0] + ".scales").q3_dtype();
       const size_t ssz = dtype_size(sdt);
-      uint32_t* qw = (uint32_t*)arena.alloc((size_t)L.out * row_words * 4);
+      // the raw rows go straight into the arena, or into a temporary that is widened into it
+      uint32_t* qw = (uint32_t*)arena.alloc((size_t)L.out * in * cbits / 8);
+      uint32_t* raw = qw;
+      std::unique_ptr<void, cudaError_t (*)(void*)> raw_tmp(nullptr, cudaFree);
+      if (widen) {
+        void* p = nullptr;
+        Q3_CUDA(cudaMalloc(&p, (size_t)L.out * row_words * 4));
+        raw_tmp.reset(p);
+        raw = (uint32_t*)p;
+      }
       char* sc = (char*)arena.alloc((size_t)L.out * row_groups * ssz);
       char* bi = (char*)arena.alloc((size_t)L.out * row_groups * ssz);
       size_t r0 = 0;
@@ -216,20 +234,25 @@ struct Loader {
         const size_t wbytes = (size_t)outs[i] * row_words * 4, sbytes = (size_t)outs[i] * row_groups * ssz;
         Q3_CHECK((w.dtype == "U32" || w.dtype == "I32") && w.nbytes == wbytes && s.nbytes == sbytes && b.nbytes == sbytes, Q3TTS_ERR_BAD_WEIGHTS,
                  "packed leaf '%s' has the wrong dtype or byte size", prefixes[i].c_str());
-        Q3_CUDA(cudaMemcpyAsync(qw + r0 * row_words, w.data, wbytes, cudaMemcpyHostToDevice, stream));
+        Q3_CUDA(cudaMemcpyAsync(raw + r0 * row_words, w.data, wbytes, cudaMemcpyHostToDevice, stream));
         Q3_CUDA(cudaMemcpyAsync(sc + r0 * row_groups * ssz, s.data, sbytes, cudaMemcpyHostToDevice, stream));
         Q3_CUDA(cudaMemcpyAsync(bi + r0 * row_groups * ssz, b.data, sbytes, cudaMemcpyHostToDevice, stream));
         r0 += outs[i];
       }
+      if (widen) {
+        LaunchCtx lc{stream, nullptr};
+        launch_widen_bits(lc, raw, L.out, in, bits, qw);
+        Q3_CUDA(cudaStreamSynchronize(stream));  // raw_tmp is freed when it leaves scope
+      }
       if (weight_dtype < 0) weight_dtype = sdt;
       if (packed) {
-        L.bits = bits; L.group = group; L.sdt = sdt; L.qw = qw; L.scales = sc; L.biases = bi;
+        L.bits = cbits; L.group = group; L.sdt = sdt; L.qw = qw; L.scales = sc; L.biases = bi;
       } else {
         // offline `dequantized(..., dtype: .float16)` (Qwen3Talker.swift:156-164) with the bit-exact kernel
         Q3_CHECK(offline_dequant, Q3TTS_ERR_BAD_CONFIG, "packed weights found but config.json has neither `quantization` nor `quantization_config`");
         __half* dense = (__half*)arena.alloc((size_t)L.out * in * 2);
         LaunchCtx lc{stream, nullptr};
-        launch_dequantize(lc, qw, sc, bi, sdt, L.out, in, group, bits, Q3TTS_F16, dense);
+        launch_dequantize(lc, qw, sc, bi, sdt, L.out, in, group, cbits, Q3TTS_F16, dense);
         L.bits = 0; L.sdt = Q3TTS_F16; L.w = dense;
         weight_dtype = Q3TTS_F16;  // what the handle computes with after the load (q3tts_info.weight_dtype)
       }
@@ -351,6 +374,7 @@ void load_talker_weights(const std::string& model_dir, const TalkerConfig& cfg, 
 
   out.talker_step_bytes = stack_bytes(out.talker) + out.codec_head.weight_bytes();
   out.cp_pass_bytes = stack_bytes(out.cp) + out.lm_head[0].weight_bytes() + (out.has_mtp ? out.small_to_mtp.weight_bytes() : 0);
+  out.checkpoint_bits = L.ckpt_bits;
   weight_dtype = L.weight_dtype < 0 ? Q3TTS_BF16 : L.weight_dtype;
   eff_bits = out.talker.layer[0].qkv.bits;
   eff_group = group;

@@ -36,7 +36,7 @@ class Info(C.Structure):
                                    "num_speakers", "has_codec", "codec_num_quantizers", "codec_total_upsample", "model_type",
                                    "codec_eos_id", "codec_pad_id", "max_batch", "kv_capacity", "max_frames")] + \
                [("device_bytes", i64), ("has_audio_encoder", i32), ("audio_encoder_hidden", i32), ("has_speaker_encoder", i32), ("speaker_embedding_dim", i32),
-                ("reserved", i32 * 4)]
+                ("checkpoint_quant_bits", i32), ("reserved", i32 * 3)]
 
 
 class Request(C.Structure):
