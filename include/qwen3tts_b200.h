@@ -298,6 +298,35 @@ q3tts_status q3tts_quantized_matmul_tc(int32_t device, const float* x, int32_t m
 q3tts_status q3tts_sample_token(q3tts_handle* h, const float* logits, int32_t vocab, float temperature, int32_t top_k,
                                 float top_p, float repetition_penalty, const int32_t* token_set, int32_t n_token_set,
                                 uint64_t seed, uint64_t counter, int32_t* id_out);
+/* The engine's device sampler (sampleToken, Model/Qwen3Talker.swift:274-322) on n_rows rows, one CTA per row, on host buffers.
+ * form: 0 = the 512-thread form the CUDA-graph path and q3tts_sample_token run, 1 = the form of the persistent frame kernel (named
+ * barrier 1 over warps 0-14 of a 512-thread CTA).  logits [n_rows][ld] fp32, V entries per row (ld = 0: every row reads row 0).
+ * Per row r: temperature, top_k, top_p, repetition_penalty, seed and counter (the position in the sampler stream); token_sets
+ * [n_rows][128] uint32 bitmaps (bit i % 32 of word i / 32 = id i is in the set) or NULL.  The valid-id mask applies when V == codec_vocab.
+ * ids_out [n_rows]; processed_out [n_rows][V] or NULL: the row just before the Gumbel step (for greedy rows, right after the penalty),
+ * -inf where removed.  1 <= V <= 4096, 1 <= n_rows <= 65535, ld = 0 or >= V, temperature / top_p / repetition_penalty finite and
+ * top_p > 0; anything else returns Q3TTS_ERR_INVALID_ARG without touching the device. */
+q3tts_status q3tts_sampler_probe(int32_t device, int32_t form, const float* logits, int32_t n_rows, int32_t V, int32_t ld, int32_t codec_vocab,
+                                 const float* temperature, const int32_t* top_k, const float* top_p, const float* repetition_penalty,
+                                 const uint32_t* token_sets, const uint64_t* seed, const uint64_t* counter, int32_t* ids_out,
+                                 float* processed_out);
+/* One sampling point of one group for n_slots slots, with the generation loop's per-slot rules, as the engine runs it: form 0 = the
+ * sampler launch of the CUDA-graph path, 1 = the form of the persistent frame kernel.  group 0 = code0 (EOS / pad suppressed while
+ * trailing_idx < total_text, the EOS and 7-pad stops unless the slot is forced, max_tokens, sets frame_alive); group g >= 1 = code-predictor
+ * group g - 1 (nothing unless frame_alive; the id is added to the slot's set of group g; stream_variant drops the penalty).
+ * logits [n_slots][V].  Slot state, one int32 array of n_slots per field, in/out: active, finished, step, max_tokens, trailing_idx,
+ * total_text, consecutive_pad, n_forced, stream_variant, frame_alive, logits_cap.  Sampling fields per slot: temperature, top_k,
+ * top_p, repetition_penalty, seed (the counter is step * 16 + group).  token_sets [n_slots][16][set_words] in/out (set_words * 32 >= V);
+ * forced [n_slots][max_frames][16] or NULL (read when n_forced > 0); cur_codes [n_slots][16] in/out (a sampled slot writes [s][group]).
+ * dump [dump_frames][V] or NULL: slot dump_slot's raw logits land in row `step` while step < logits_cap.  Arguments are validated on
+ * the host (see q3tts_sampler_probe; also step >= 0, step < max_frames for forced slots, logits_cap[dump_slot] <= dump_frames). */
+q3tts_status q3tts_sampler_slot_probe(int32_t device, int32_t form, int32_t group, int32_t n_slots, int32_t V, int32_t codec_vocab, int32_t eos_id,
+                                      int32_t pad_id, const float* logits, int32_t* active, int32_t* finished, int32_t* step, int32_t* max_tokens,
+                                      int32_t* trailing_idx, int32_t* total_text, int32_t* consecutive_pad, int32_t* n_forced,
+                                      int32_t* stream_variant, int32_t* frame_alive, int32_t* logits_cap, const float* temperature,
+                                      const int32_t* top_k, const float* top_p, const float* repetition_penalty, const uint64_t* seed,
+                                      uint32_t* token_sets, int32_t set_words, const int32_t* forced, int32_t max_frames, float* dump,
+                                      int32_t dump_slot, int32_t dump_frames, int32_t* cur_codes);
 /* SplitResidualVectorQuantizer code -> embedding lookup (Vocoder/SpeechTokenizer.swift:504-506, 566-582, 684-691),
  * bit-exact contract: fp32 gather-sum in codebook order.  codes [B][F][16]; first_out/rest_out [B][F][dim] fp32
  * (rvq_first and rvq_rest sums before their 1x1 output projections). */

@@ -3,6 +3,7 @@
 #include <atomic>
 #include <deque>
 #include <chrono>
+#include <cmath>
 #include <map>
 #include <thread>
 
@@ -13,6 +14,7 @@
 #include "codec_unit.h"
 #include "engine.h"
 #include "gemm_tc.h"
+#include "sampler.cuh"
 #include "tc_ptx.cuh"
 
 using namespace q3;
@@ -1679,6 +1681,135 @@ q3tts_status q3tts_codec_rowop_probe(int32_t device, int32_t op, const float* x,
       Q3_CUDA(cudaGetLastError());
       Q3_CUDA(cudaDeviceSynchronize());
       Q3_CUDA(cudaMemcpy(y, dy, ny * 4, cudaMemcpyDeviceToHost));
+    }
+    return Q3TTS_OK;
+  } catch (const Error& e) {
+    return probe_failed(e);
+  }
+}
+
+// ------------------------------------------------------------------------------------------------ sampler probes
+namespace {
+void* upload(ProbeBuffers& buf, const void* src, size_t bytes) {
+  void* d = buf.alloc(bytes);
+  Q3_CUDA(cudaMemcpy(d, src, bytes, cudaMemcpyHostToDevice));
+  return d;
+}
+// the per-row (or per-slot) sampling fields the sampler reads: a non-finite value or top_p <= 0 has no meaning in sampleToken
+void check_sampling_fields(int n, const float* temperature, const float* top_p, const float* rep_penalty) {
+  for (int r = 0; r < n; ++r)
+    Q3_CHECK(std::isfinite(temperature[r]) && std::isfinite(top_p[r]) && std::isfinite(rep_penalty[r]) && top_p[r] > 0.f, Q3TTS_ERR_INVALID_ARG,
+             "row %d: temperature %g, top_p %g, repetition_penalty %g (finite, top_p > 0)", r, temperature[r], top_p[r], rep_penalty[r]);
+}
+}  // namespace
+
+q3tts_status q3tts_sampler_probe(int32_t device, int32_t form, const float* logits, int32_t n_rows, int32_t V, int32_t ld, int32_t codec_vocab,
+                                 const float* temperature, const int32_t* top_k, const float* top_p, const float* repetition_penalty,
+                                 const uint32_t* token_sets, const uint64_t* seed, const uint64_t* counter, int32_t* ids_out,
+                                 float* processed_out) {
+  ProbeBuffers buf;
+  try {
+    Q3_CHECK(logits && temperature && top_k && top_p && repetition_penalty && seed && counter && ids_out, Q3TTS_ERR_INVALID_ARG, "NULL argument");
+    Q3_CHECK(form == 0 || form == 1, Q3TTS_ERR_INVALID_ARG, "form must be 0 (sample_kernel) or 1 (frame kernel)");
+    Q3_CHECK(V >= 1 && V <= kMaxVocab, Q3TTS_ERR_INVALID_ARG, "V %d outside 1..%d", V, kMaxVocab);
+    Q3_CHECK(n_rows >= 1 && n_rows <= 65535, Q3TTS_ERR_INVALID_ARG, "n_rows %d outside 1..65535", n_rows);
+    Q3_CHECK(ld == 0 || ld >= V, Q3TTS_ERR_INVALID_ARG, "ld %d (0 or >= V %d)", ld, V);
+    check_sampling_fields(n_rows, temperature, top_p, repetition_penalty);
+    const size_t n_logits = ld == 0 ? (size_t)V : (size_t)(n_rows - 1) * ld + V;
+    Q3_CHECK(n_logits < kProbeMaxElems && (size_t)n_rows * V < kProbeMaxElems, Q3TTS_ERR_INVALID_ARG, "logits too large");
+    require_device(device);
+    LaunchCtx c{nullptr, nullptr};
+    SamplerProbeRows rows;
+    rows.temperature = (const float*)upload(buf, temperature, (size_t)n_rows * 4);
+    rows.top_k = (const int*)upload(buf, top_k, (size_t)n_rows * 4);
+    rows.top_p = (const float*)upload(buf, top_p, (size_t)n_rows * 4);
+    rows.rep_penalty = (const float*)upload(buf, repetition_penalty, (size_t)n_rows * 4);
+    rows.sets = token_sets ? (const unsigned*)upload(buf, token_sets, (size_t)n_rows * kMaxVocab / 8) : nullptr;
+    rows.seed = (const unsigned long long*)upload(buf, seed, (size_t)n_rows * 8);
+    rows.counter = (const unsigned long long*)upload(buf, counter, (size_t)n_rows * 8);
+    const float* dl = (const float*)upload(buf, logits, n_logits * 4);
+    int* dids = (int*)buf.alloc((size_t)n_rows * 4);
+    float* dproc = nullptr;
+    if (processed_out) {
+      dproc = buf.f32(nullptr, (size_t)n_rows * V);
+      Q3_CUDA(cudaMemset(dproc, 0x7f, (size_t)n_rows * V * 4));  // an entry the dump does not write reads as 3.4e38
+    }
+    launch_sampler_probe(c, form, dl, ld, n_rows, V, codec_vocab, rows, dids, dproc);
+    Q3_CUDA(cudaGetLastError());
+    Q3_CUDA(cudaDeviceSynchronize());
+    Q3_CUDA(cudaMemcpy(ids_out, dids, (size_t)n_rows * 4, cudaMemcpyDeviceToHost));
+    if (processed_out) Q3_CUDA(cudaMemcpy(processed_out, dproc, (size_t)n_rows * V * 4, cudaMemcpyDeviceToHost));
+    return Q3TTS_OK;
+  } catch (const Error& e) {
+    return probe_failed(e);
+  }
+}
+
+q3tts_status q3tts_sampler_slot_probe(int32_t device, int32_t form, int32_t group, int32_t n_slots, int32_t V, int32_t codec_vocab, int32_t eos_id,
+                                      int32_t pad_id, const float* logits, int32_t* active, int32_t* finished, int32_t* step, int32_t* max_tokens,
+                                      int32_t* trailing_idx, int32_t* total_text, int32_t* consecutive_pad, int32_t* n_forced,
+                                      int32_t* stream_variant, int32_t* frame_alive, int32_t* logits_cap, const float* temperature,
+                                      const int32_t* top_k, const float* top_p, const float* repetition_penalty, const uint64_t* seed,
+                                      uint32_t* token_sets, int32_t set_words, const int32_t* forced, int32_t max_frames, float* dump,
+                                      int32_t dump_slot, int32_t dump_frames, int32_t* cur_codes) {
+  ProbeBuffers buf;
+  try {
+    int32_t* const fields[] = {active, finished, step, max_tokens, trailing_idx, total_text, consecutive_pad, n_forced, stream_variant, frame_alive,
+                               logits_cap};
+    for (int32_t* f : fields) Q3_CHECK(f, Q3TTS_ERR_INVALID_ARG, "NULL slot-state field");
+    Q3_CHECK(logits && temperature && top_k && top_p && repetition_penalty && seed && token_sets && cur_codes, Q3TTS_ERR_INVALID_ARG, "NULL argument");
+    Q3_CHECK(form == 0 || form == 1, Q3TTS_ERR_INVALID_ARG, "form must be 0 (sample_kernel) or 1 (frame kernel)");
+    Q3_CHECK(group >= 0 && group < 16, Q3TTS_ERR_INVALID_ARG, "group %d outside 0..15", group);
+    Q3_CHECK(V >= 1 && V <= kMaxVocab, Q3TTS_ERR_INVALID_ARG, "V %d outside 1..%d", V, kMaxVocab);
+    Q3_CHECK(n_slots >= 1 && n_slots <= 4096, Q3TTS_ERR_INVALID_ARG, "n_slots %d outside 1..4096", n_slots);
+    Q3_CHECK(set_words >= (V + 31) / 32 && set_words <= kMaxVocab / 32, Q3TTS_ERR_INVALID_ARG, "set_words %d cannot hold ids < %d", set_words, V);
+    check_sampling_fields(n_slots, temperature, top_p, repetition_penalty);
+    Q3_CHECK(!forced || (max_frames >= 1 && max_frames <= 65536), Q3TTS_ERR_INVALID_ARG, "max_frames %d outside 1..65536", max_frames);
+    Q3_CHECK(!dump || (dump_frames >= 0 && dump_frames <= 65536), Q3TTS_ERR_INVALID_ARG, "dump_frames %d outside 0..65536", dump_frames);
+    for (int s = 0; s < n_slots; ++s) {
+      Q3_CHECK(step[s] >= 0, Q3TTS_ERR_INVALID_ARG, "slot %d: step %d < 0", s, step[s]);
+      Q3_CHECK(!forced || n_forced[s] <= 0 || step[s] < max_frames, Q3TTS_ERR_INVALID_ARG, "slot %d: forced ids end at max_frames %d <= step %d", s,
+               max_frames, step[s]);
+    }
+    Q3_CHECK(!dump || (dump_slot >= 0 && dump_slot < n_slots && logits_cap[dump_slot] <= dump_frames), Q3TTS_ERR_INVALID_ARG,
+             "dump: slot %d of %d, logits_cap above dump_frames %d", dump_slot, n_slots, dump_frames);
+    require_device(device);
+    LaunchCtx c{nullptr, nullptr};
+    std::vector<SlotState> st(n_slots);
+    for (int s = 0; s < n_slots; ++s) {
+      SlotState& x = st[s];
+      memset(&x, 0, sizeof(x));
+      x.active = active[s]; x.finished = finished[s]; x.step = step[s]; x.max_tokens = max_tokens[s];
+      x.trailing_idx = trailing_idx[s]; x.total_text = total_text[s]; x.consecutive_pad = consecutive_pad[s]; x.n_forced = n_forced[s];
+      x.stream_variant = stream_variant[s]; x.frame_alive = frame_alive[s]; x.logits_cap = logits_cap[s];
+      x.temperature = temperature[s]; x.top_k = top_k[s]; x.top_p = top_p[s]; x.rep_penalty = repetition_penalty[s]; x.seed = seed[s];
+    }
+    SamplerParams p;
+    p.vocab = V; p.group = group; p.codec_vocab = codec_vocab; p.eos_id = eos_id; p.pad_id = pad_id; p.groups = 16; p.set_words = set_words;
+    const size_t n_set = (size_t)n_slots * 16 * set_words;
+    SlotState* dst = (SlotState*)upload(buf, st.data(), (size_t)n_slots * sizeof(SlotState));
+    unsigned* dsets = (unsigned*)upload(buf, token_sets, n_set * 4);
+    int* dcodes = (int*)upload(buf, cur_codes, (size_t)n_slots * 16 * 4);
+    const int* dforced = forced ? (const int*)upload(buf, forced, (size_t)n_slots * max_frames * 16 * 4) : nullptr;
+    float* ddump = nullptr;
+    if (dump) {
+      ddump = buf.f32(nullptr, (size_t)std::max(dump_frames, 1) * V);
+      Q3_CUDA(cudaMemset(ddump, 0x7f, (size_t)std::max(dump_frames, 1) * V * 4));
+    }
+    const float* dl = (const float*)upload(buf, logits, (size_t)n_slots * V * 4);
+    if (form == 0) launch_sample(c, dl, V, n_slots, dst, p, dsets, dcodes, dforced, max_frames, ddump, V, 0, dump_slot);
+    else launch_sample_frame_form(c, dl, V, n_slots, dst, p, dsets, dcodes, dforced, max_frames, ddump, V, 0, dump_slot);
+    Q3_CUDA(cudaGetLastError());
+    Q3_CUDA(cudaDeviceSynchronize());
+    Q3_CUDA(cudaMemcpy(st.data(), dst, (size_t)n_slots * sizeof(SlotState), cudaMemcpyDeviceToHost));
+    Q3_CUDA(cudaMemcpy(token_sets, dsets, n_set * 4, cudaMemcpyDeviceToHost));
+    Q3_CUDA(cudaMemcpy(cur_codes, dcodes, (size_t)n_slots * 16 * 4, cudaMemcpyDeviceToHost));
+    if (dump && dump_frames > 0) Q3_CUDA(cudaMemcpy(dump, ddump, (size_t)dump_frames * V * 4, cudaMemcpyDeviceToHost));
+    for (int s = 0; s < n_slots; ++s) {
+      const SlotState& x = st[s];
+      active[s] = x.active; finished[s] = x.finished; step[s] = x.step; max_tokens[s] = x.max_tokens; trailing_idx[s] = x.trailing_idx;
+      total_text[s] = x.total_text; consecutive_pad[s] = x.consecutive_pad; n_forced[s] = x.n_forced; stream_variant[s] = x.stream_variant;
+      frame_alive[s] = x.frame_alive; logits_cap[s] = x.logits_cap;
     }
     return Q3TTS_OK;
   } catch (const Error& e) {

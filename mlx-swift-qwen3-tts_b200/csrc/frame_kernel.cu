@@ -26,6 +26,7 @@ namespace {
 
 constexpr int kCWarps = 15;            // consumer warps
 constexpr int kCons = kCWarps * 32;    // 480 consumer threads (named barrier 1)
+static_assert(kCons == kFrameSampleThreads, "q3tts_sampler_probe runs the sampler form of the frame kernel with kFrameSampleThreads");
 constexpr int kMegaThreads = 512;
 constexpr int kKeyTile = 128;          // keys per attention item (host sizes nsplit so that a split never exceeds it)
 constexpr int kKeyGroups = 3;          // P.V key groups: 3 x 128 threads

@@ -150,6 +150,26 @@ void launch_sample_probe(const LaunchCtx& c, const float* logits, int vocab, int
                          float top_p, float rep_penalty, const unsigned* set_bitmap, unsigned long long seed,
                          unsigned long long counter, int* id_out);
 
+// q3tts_sampler_probe: sample_block on rows r < n_rows (logits + r * ld, V entries), one CTA per row, each row with its own
+// parameters (device arrays of n_rows; sets = [n_rows][kMaxVocab / 32] bitmaps or null).  form 0 = the 512-thread form of
+// sample_kernel, 1 = the 480-thread named-barrier form of frame_megakernel.  processed (or null): [n_rows][V], the row just before the
+// Gumbel step (greedy rows: after the penalty).
+struct SamplerProbeRows {
+  const float* temperature;
+  const int* top_k;
+  const float* top_p;
+  const float* rep_penalty;
+  const unsigned* sets;
+  const unsigned long long* seed;
+  const unsigned long long* counter;
+};
+void launch_sampler_probe(const LaunchCtx& c, int form, const float* logits, int ld, int n_rows, int V, int codec_vocab,
+                          const SamplerProbeRows& rows, int* ids, float* processed);
+// launch_sample's work (NextInput mode 0) in the form frame_megakernel's sample_phase runs it: sample_slot<1, 480> (q3tts_sampler_slot_probe)
+void launch_sample_frame_form(const LaunchCtx& c, const float* logits, int ld, int n_slots, SlotState* st, const SamplerParams& p,
+                              unsigned* token_sets, int* cur_codes, const int* forced, int max_frames, float* logits_dump,
+                              int dump_stride_frame, int dump_offset, int dump_slot);
+
 // code-predictor input rows (Model/Qwen3Talker.swift:503-510): pass 0 -> rows (2s, 2s+1) = [h_last[s], codec_embedding[code0]];
 // pass g >= 1 -> row s = cp_codec_embedding[g-1][codes[s][g]]
 void launch_cp_input(const LaunchCtx& c, int pass, int n_slots, const float* h_last, int H, const Embedding& codec,

@@ -32,12 +32,16 @@ __device__ __forceinline__ float counter_uniform(unsigned long long seed, unsign
   x ^= x >> 31;
   return (__uint2float_rn((unsigned)(x >> 41)) + 0.5f) * (1.0f / 8388608.0f);
 }
-__device__ __forceinline__ unsigned ordered_key(float f) {  // monotone float -> uint map
-  const unsigned u = __float_as_uint(f);
+// Monotone float -> uint map.  -0.0 is mapped as +0.0: the thresholds compare floats, for which -0.0 == +0.0, so a signed
+// zero tied at the top-k or top-p threshold survives like any other tie.
+__device__ __forceinline__ unsigned ordered_key(float f) {
+  unsigned u = __float_as_uint(f);
+  if (u == 0x80000000u) u = 0u;
   return (u & 0x80000000u) ? ~u : (u | 0x80000000u);
 }
 
 constexpr int kSampleThreads = 512;
+constexpr int kFrameSampleThreads = 15 * 32;  // frame_megakernel's consumer warps 0-14 run sample_slot<1, kFrameSampleThreads>
 constexpr int kMaxVocab = 4096;
 
 struct BlockRed {
@@ -106,15 +110,21 @@ __device__ float block_max(float v, BlockRed& br) {
 
 // Qwen3Talker.sampleToken (Model/Qwen3Talker.swift:274-322) over sl[0..V) held in shared memory (already carrying
 // the EOS/pad suppression of :470-475 where it applies).  Returns the id to every thread.
-template <int BAR, int NT>
+// DUMP (q3tts_sampler_probe only): processed[0..V) receives the row as it stands just before the Gumbel step -- for a greedy
+// row, right after the penalty.
+template <int BAR, int NT, bool DUMP = false>
 __device__ int sample_block(float* sl, int V, int codec_vocab, float temperature, int top_k, float top_p, float rep_penalty,
-                            const unsigned* set_bitmap, unsigned long long seed, unsigned long long counter, BlockRed& br) {
+                            const unsigned* set_bitmap, unsigned long long seed, unsigned long long counter, BlockRed& br,
+                            float* processed = nullptr) {
   if (set_bitmap != nullptr && rep_penalty != 1.0f) {  // set-based, division regardless of sign (:288-299)
     for (int i = threadIdx.x; i < V; i += NT)
       if (set_bitmap[i >> 5] & (1u << (i & 31))) sl[i] = sl[i] / rep_penalty;
   }
   block_sync<BAR, NT>();
-  if (!(temperature > 0.f)) return block_argmax<BAR, NT>(sl, V, br);  // greedy: before the valid-token mask (:301-305)
+  if (!(temperature > 0.f)) {  // greedy: before the valid-token mask (:301-305)
+    if constexpr (DUMP) for (int i = threadIdx.x; i < V; i += NT) processed[i] = sl[i];
+    return block_argmax<BAR, NT>(sl, V, br);
+  }
   for (int i = threadIdx.x; i < V; i += NT) sl[i] = sl[i] / temperature;
   block_sync<BAR, NT>();
   if (top_k > 0 && top_k < V) {  // threshold = k-th largest; ties at the threshold survive (:307-314)
@@ -156,6 +166,7 @@ __device__ int sample_block(float* sl, int V, int codec_vocab, float temperature
   // MLXRandom.categorical == Gumbel-max (:321)
   for (int i = threadIdx.x; i < V; i += NT) {
     const float l = sl[i];
+    if constexpr (DUMP) processed[i] = l;
     if (l > -INFINITY) {
       const float u = counter_uniform(seed, counter, (unsigned)i);
       sl[i] = l + (-logf(-logf(u)));

@@ -986,6 +986,57 @@ void launch_sample_probe(const LaunchCtx& c, const float* logits, int vocab, int
   c.tick();
 }
 
+// q3tts_sampler_probe / q3tts_sampler_slot_probe.  FORM 0 runs the sampler as sample_kernel does (__syncthreads over 512
+// threads), FORM 1 as frame_megakernel does: named barrier 1 over warps 0-14 of a 512-thread CTA, warp 15 idle.
+template <int FORM>
+constexpr int probe_threads() { return FORM == 0 ? kSampleThreads : kFrameSampleThreads; }
+
+template <int FORM, bool DUMP>
+__global__ void __launch_bounds__(kSampleThreads) sampler_probe_kernel(const float* __restrict__ logits, int ld, int V, int codec_vocab,
+                                                                      SamplerProbeRows rows, int* __restrict__ ids,
+                                                                      float* __restrict__ processed) {
+  constexpr int NT = probe_threads<FORM>();
+  __shared__ float sl[kMaxVocab];
+  __shared__ BlockRed br;
+  if (threadIdx.x >= NT) return;
+  const int r = blockIdx.x;
+  for (int i = threadIdx.x; i < V; i += NT) sl[i] = logits[(size_t)r * ld + i];
+  block_sync<FORM, NT>();
+  const int tok = sample_block<FORM, NT, DUMP>(sl, V, codec_vocab, rows.temperature[r], rows.top_k[r], rows.top_p[r], rows.rep_penalty[r],
+                                               rows.sets ? rows.sets + (size_t)r * (kMaxVocab / 32) : nullptr, rows.seed[r], rows.counter[r],
+                                               br, DUMP ? processed + (size_t)r * V : nullptr);
+  if (threadIdx.x == 0) ids[r] = tok;
+}
+void launch_sampler_probe(const LaunchCtx& c, int form, const float* logits, int ld, int n_rows, int V, int codec_vocab,
+                          const SamplerProbeRows& rows, int* ids, float* processed) {
+  Q3_CHECK(V >= 1 && V <= kMaxVocab && n_rows >= 1 && (form == 0 || form == 1), Q3TTS_ERR_INVALID_ARG, "sampler probe: bad V %d / rows %d / form %d",
+           V, n_rows, form);
+  auto k = form == 0 ? (processed ? sampler_probe_kernel<0, true> : sampler_probe_kernel<0, false>)
+                     : (processed ? sampler_probe_kernel<1, true> : sampler_probe_kernel<1, false>);
+  k<<<n_rows, kSampleThreads, 0, c.stream>>>(logits, ld, V, codec_vocab, rows, ids, processed);
+  c.tick();
+}
+
+__global__ void __launch_bounds__(kSampleThreads) sample_slot_frame_form_kernel(const float* __restrict__ logits, int ld, SlotState* __restrict__ st,
+                                                                               SamplerParams p, unsigned* __restrict__ token_sets,
+                                                                               int* __restrict__ cur_codes, const int* __restrict__ forced,
+                                                                               int max_frames, float* __restrict__ dump, int dump_stride_frame,
+                                                                               int dump_offset, int dump_slot) {
+  __shared__ float sl[kMaxVocab];
+  __shared__ BlockRed br;
+  if (threadIdx.x >= kFrameSampleThreads) return;
+  sample_slot<1, kFrameSampleThreads>(blockIdx.x, logits, ld, st, p, token_sets, cur_codes, forced, max_frames, dump, dump_stride_frame,
+                                      dump_offset, dump_slot, sl, br);
+}
+void launch_sample_frame_form(const LaunchCtx& c, const float* logits, int ld, int n_slots, SlotState* st, const SamplerParams& p,
+                              unsigned* token_sets, int* cur_codes, const int* forced, int max_frames, float* logits_dump,
+                              int dump_stride_frame, int dump_offset, int dump_slot) {
+  Q3_CHECK(p.vocab <= kMaxVocab, Q3TTS_ERR_BAD_CONFIG, "sampler supports vocab <= %d (got %d)", kMaxVocab, p.vocab);
+  sample_slot_frame_form_kernel<<<n_slots, kSampleThreads, 0, c.stream>>>(logits, ld, st, p, token_sets, cur_codes, forced, max_frames,
+                                                                          logits_dump, dump_stride_frame, dump_offset, dump_slot);
+  c.tick();
+}
+
 // ------------------------------------------------------------------------------------------------ frame plumbing
 __global__ void cp_input_kernel(int pass, const float* __restrict__ h_last, int H, Embedding codec, const Embedding* __restrict__ cp_emb,
                                 const int* __restrict__ cur_codes, float* __restrict__ y, int groups) {

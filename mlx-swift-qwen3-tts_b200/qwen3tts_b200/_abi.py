@@ -96,6 +96,9 @@ SYMBOLS = {
     "q3tts_skinny_trace_q": (i32, [i32, i32, i32, i32, i32, i32, i32, i32, C.POINTER(C.c_uint64), i32, C.POINTER(i32), C.POINTER(i32), C.POINTER(i32),
                                    C.POINTER(C.c_double)]),
     "q3tts_sample_token": (i32, [C.c_void_p, p_f32, i32, f32, i32, f32, f32, p_i32, i32, u64, u64, p_i32]),
+    "q3tts_sampler_probe": (i32, [i32, i32, p_f32, i32, i32, i32, i32, p_f32, p_i32, p_f32, p_f32, C.c_void_p, C.c_void_p, C.c_void_p, p_i32, p_f32]),
+    "q3tts_sampler_slot_probe": (i32, [i32, i32, i32, i32, i32, i32, i32, i32, p_f32] + [p_i32] * 11 + [p_f32, p_i32, p_f32, p_f32, C.c_void_p, C.c_void_p, i32,
+                                                                                            p_i32, i32, p_f32, i32, i32, p_i32]),
     "q3tts_rvq_embed": (i32, [C.c_void_p, p_i32, i32, i32, p_f32, p_f32, p_i32]),
     "q3tts_encode_reference_audio": (i32, [C.c_void_p, p_f32, i64, p_i32, i32, p_i32, p_i32, p_f32]),
     "q3tts_extract_speaker_embedding": (i32, [C.c_void_p, p_f32, i64, p_f32, i32, p_i32, p_f32]),

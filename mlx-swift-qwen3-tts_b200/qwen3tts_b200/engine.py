@@ -527,3 +527,53 @@ def codec_rowop_probe(op, x, C, w=None, b=None, eps=1e-6, T=0, device=0):
     y = np.zeros((rows, C), dtype=np.float32)
     A.check(A.lib().q3tts_codec_rowop_probe(device, CODEC_ROWOPS[op], _pf(x), rows, ldx, C, T, _pf(w), _pf(b), eps, _pf(y)), None)
     return y
+
+
+def sampler_probe(form, logits, temperature, top_k, top_p, repetition_penalty, seed, counter, token_sets=None, codec_vocab=0,
+                  want_processed=False, n_rows=None, device=0):
+    """`q3tts_sampler_probe`: the device sampler on each row of logits [n, V] (or one row [V] shared by n_rows rows).  The sampling
+    arguments are scalars or arrays of n; token_sets is [n, 128] uint32 bitmaps or None.  form 0 = sample_kernel's form, 1 = the
+    frame kernel's.  -> (ids int32 [n], processed [n, V] fp32 or None)."""
+    lg = _f32(logits)
+    V = lg.shape[-1]
+    n = lg.shape[0] if lg.ndim == 2 else int(n_rows or 1)
+    ld = V if lg.ndim == 2 else 0
+    row = lambda a, dt: np.ascontiguousarray(np.broadcast_to(np.asarray(a, dtype=dt), (n,)))
+    t, k, p, r = row(temperature, np.float32), row(top_k, np.int32), row(top_p, np.float32), row(repetition_penalty, np.float32)
+    sd, ct = row(seed, np.uint64), row(counter, np.uint64)
+    sets = None if token_sets is None else np.ascontiguousarray(np.broadcast_to(np.asarray(token_sets, dtype=np.uint32), (n, 128)))
+    ids = np.zeros(n, np.int32)
+    proc = np.zeros((n, V), np.float32) if want_processed else None
+    pi = lambda a: a.ctypes.data_as(A.p_i32)
+    A.check(A.lib().q3tts_sampler_probe(device, form, _pf(lg), n, V, ld, codec_vocab, _pf(t), pi(k), _pf(p), _pf(r),
+                                        None if sets is None else sets.ctypes.data, sd.ctypes.data, ct.ctypes.data, pi(ids), _pf(proc)), None)
+    return ids, proc
+
+
+SLOT_FIELDS = ("active", "finished", "step", "max_tokens", "trailing_idx", "total_text", "consecutive_pad", "n_forced", "stream_variant",
+               "frame_alive", "logits_cap")
+
+
+def sampler_slot_probe(form, group, logits, state, sampling, token_sets, cur_codes, eos_id, pad_id, codec_vocab, forced=None,
+                       dump_slot=0, dump_frames=None, device=0):
+    """`q3tts_sampler_slot_probe`: one sampling point of `group` for every slot of logits [n, V].  state: {SLOT_FIELDS name: int [n]};
+    sampling: {temperature, top_k, top_p, repetition_penalty, seed: [n]}; token_sets uint32 [n, 16, set_words]; cur_codes int [n, 16];
+    forced int [n, max_frames, 16] or None; dump_frames: rows of the logits dump of slot dump_slot, or None (no dump).
+    -> (state after the launch, token_sets, cur_codes, dump [dump_frames, V] or None); the inputs are not modified."""
+    lg = _f32(logits)
+    n, V = lg.shape
+    st = {f: np.array(np.broadcast_to(np.asarray(state[f], dtype=np.int32), (n,))) for f in SLOT_FIELDS}
+    row = lambda name, dt: np.ascontiguousarray(np.broadcast_to(np.asarray(sampling[name], dtype=dt), (n,)))
+    t, k, p, r = row("temperature", np.float32), row("top_k", np.int32), row("top_p", np.float32), row("repetition_penalty", np.float32)
+    sd = row("seed", np.uint64)
+    sets = np.array(token_sets, dtype=np.uint32)
+    assert sets.ndim == 3 and sets.shape[:2] == (n, 16)
+    codes = np.array(cur_codes, dtype=np.int32).reshape(n, 16)
+    fz = None if forced is None else np.ascontiguousarray(forced, dtype=np.int32)
+    max_frames = 0 if fz is None else fz.shape[1]
+    dump = None if dump_frames is None else np.zeros((dump_frames, V), np.float32)
+    pi = lambda a: None if a is None else a.ctypes.data_as(A.p_i32)
+    A.check(A.lib().q3tts_sampler_slot_probe(device, form, group, n, V, codec_vocab, eos_id, pad_id, _pf(lg), *[pi(st[f]) for f in SLOT_FIELDS],
+                                             _pf(t), pi(k), _pf(p), _pf(r), sd.ctypes.data, sets.ctypes.data, sets.shape[2], pi(fz), max_frames,
+                                             _pf(dump), dump_slot, 0 if dump_frames is None else dump_frames, pi(codes)), None)
+    return st, sets, codes, dump
