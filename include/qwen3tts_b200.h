@@ -369,7 +369,7 @@ q3tts_status q3tts_attention_probe(int32_t device, int32_t kernel, int32_t kv_f1
  * as 3.4e38 (fp32) or NaN (fp16).
  *
  * Codec-transformer attention (head_dim 64, scale 1/sqrt(64)).  kernel: 0 = the tcgen05 pipeline's fp16-output launch on the
- * mma.sync kernel (whatever Q3TTS_CODEC_ATT_MMA says), 1 = the SIMT pipeline's fp32 kernel (causal), 2 = its bidirectional form (ICL
+ * mma.sync kernel, 1 = the SIMT pipeline's fp32 kernel (causal), 2 = its bidirectional form (ICL
  * encoder), 3 = the fp16-output SIMT kernel (the fallback of kernel 0's launcher).  qkv [B][T][(nh + 2*nkv)*64] fp32, in/out: when
  * inv_freq [32] is given the codec RoPE runs on it first, in place (positions t = row % T), and the roped rows come back.
  * out [B][T][nh*64] fp32 (fp16 values widened for kernels 0 and 3).  1 <= B <= 64, 1 <= T <= 2400, nh <= 64, nh % nkv == 0. */
@@ -410,12 +410,6 @@ q3tts_status q3tts_codec_rowop_probe(int32_t device, int32_t op, const float* x,
  * ---------------------------------------------------------------------------------------------------- */
 q3tts_status q3tts_profile_linear(q3tts_handle* h, int32_t which, int32_t m, int32_t iters, double* ms_out,
                                   int64_t* launches_out, int64_t* bytes_per_iter_out);
-
-/* test hook: launches a kernel that waits on an mbarrier nobody arrives at -- the failure mode of a broken TMA / tcgen05 protocol.  The
- * bounded wait (csrc/tc_ptx.cuh mbar_wait) traps instead of hanging the GPU; the call returns Q3TTS_ERR_CUDA, the handle is POISONED (a
- * kernel fault is sticky for the process's CUDA context): every later call on it returns Q3TTS_ERR_CUDA with the same q3tts_last_error
- * text, q3tts_destroy still works.  No reference counterpart. */
-q3tts_status q3tts_debug_trap(q3tts_handle* h);
 
 /* measurement hook (scripts/skinny_trace.py): `iters` back-to-back launches (one CUDA graph, programmatic dependent launch,
  * a different weight matrix each) of the <= 128-row split-K cluster GEMM (csrc/gemm_skinny.cu) for an [M x K] . [N x K]^T

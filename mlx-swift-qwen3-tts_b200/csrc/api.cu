@@ -15,7 +15,6 @@
 #include "engine.h"
 #include "gemm_tc.h"
 #include "sampler.cuh"
-#include "tc_ptx.cuh"
 
 using namespace q3;
 
@@ -482,7 +481,6 @@ q3tts_status q3tts_create(const char* model_dir, const q3tts_options* opts, q3tt
       // speech_tokenizer/{config...} + model.safetensors (Qwen3TTSPipeline.swift:191-208)
       // one pass holds up to codec_max_frames frames (batch x window); the workspace itself is allocated on first use
       h->codec.reset(new CodecDecoder(dir + "/speech_tokenizer", h->stream, &h->counter, h->opt.codec_max_frames));
-      h->codec->set_use_graph(h->opt.use_cuda_graph != 0);
       // audio encoder for ICL, optional: a failing load leaves ICL unavailable, it does not fail the pipeline (Qwen3TTSPipeline.swift:210-218)
       if (AudioEncoder::present(dir + "/speech_tokenizer")) {
         try {
@@ -533,7 +531,6 @@ q3tts_status q3tts_clone(q3tts_handle* parent, q3tts_handle** out) {
     }
     if (parent->codec) {  // codec weights are small (0.6 GB with their fp16 copies): loaded again, with their own workspace
       h->codec.reset(new CodecDecoder(h->model_dir + "/speech_tokenizer", h->stream, &h->counter, h->opt.codec_max_frames));
-      h->codec->set_use_graph(h->opt.use_cuda_graph != 0);
     }
     Q3_CUDA(cudaStreamSynchronize(h->stream));
     *out = h;
@@ -624,27 +621,6 @@ q3tts_status q3tts_clear_cache(q3tts_handle* h) {
   return guarded(h, [&] {
     Q3_CUDA(cudaStreamSynchronize(h->stream));
     if (h->talker) h->talker->drop_graphs();
-  });
-}
-
-namespace {
-// test hook: the failure mode of a broken TMA / mbarrier protocol -- a wait on a barrier nobody arrives at
-__global__ void debug_mbar_trap_kernel() {
-  __shared__ uint64_t bar;
-  if (threadIdx.x == 0) {
-    q3::tcptx::mbar_init(&bar, 1);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-  }
-  __syncthreads();
-  if (threadIdx.x == 0) q3::tcptx::mbar_wait(&bar, 0);
-}
-}  // namespace
-
-q3tts_status q3tts_debug_trap(q3tts_handle* h) {
-  return guarded(h, [&] {
-    debug_mbar_trap_kernel<<<1, 32, 0, h->stream>>>();
-    Q3_CUDA(cudaGetLastError());
-    Q3_CUDA(cudaStreamSynchronize(h->stream));
   });
 }
 

@@ -62,8 +62,8 @@ const __half* CodecDecoder::upload_f16(const std::vector<float>& h, int reps, si
 
 // copies of a conv weight for the L2-slice spreading described at ConvW::w16_reps: only matrices small enough that the re-reads matter
 static int weight_reps(size_t halves) {
-  static const int env = [] { const char* e = getenv("Q3TTS_CODEC_WREP"); return e ? std::max(1, std::min(32, atoi(e))) : 8; }();
-  return halves * 2 <= (size_t)(2u << 20) ? env : 1;
+  constexpr int kReps = 8;
+  return halves * 2 <= (size_t)(2u << 20) ? kReps : 1;
 }
 
 // A contraction can take the tcgen05 path when its K rows are 16-byte multiples (TMA) and N is a multiple of 32 (epilogue chunks).
@@ -369,14 +369,7 @@ CodecDecoder::CodecDecoder(const std::string& dir, cudaStream_t stream, LaunchCo
     if (e[0] == '1') use_tc_ = false;  // A/B switch: run the fp32 SIMT pipeline
 }
 
-void CodecDecoder::drop_graphs() {
-  for (auto& g : graphs_)
-    if (g.second.exec) cudaGraphExecDestroy(g.second.exec);
-  graphs_.clear();
-}
-
 CodecDecoder::~CodecDecoder() {
-  drop_graphs();
   for (float*& p : ws_)
     if (p) { cudaFree(p); p = nullptr; }
   for (__half*& p : hs_)
@@ -398,8 +391,6 @@ void CodecDecoder::ensure_workspace(int frames) {
   per = std::max(per, rate * c.decoder_dim);
   for (auto& b : blocks_) { per = std::max(per, rate * b.cin); rate *= b.rate; per = std::max(per, rate * b.cout); }
   Q3_CUDA(cudaStreamSynchronize(stream_));
-  drop_graphs();  // they hold the old workspace pointers
-  seen_.clear();
   for (float*& p : ws_)
     if (p) { cudaFree(p); p = nullptr; }
   for (__half*& p : hs_)
@@ -422,46 +413,8 @@ void CodecDecoder::rvq_embed(const int32_t* d_codes, int B, int T, float* d_firs
 }
 
 void CodecDecoder::decode_pass(const int32_t* d_codes, int B, int T, float* d_pcm) {
-  // Opt-in (Q3TTS_CODEC_GRAPH=1): measured on B200, capture + instantiate of the ~110-node pass costs 100-500 ms, and the windows of
-  // a continuous batch rarely repeat their exact (B, T) (one utterance stopping early changes both), so replay seldom pays it back.
-  static const bool env_graph = [] { const char* e = getenv("Q3TTS_CODEC_GRAPH"); return e && atoi(e) != 0; }();
-  auto eager = [&] {
-    if (use_tc_) decode_pass_tc(d_codes, B, T, d_pcm);
-    else decode_pass_simt(d_codes, B, T, d_pcm);
-  };
-  if (!use_graph_ || !env_graph || B * T <= 0) return eager();
-  // ~110 launches (two host-encoded tensor maps each) per pass: replayed as one graph the pass does not depend on the host
-  // keeping up -- measured 47 ms -> 94-135 ms for the same pass whenever the submitting thread was stalled.
-  Q3_CHECK(B * T <= pass_frames_, Q3TTS_ERR_CAPACITY, "codec pass of %d frames exceeds pass capacity %d", B * T, pass_frames_);
-  ensure_workspace(B * T);  // may drop every cached graph; never runs inside a capture
-  const PassKey key{B, T, d_codes, d_pcm};
-  auto it = graphs_.find(key);
-  if (it == graphs_.end()) {
-    // capture + instantiate costs 100-400 ms: only shapes that keep coming back (steady serving windows) are worth it;
-    // one-off shapes (an utterance that stopped early changes the batch of a window) stay eager
-    if (++seen_[key] < 3) return eager();
-    if (graphs_.size() >= 64) drop_graphs();
-    PassGraph pg;
-    cudaGraph_t graph = nullptr;
-    const bool was = counter_ ? counter_->capturing : false;
-    if (counter_) { counter_->capturing = true; counter_->captured = 0; }
-    Q3_CUDA(cudaStreamBeginCapture(stream_, cudaStreamCaptureModeThreadLocal));
-    try {
-      eager();
-    } catch (...) {
-      cudaStreamEndCapture(stream_, &graph);
-      if (graph) cudaGraphDestroy(graph);
-      if (counter_) counter_->capturing = was;
-      throw;
-    }
-    Q3_CUDA(cudaStreamEndCapture(stream_, &graph));
-    if (counter_) { pg.launches = counter_->captured; counter_->capturing = was; }
-    Q3_CUDA(cudaGraphInstantiate(&pg.exec, graph, 0));
-    cudaGraphDestroy(graph);
-    it = graphs_.emplace(key, pg).first;
-  }
-  Q3_CUDA(cudaGraphLaunch(it->second.exec, stream_));
-  if (counter_) counter_->n += it->second.launches;
+  if (use_tc_) decode_pass_tc(d_codes, B, T, d_pcm);
+  else decode_pass_simt(d_codes, B, T, d_pcm);
 }
 
 // tcgen05 pipeline: every dense contraction is one launch of the implicit-GEMM kernel with its elementwise neighbours fused
@@ -525,15 +478,14 @@ void CodecDecoder::decode_pass_tc(const int32_t* d_codes, int B, int T, float* d
   std::swap(cur, oa);  // cur = snake(init conv output)
   // The blocks' residual stream lives in fp16 (R0, carved out of the fp32 buffer F0): at 96-192 channels and 640-1920 samples per
   // frame it was the largest HBM stream of the pass (fp32: 1.2 GB read + 1.2 GB written per 1x1 conv at 64 x 26 frames); the
-  // arithmetic stays fp32, one more fp16 rounding per unit (Q3TTS_CODEC_RES32=1 keeps the fp32 stream).
-  static const bool res32 = [] { const char* e = getenv("Q3TTS_CODEC_RES32"); return e && atoi(e) != 0; }();
+  // arithmetic stays fp32, one more fp16 rounding per unit.
   __half* R0 = reinterpret_cast<__half*>(F0);
   for (size_t bi = 0; bi < blocks_.size(); ++bi) {  // DecoderBlock (:753-784)
     Block& b = blocks_[bi];
     // polyphase transposed conv: y (residual stream) and snake_act1(y) (fp16 operand)
     {
       TcGemm g = gemm(b.convT, cur, B, Tc);
-      if (res32) { g.out32 = F0; } else { g.outr16 = R0; g.allow_skinny = 0; }
+      g.outr16 = R0; g.allow_skinny = 0;
       g.ld32 = b.convT.n; g.out16 = oa; g.ld16 = b.convT.n; with_snake(g, b.unit[0].act1);
       launch_tc_gemm(lc, g);
     }
@@ -541,7 +493,7 @@ void CodecDecoder::decode_pass_tc(const int32_t* d_codes, int B, int T, float* d
     for (int j = 0; j < 3; ++j) {  // DecoderResidualUnit (:696-718)
       const bool last = j == 2;
       const SnakeW& nxt = !last ? b.unit[j + 1].act1 : (bi + 1 < blocks_.size() ? blocks_[bi + 1].snake : out_snake_);
-      if (!res32) {  // thin stages: the whole unit in one persistent kernel (codec_unit.cu), the intermediate never leaves the SM
+      {  // thin stages: the whole unit in one persistent kernel (codec_unit.cu), the intermediate never leaves the SM
         CodecUnit u;
         u.Bt = B; u.T = Tc; u.C = b.cout; u.dil = b.unit[j].conv1.dil;
         u.a = oa; u.w7 = b.unit[j].conv1.w16; u.b7 = b.unit[j].conv1.bias;
@@ -561,22 +513,14 @@ void CodecDecoder::decode_pass_tc(const int32_t* d_codes, int B, int T, float* d
       { TcGemm g = gemm(b.unit[j].conv1, oa, B, Tc); g.out16 = ob; g.ld16 = b.cout; with_snake(g, b.unit[j].act2); launch_tc_gemm(lc, g); }
       TcGemm g = gemm(b.unit[j].conv2, ob, B, Tc);
       g.ld_res = b.cout; g.ld32 = b.cout;
-      const bool last_unit = j == 2;
-      if (res32) {
-        g.res = F0;
-        if (!last_unit) g.out32 = F0;
-      } else {
-        g.res16 = R0; g.allow_skinny = 0;
-        if (!last_unit) g.outr16 = R0;
-      }
-      g.out16 = last_unit ? cur : oa; g.ld16 = b.cout;
-      const SnakeW& next = !last_unit ? b.unit[j + 1].act1 : (bi + 1 < blocks_.size() ? blocks_[bi + 1].snake : out_snake_);
-      with_snake(g, next);
+      g.res16 = R0; g.allow_skinny = 0;
+      if (!last) g.outr16 = R0;
+      g.out16 = last ? cur : oa; g.ld16 = b.cout;
+      with_snake(g, nxt);
       launch_tc_gemm(lc, g);
     }
   }
-  static const bool out_stream = !(getenv("Q3TTS_CODEC_OUT_STREAM") && atoi(getenv("Q3TTS_CODEC_OUT_STREAM")) == 0);
-  if (out_stream && out_conv_stream_supported(out_ch_)) {
+  if (out_conv_stream_supported(out_ch_)) {
     launch_out_conv_stream_f16(lc, cur, out_w_, out_b_, out_ch_, B, Tc, d_pcm);  // HBM-bound: streamed once, fp32 weights in registers
   } else {
     TcGemm g = gemm(out_tc_, cur, B, Tc); g.pcm = d_pcm; launch_tc_gemm(lc, g);

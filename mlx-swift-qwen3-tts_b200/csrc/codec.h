@@ -62,11 +62,8 @@ class CodecDecoder {
   int vq_dim() const { return cfg_.codebook_dim / 2; }
 
   // decodeImpl (Vocoder/SpeechTokenizer.swift:917-952): d_codes [B][T][Q] int32 -> d_pcm [B][T*up] fp32 (clipped to [-1,1]).
-  // B*T must be <= pass_frames().
-  // With Q3TTS_CODEC_GRAPH=1 the launches of a pass whose (B, T, buffers) keeps recurring are captured as a CUDA graph and
-  // replayed; default: eager launches (see decode_pass).
+  // B*T must be <= pass_frames().  Eager launches: a CUDA graph of a pass rarely pays back its capture (DESIGN.md §7).
   void decode_pass(const int32_t* d_codes, int B, int T, float* d_pcm);
-  void set_use_graph(bool on) { use_graph_ = on; }
   bool uses_tensor_cores() const { return use_tc_; }
   // code -> embedding gather-sums (bit-exact probe): d_first/d_rest [B*T][vq_dim]
   void rvq_embed(const int32_t* d_codes, int B, int T, float* d_first, float* d_rest);
@@ -74,7 +71,6 @@ class CodecDecoder {
 
  private:
   void ensure_workspace(int frames);
-  void drop_graphs();
   void decode_pass_simt(const int32_t* d_codes, int B, int T, float* d_pcm);
   void decode_pass_tc(const int32_t* d_codes, int B, int T, float* d_pcm);
   void finish_weight(ConvW& w);           // uploads the fp16 copy, updates use_tc_
@@ -85,15 +81,6 @@ class CodecDecoder {
   ConvW load_linear(const std::map<std::string, STensor>& t, const std::string& key, int cout, int cin, bool bias);
   const float* load_vec(const std::map<std::string, STensor>& t, const std::string& key, int n);
   SnakeW load_snake(const std::map<std::string, STensor>& t, const std::string& prefix, int ch);
-
-  struct PassGraph { cudaGraphExec_t exec = nullptr; int64_t launches = 0; };
-  struct PassKey {
-    int B, T; const void* codes; const void* pcm;
-    bool operator<(const PassKey& o) const { return std::tie(B, T, codes, pcm) < std::tie(o.B, o.T, o.codes, o.pcm); }
-  };
-  std::map<PassKey, PassGraph> graphs_;
-  std::map<PassKey, int> seen_;
-  bool use_graph_ = true;
 
   CodecConfig cfg_;
   cudaStream_t stream_;

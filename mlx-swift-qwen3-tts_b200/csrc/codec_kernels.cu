@@ -419,10 +419,6 @@ __global__ void __launch_bounds__(128) codec_attention_mma_kernel(const float* _
   }
 }
 
-void launch_codec_attention_f16(const LaunchCtx& c, const float* qkv, int ld, int B, int T, int nh, int nkv, __half* out, int ldo) {
-  static const bool mma = !(getenv("Q3TTS_CODEC_ATT_MMA") && atoi(getenv("Q3TTS_CODEC_ATT_MMA")) == 0);
-  launch_codec_attention_f16(c, qkv, ld, B, T, nh, nkv, out, ldo, mma);
-}
 void launch_codec_attention_f16(const LaunchCtx& c, const float* qkv, int ld, int B, int T, int nh, int nkv, __half* out, int ldo, bool mma) {
   if (B <= 0 || T <= 0) return;
   if (mma && ld % 4 == 0 && ldo % 2 == 0) {
@@ -598,10 +594,6 @@ __global__ void __launch_bounds__(128) out_conv_stream_kernel(const __half* __re
   }
 }
 bool out_conv_stream_supported(int C) { return C == 32 || C == 64 || C == 96 || C == 128; }
-void launch_out_conv_stream_f16(const LaunchCtx& c, const __half* x, const float* w, const float* bias, int C, int B, int T, float* y) {
-  static const int strip_env = getenv("Q3TTS_OUT_STRIP") ? atoi(getenv("Q3TTS_OUT_STRIP")) : 0;
-  launch_out_conv_stream_f16(c, x, w, bias, C, B, T, y, strip_env);
-}
 void launch_out_conv_stream_f16(const LaunchCtx& c, const __half* x, const float* w, const float* bias, int C, int B, int T, float* y, int strip_rows) {
   if (B <= 0 || T <= 0) return;
   const int strip = strip_rows >= 32 ? (strip_rows & ~31) : 256;  // multiple of 32 (outputs are stored 32 at a time); ~3 waves of warps at B x T = 64 x 49 920

@@ -17,9 +17,8 @@ void launch_layernorm_f16(const LaunchCtx& c, const float* x, int rows, int C, c
 void launch_silu_mul(const LaunchCtx& c, const float* gu, size_t rows, int I, float* y);
 void launch_codec_rope(const LaunchCtx& c, float* qkv, int ld, int M, int T, int n_rot_heads, const float* inv_freq);
 void launch_codec_attention(const LaunchCtx& c, const float* qkv, int ld, int B, int T, int nh, int nkv, float* out, int ldo);
-void launch_codec_attention_f16(const LaunchCtx& c, const float* qkv, int ld, int B, int T, int nh, int nkv, __half* out, int ldo);
-// mma: the mma.sync kernel (when ld % 4 == 0 and ldo % 2 == 0) or the SIMT kernel; the form above takes it from Q3TTS_CODEC_ATT_MMA
-void launch_codec_attention_f16(const LaunchCtx& c, const float* qkv, int ld, int B, int T, int nh, int nkv, __half* out, int ldo, bool mma);
+// mma: the mma.sync kernel (when ld % 4 == 0 and ldo % 2 == 0) or the SIMT kernel
+void launch_codec_attention_f16(const LaunchCtx& c, const float* qkv, int ld, int B, int T, int nh, int nkv, __half* out, int ldo, bool mma = true);
 // ICL audio encoder (audio_encoder.cu)
 void launch_codec_attention_bidir(const LaunchCtx& c, const float* qkv, int ld, int B, int T, int nh, int nkv, float* out, int ldo);
 void launch_elu(const LaunchCtx& c, const float* x, size_t total, float* y);
@@ -31,9 +30,9 @@ void launch_out_conv(const LaunchCtx& c, const float* x, const float* w, const f
 void launch_out_conv_f16(const LaunchCtx& c, const __half* x, const float* w, const float* bias, int C, int B, int T, float* y);
 // streaming form (one pass over the activations, weights in registers); C in {32, 64, 96, 128}
 bool out_conv_stream_supported(int C);
-void launch_out_conv_stream_f16(const LaunchCtx& c, const __half* x, const float* w, const float* bias, int C, int B, int T, float* y);
-// strip_rows: outputs per warp, rounded down to a multiple of 32; below 32 = the default (256).  The form above reads Q3TTS_OUT_STRIP once.
-void launch_out_conv_stream_f16(const LaunchCtx& c, const __half* x, const float* w, const float* bias, int C, int B, int T, float* y, int strip_rows);
+// strip_rows: outputs per warp, rounded down to a multiple of 32; below 32 = the default (256)
+void launch_out_conv_stream_f16(const LaunchCtx& c, const __half* x, const float* w, const float* bias, int C, int B, int T, float* y,
+                                int strip_rows = 0);
 // emb fp32 [M][2D] (bit-exact gather-sums) and/or its fp16 copy
 void launch_rvq_embed_f16(const LaunchCtx& c, const int* codes, const float* const* codebooks, int Q, int n_sem, int D, int size, int M,
                           __half* emb16);

@@ -39,7 +39,8 @@ constexpr int kBlockK = 64;
 constexpr int kHaloRowsMax = 192;
 constexpr int kHaloBytes = kHaloRowsMax * kBlockK * 2;  // 24 KB
 constexpr int kTaps = 7;
-constexpr int kMaxThreads = 448;
+constexpr int kMaxEpiSets = 3;                       // sets of 4 epilogue warps
+constexpr int kMaxThreads = 64 + 128 * kMaxEpiSets;
 constexpr int kMaxC = 192;
 constexpr int kTraceTiles = 8;
 constexpr int kTraceSlots = 12;
@@ -434,26 +435,18 @@ void launch_codec_unit(const LaunchCtx& c, const CodecUnit& u) {
   // three accumulators when tensor memory allows (C <= 128): conv7 of tile i+2 runs while E2 drains tile i (with two, the tensor
   // pipe idles for the length of an E2 per tile); the halo ring holds two tiles' worth of channel blocks so that the next tile's
   // activations are in flight while this tile's MMAs run
-  static const int acc_env = [] { const char* e = getenv("Q3TTS_CODEC_UNIT_NACC"); return e ? atoi(e) : 3; }();
-  static const int ast_env = [] { const char* e = getenv("Q3TTS_CODEC_UNIT_ASTAGES"); return e ? atoi(e) : 3; }();
-  p.n_acc = (acc_env >= 3 && 3 * u.C + u.C / 2 <= 512) ? 3 : 2;
-  p.a_stages = std::max(2, std::min(ast_env, 4));
+  p.n_acc = 3 * u.C + u.C / 2 <= 512 ? 3 : 2;
+  p.a_stages = 3;
   const int ring_budget = 212 * 1024 - 12 * epiio::kPatchBytes;  // 188 KB for the two operand rings
-  static const int tps_env = [] { const char* e = getenv("Q3TTS_CODEC_UNIT_TPS"); return e ? atoi(e) : 2; }();
-  p.tps = (tps_env >= 2 && p.b_bytes <= 16 * 1024) ? 2 : 1;  // C <= 128: two weight tiles per ring stage
+  p.tps = p.b_bytes <= 16 * 1024 ? 2 : 1;  // C <= 128: two weight tiles per ring stage
   const int sbytes = p.tps * p.b_bytes;
   if (sbytes * 3 + p.a_stages * kHaloBytes > ring_budget) p.a_stages = std::max(2, (ring_budget - 3 * sbytes) / kHaloBytes);
   p.b_stages = std::max(2, std::min(12, (ring_budget - p.a_stages * kHaloBytes) / sbytes));
-  {
-    static const int bs_env = [] { const char* e = getenv("Q3TTS_CODEC_UNIT_BSTAGES"); return e ? atoi(e) : 0; }();
-    if (bs_env > 0) p.b_stages = std::min(p.b_stages, bs_env);
-  }
   p.h_col0 = p.n_acc * u.C;
   int cols = 32;
   while (cols < p.n_acc * u.C + u.C / 2) cols <<= 1;
   p.tmem_cols = cols;
-  static const int max_sets = [] { const char* e = getenv("Q3TTS_TC_EPI_SETS"); return e ? std::max(1, std::min(3, atoi(e))) : 3; }();
-  p.epi_sets = std::max(1, std::min(max_sets, u.C / 32));
+  p.epi_sets = std::max(1, std::min(kMaxEpiSets, u.C / 32));
   p.b7 = u.b7; p.ea2 = u.snake2_ea; p.ieb2 = u.snake2_ieb; p.b1 = u.b1; p.ea3 = u.next_ea; p.ieb3 = u.next_ieb;
   p.res16 = u.res16; p.outr16 = u.outr16; p.out16 = u.out16;
 

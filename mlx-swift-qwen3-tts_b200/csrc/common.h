@@ -66,41 +66,6 @@ inline bool pdl_enabled() {
 }
 #endif
 
-// ---- chain signals: flag hand-off between consecutive kernels of a decode step -------------------------------------------------
-// A kernel launched with programmatic dependent launch is resident (weights prefetched, operands dequantised) long before its
-// predecessor retires, but griddepcontrol.wait only returns once the WHOLE predecessor grid has completed and flushed.  Chained
-// kernels hand over earlier: every CTA of the producer, after its last global store, does fence + one increment of the launch's
-// counter; the consumer spins on that counter (acquire) until all producer CTAs have signalled, and never executes
-// griddepcontrol.wait.  Safe because a dependent grid only starts once ALL CTAs of its primary are resident (they called
-// launch_dependents), so a spinning consumer can never keep its producer from running; every CTA signals after ALL its reads and
-// writes, so later launches may reuse the producer's input buffers; visibility to later launches follows from the
-// release/acquire chain.  Counters are zeroed by a memset node at the head of every frame graph.
-struct ChainSig {
-  unsigned* out = nullptr;        // incremented once per CTA of this launch
-  const unsigned* in = nullptr;   // non-null: wait for *in >= in_target instead of griddepcontrol.wait
-  unsigned in_target = 0;
-};
-#ifdef __CUDACC__
-__device__ __forceinline__ void chain_signal(unsigned* sig) {  // ONE thread, after a CTA barrier that follows the CTA's last store
-  __threadfence();
-  asm volatile("red.release.gpu.global.add.u32 [%0], 1;" ::"l"(sig) : "memory");
-}
-__device__ __forceinline__ void chain_wait(const unsigned* sig, unsigned target) {
-  unsigned v, spins = 0;
-  while (true) {
-    asm volatile("ld.acquire.gpu.global.u32 %0, [%1];" : "=r"(v) : "l"(sig) : "memory");
-    if (v >= target) break;
-    if (++spins > (1u << 25)) __trap();  // a protocol bug must surface as an error, never as a hung GPU
-  }
-}
-#endif
-struct ChainState {
-  unsigned* base = nullptr;       // device counters of one frame graph
-  int capacity = 0, next = 0;
-  const unsigned* prev = nullptr; // counter of the launch issued last, when that launch signals
-  unsigned prev_ctas = 0;
-};
-
 // Counts every kernel this library launches (reported as q3tts_timing.kernel_launches / bench gpu_launches).
 struct LaunchCounter {
   int64_t n = 0;

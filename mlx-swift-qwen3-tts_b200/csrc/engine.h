@@ -109,13 +109,13 @@ class TalkerEngine {
   bool use_tc(int) const { return handle_tc_; }
   // decode steps: ONE numeric path per handle, fixed at creation from max_batch (not from how many slots happen to be live in a
   // frame), so a request's codes do not depend on what it is co-batched with or on utterances finishing around it:
-  //   max_batch >= tc_min_rows_step_ (3)  -> every decode step on the tcgen05 GEMMs (fp16 operands, fp32 accumulate)
-  //   max_batch <= 2                      -> the persistent frame kernel (fp32 activations), else the SIMT graph path
+  //   max_batch >= tc_min_rows_ (3)  -> every decode step on the tcgen05 GEMMs (fp16 operands, fp32 accumulate)
+  //   max_batch <= 2                 -> the persistent frame kernel (fp32 activations), else the SIMT graph path
   bool use_tc_step(int) const { return handle_tc_; }
   bool use_mega(int n_slots) const { return mega_.ok && !handle_tc_ && opt_.max_batch <= mega_.max_slots && n_slots <= mega_.max_slots; }
   // y = epilogue(x16 . W^T): one tcgen05 GEMM launch over m rows
   void linear_tc(const TcLinear& L, const void* x16, int m, float* out32, int ld32, void* out16, int ld16, const float* res, int act, int swiglu, bool row_count_invariant = false);
-  LaunchCtx ctx() { return LaunchCtx{stream_, counter_, chain_on_ ? &chain_ : nullptr}; }
+  LaunchCtx ctx() { return LaunchCtx{stream_, counter_}; }
 
   TalkerConfig cfg_;
   EngineOptions opt_;
@@ -127,10 +127,10 @@ class TalkerEngine {
   TalkerWeights& w_;
 
   int max_rows_ = 0, max_tp_rows_ = 0, set_words_ = 0;
-  // rows from which linears run on tensor cores (env Q3TTS_TC_MIN_ROWS sets both; 0 disables).  Decode steps switch at 3
-  // utterances: measured per frame-step (0.6B 4-bit) 6.5 / 10.3 / 17.2 ms at 3 / 8 / 12 rows on the SIMT path against a flat
-  // 3.45-3.5 ms on the split-K cluster GEMM; 1-2 utterances stay on the persistent frame kernel (2.2 ms).
-  int tc_min_rows_ = 16, tc_min_rows_step_ = 3;
+  // max_batch from which a handle runs on tensor cores and keeps fp16 KV rings (env Q3TTS_TC_MIN_ROWS; 0 disables).  Decode steps
+  // switch at 3 utterances: measured per frame-step (0.6B 4-bit) 6.5 / 10.3 / 17.2 ms at 3 / 8 / 12 rows on the SIMT path against a
+  // flat 3.45-3.5 ms on the split-K cluster GEMM; 1-2 utterances stay on the persistent frame kernel (2.2 ms).
+  int tc_min_rows_ = 3;
   bool step_tc_ = false;  // set by issue_frame for the launches of the current frame step
   bool handle_tc_ = false;  // decode steps of this handle run on tensor cores (see use_tc_step)
   // 3..128-row GEMMs of a quantised checkpoint read the packed weights (gemm_skinny_q.cu) instead of the fp16 copies: q3tts_options::
@@ -138,10 +138,6 @@ class TalkerEngine {
   // dequantisation in front of the MMAs lengthens every link (measured 4.95-5.4 ms against 4.18 ms per frame-step; DESIGN.md 3.2).
   bool packed_gemm_ = false;
   void attach_packed(struct TcGemm& g, const TcLinear& L) const;
-  // chain signals (common.h): counters of one frame graph + the link state while issue_frame records its launches
-  static constexpr int kChainCounters = 1024;
-  ChainState chain_;
-  bool chain_on_ = false, chain_enabled_ = false;
   float* d_rs_ = nullptr;                     // [max_rows] RMSNorm row factors for the 128-row-tile kernel (prefill)
   static constexpr float kX16Div = 16.0f;     // the fp16 copy of the residual stream is x / 16 (range headroom; exact power of two)
   void *d_h16_ = nullptr, *d_attn16_ = nullptr, *d_act16_ = nullptr, *d_tpe16_ = nullptr, *d_tph16_ = nullptr;

@@ -98,12 +98,7 @@ tc_skinny_kernel(const __grid_constant__ CUtensorMap tmW, const __grid_constant_
         // tiles into L2 now, so that request is an L2 hit instead of a DRAM round trip on the critical path
         for (int i = pre; i < nkb; ++i) tma_prefetch_2d(&tmW, (kb0 + i) * kBlockK, n0);
       }
-      if (p.sig.in) {
-        if (lead) sk_wait_dependency_tma(p);
-        __syncwarp();
-      } else {
-        pdl_wait();
-      }
+      pdl_wait();
       int s = 0;
       uint32_t ph = 0;  // ring position as wrapping counters: no integer division per k-block in the issuing threads
       for (int i = 0; i < nkb; ++i) {
@@ -145,7 +140,7 @@ tc_skinny_kernel(const __grid_constant__ CUtensorMap tmW, const __grid_constant_
     __syncwarp();
   } else {
     // ---------------- epilogue warps: warp w may touch TMEM lanes [32*(w%4), +32); thread = one weight row
-    sk_wait_dependency_warp(p);  // residual rows were written by earlier kernels
+    pdl_wait();  // residual rows were written by earlier kernels
     if (p.rms_x) sk_row_factors(p, rowscale_s, rank);  // while the operands stream in
     if (p.split > 1) cluster_wait_acquire();  // A: every peer CTA is resident, its mbarriers initialised (long complete by now)
     mbar_wait(tmem_full, 0);
@@ -167,10 +162,7 @@ tc_skinny_kernel(const __grid_constant__ CUtensorMap tmW, const __grid_constant_
   }
 }
 
-int env_int(const char* name, int dflt) {
-  const char* e = getenv(name);
-  return e ? atoi(e) : dflt;
-}
+constexpr int kSmemKB = 108;  // operand ring + reduction buffer
 
 struct SkPlan {
   int m_pad, split, stages, num_kb, tiles;
@@ -178,22 +170,16 @@ struct SkPlan {
 };
 
 SkPlan plan(const TcGemm& g) {
-  static const int max_split = std::max(1, std::min(16, env_int("Q3TTS_SK_MAX_SPLIT", 8)));  // > 8: non-portable cluster size (B200 allows 16)
-  // up to ~1.3 waves: 48 weight tiles (gate|up) take 4 K slices = 192 CTAs of 4 k-blocks (two co-resident per SM on 44 SMs)
-  // rather than 96 CTAs of 8 k-blocks; measured 13.5 -> ~9 us per launch at 64 rows
-  static const int cta_target = env_int("Q3TTS_SK_CTAS", 200);
-  static const int smem_kb = env_int("Q3TTS_SK_SMEM_KB", 108);
   SkPlan s{};
   const int M = g.Bt * g.T;
   s.m_pad = M <= 32 ? 32 : (M <= 64 ? 64 : 128);
   s.tiles = (g.N + kRowsW - 1) / kRowsW;
   s.num_kb = (g.cin + kBlockK - 1) / kBlockK;
-  s.split = 1;
-  while (s.split * 2 <= max_split && s.tiles * s.split * 2 <= cta_target && s.split * 2 <= s.num_kb && s.m_pad / (s.split * 2) >= 4) s.split *= 2;
+  s.split = k_split(s.tiles, s.num_kb, s.m_pad);
   const int stage_bytes = kWBytes + s.m_pad * kBlockK * 2;
   const int red_bytes = kRowsW * s.m_pad * 4;
   const int nkb_max = (s.num_kb + s.split - 1) / s.split;
-  s.stages = std::max(2, (smem_kb * 1024 - red_bytes) / stage_bytes);
+  s.stages = std::max(2, (kSmemKB * 1024 - red_bytes) / stage_bytes);
   s.stages = std::max(1, std::min(s.stages, nkb_max));
   // the ring doubles as the outgoing staging buffer [owner][128][mc] fp32 (= red_bytes) once the MMAs are done
   while (s.stages * stage_bytes < red_bytes) ++s.stages;
@@ -203,15 +189,9 @@ SkPlan plan(const TcGemm& g) {
 
 }  // namespace
 
-bool tc_skinny_enabled() {
-  static const bool on = env_int("Q3TTS_SKINNY", 1) != 0;
-  return on;
-}
-
 bool tc_skinny_supported(const TcGemm& g) {
-  const bool on = tc_skinny_enabled();
   const long long M = (long long)g.Bt * g.T;
-  return on && g.allow_skinny && !g.res16 && !g.outr16 && g.ntap == 1 && M >= 1 && M <= 128 && !g.snake_ea && !g.pcm && !(g.swiglu && g.act != TC_ACT_NONE) && tc_gemm_supported(g);
+  return g.allow_skinny && !g.res16 && !g.outr16 && g.ntap == 1 && M >= 1 && M <= 128 && !g.snake_ea && !g.pcm && !(g.swiglu && g.act != TC_ACT_NONE) && tc_gemm_supported(g);
 }
 
 using SkKernel = void (*)(const CUtensorMap, const CUtensorMap, const SkParams);
@@ -260,7 +240,6 @@ void launch_tc_skinny(const LaunchCtx& c, const TcGemm& g) {
   p.rms_a = 1.0f / (g.in_scale * g.in_scale * (float)g.cin); p.rms_eps = g.rms_eps; p.rms_mult = 1.0f / g.in_scale;
   Q3_CHECK(!g.row_scale, Q3TTS_ERR_INVALID_ARG, "tc_skinny: pass rms_in instead of precomputed row factors");
   p.trace = g_sk_trace;
-  p.sig = c.chain_link((unsigned)(s.tiles * s.split));
 
   const uint64_t wdims[2] = {(uint64_t)g.cin, (uint64_t)g.N};
   const uint64_t wstr[1] = {(uint64_t)g.cin * 2};
@@ -292,7 +271,7 @@ void launch_tc_skinny(const LaunchCtx& c, const TcGemm& g) {
   cfg.attrs = attr;
   cfg.numAttrs = na;
   Q3_CUDA(cudaLaunchKernelEx(&cfg, pick_kernel(g.act, g.swiglu), mw, mx, p));
-  c.tick_chained();
+  c.tick();
 }
 
 }  // namespace q3

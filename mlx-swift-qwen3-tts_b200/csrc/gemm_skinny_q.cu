@@ -12,11 +12,10 @@
 //   * warps 2-5: one thread per weight row.  Per k-block it reads its 32 / 64 packed bytes, expands the codes with the
 //     0x6400 exponent trick (4-bit) / PRMT (8-bit), applies scale and bias in fp32 exactly as MLX `dequantized` does
 //     (deq32 = fp32(s) * q + fp32(b): the product is exact, so mul + add == fma), multiplies by the folded RMSNorm weight,
-//     rounds ONCE to fp16 and stores the 128-byte row into the A tile in the 128-byte-swizzled K-major layout the UMMA
-//     descriptor expects (16-byte chunk j of row r at chunk position j ^ (r & 7)); fence.proxy.async + mbarrier hand the tile
-//     to the MMA thread.  The bits that enter the tensor core are identical to the fp16 copies the engine used to keep
+//     rounds ONCE to fp16 and writes the row into its own lane of tensor memory (tcgen05.st); an mbarrier hands the tile to the
+//     MMA thread.  The bits that enter the tensor core are identical to the fp16 copies the engine used to keep
 //     (q3tts_dequantize contract), so parity numbers do not move;
-//   * warp 1 issues tcgen05.mma 128 x m_pad x 16 from (A tile, X tile) into TMEM, commits each stage back to the ring;
+//   * warp 1 issues tcgen05.mma 128 x m_pad x 16 from (A in TMEM, X tile in shared memory) into TMEM, commits each stage back to the ring;
 //   * warps 2-5 then run the shared reduce + epilogue (skinny_common.cuh).
 #include <cuda.h>
 
@@ -76,9 +75,6 @@ __device__ __forceinline__ void fill_sb_table(float* my_sb, const void* scales, 
       }
     }
   }
-}
-__device__ __forceinline__ void sts_v4(uint32_t saddr, uint32_t a, uint32_t b, uint32_t c, uint32_t d) {
-  asm volatile("st.shared.v4.b32 [%0], {%1, %2, %3, %4};" ::"r"(saddr), "r"(a), "r"(b), "r"(c), "r"(d) : "memory");
 }
 __device__ __forceinline__ uint4 lds_u4(uint32_t saddr) {
   uint4 v;
@@ -141,16 +137,9 @@ __device__ __forceinline__ void dequant_row(uint32_t prow_s, const float (&sc)[2
   }
 }
 
-// 64 fp16 values of tile row `row` -> the 128-byte-swizzled K-major A tile: 16-byte chunk j at chunk position j ^ (row & 7)
-__device__ __forceinline__ void store_row_swizzled(uint32_t arow, int rsw, const uint32_t (&v)[32]) {
-#pragma unroll
-  for (int j = 0; j < 8; ++j) sts_v4(arow + (uint32_t)((j ^ rsw) << 4), v[4 * j], v[4 * j + 1], v[4 * j + 2], v[4 * j + 3]);
-}
-
-// TS = true: the dequantised weight tile is the MMA's A operand straight from TENSOR MEMORY (every k-block is written there once by
-// its row's thread, tcgen05.st; no shared-memory A ring, no re-staging behind the MMAs); TS = false: A through a 2-3 stage
-// shared-memory ring in the 128-byte-swizzled layout, later k-blocks parked in TMEM and re-staged as stages free up.
-template <int BITS, bool SWIGLU, bool TS>
+// The dequantised weight tile is the MMA's A operand straight from TENSOR MEMORY: every k-block is written there once by its row's
+// thread (tcgen05.st).
+template <int BITS, bool SWIGLU>
 __global__ void __launch_bounds__(kThreads, 1)
 tc_skinny_q_kernel(const __grid_constant__ CUtensorMap tmP, const __grid_constant__ CUtensorMap tmX, const SkParams p) {
   extern __shared__ uint8_t smem_raw[];
@@ -158,19 +147,16 @@ tc_skinny_q_kernel(const __grid_constant__ CUtensorMap tmP, const __grid_constan
   constexpr int kPBytes = kRowsW * kBlockK * BITS / 8;   // packed bytes of one k-block: 4 KB / 8 KB
   constexpr int kPRow = kBlockK * BITS / 8;              // per row and k-block: 32 B / 64 B
   const int x_bytes = p.m_pad * kBlockK * 2;
-  const int AS = p.stages, PS = p.q_pstages, XS = p.q_xstages, XOWN = p.q_xown;  // TS: AS == 0 (no shared-memory A ring)
-  const int NA = AS > 0 ? AS : 1;                                                // barrier slots of the A hand-off
-  uint8_t* sA = smem;                                            // [AS][128 rows][128 B] swizzled fp16 weight tiles
-  uint8_t* sX = sA + (size_t)AS * kWBytes;                        // [XOWN][m_pad rows][128 B] activation tiles (TMA, swizzled)
+  const int PS = p.q_pstages, XS = p.q_xstages, XOWN = p.q_xown;
+  uint8_t* sX = smem;                                             // [XOWN][m_pad rows][128 B] activation tiles (TMA, swizzled)
   uint8_t* sP = sX + (size_t)XOWN * x_bytes;                      // [PS][128 rows][kPRow] packed weight k-blocks (TMA, dense)
   float* red = reinterpret_cast<float*>(sP + (size_t)PS * kPBytes);  // [split][128][mc] landing buffer of the peers' partial sums
   // Activation stages XOWN .. XS-1 ALIAS the packed-weight region: every packed block has been dequantised (and is dead) before the
   // first activation tile is requested -- the producer waits for `pdone` -- so all XS = min(nkb, ...) activation k-blocks are in
   // flight at once after the dependency resolves, instead of two at a time behind the MMAs (measured: +0.9 us per launch).
   auto x_stage = [&](int xs) -> uint8_t* { return xs < XOWN ? sX + (size_t)xs * x_bytes : sP + (size_t)(xs - XOWN) * x_bytes; };
-  uint64_t* afull = reinterpret_cast<uint64_t*>(red + (size_t)kRowsW * p.m_pad);
-  uint64_t* aempty = afull + NA;
-  uint64_t* xfull = aempty + NA;
+  uint64_t* afull = reinterpret_cast<uint64_t*>(red + (size_t)kRowsW * p.m_pad);  // every k-block of A is in tensor memory
+  uint64_t* xfull = afull + 1;
   uint64_t* xempty = xfull + XS;
   uint64_t* pfull = xempty + XS;   // [0] only: the whole packed slice arrives with one (two: gate | up) tensor load(s)
   uint64_t* pdone = pfull + PS;
@@ -198,7 +184,7 @@ tc_skinny_q_kernel(const __grid_constant__ CUtensorMap tmP, const __grid_constan
   if (threadIdx.x == 0) {
     if (p.trace) p.trace[((size_t)blockIdx.y * gridDim.x + blockIdx.x) * 16 + 0] = sk_globaltimer();
     SK_STAMP(1);
-    for (int s = 0; s < NA; ++s) { mbar_init(&afull[s], 4); mbar_init(&aempty[s], 1); }
+    mbar_init(afull, 4);
     for (int s = 0; s < XS; ++s) { mbar_init(&xfull[s], 1); mbar_init(&xempty[s], 1); }
     for (int s = 0; s < PS; ++s) mbar_init(&pfull[s], 1);
     mbar_init(pdone, 4);
@@ -232,7 +218,7 @@ tc_skinny_q_kernel(const __grid_constant__ CUtensorMap tmP, const __grid_constan
       } else {
         tma_load_2d(sP, &tmP, &pfull[0], kb0 * wpk, n0);
       }
-      sk_wait_dependency_tma(p);
+      pdl_wait();
       int xs = 0;
       uint32_t xph = 1;  // parity of (round - 1): ring positions are wrapping counters, no integer division per k-block
       for (int i = 0; i < nkb; ++i) {
@@ -248,36 +234,21 @@ tc_skinny_q_kernel(const __grid_constant__ CUtensorMap tmP, const __grid_constan
     {  // ---------------- MMA issuer: D[128 weight rows, m_pad activation rows] (+)= W_tile . X^T; warp-uniform loop, one elected lane issues
       const bool lead = elect_one();
       const uint32_t idesc = (1u << 4) | ((uint32_t)(p.m_pad >> 3) << 17) | ((uint32_t)(kRowsW >> 4) << 24);
-      int s = 0, xs = 0;
-      uint32_t aph = 0, xph = 0;
+      int xs = 0;
+      uint32_t xph = 0;
       for (int i = 0; i < nkb; ++i) {
-        if (TS) {
-          if (i == 0) mbar_wait(&afull[0], 0);  // every k-block of A sits in tensor memory
-        } else {
-          mbar_wait(&afull[s], aph);
-        }
+        if (i == 0) mbar_wait(afull, 0);
         mbar_wait(&xfull[xs], xph);
         tc_fence_after();
         if (lead && i == 0) SK_STAMP(3);
         const uint64_t bd = umma_desc(smem_u32(x_stage(xs)));
-        if (TS) {
-          const uint32_t at = tmem_base + (uint32_t)p.m_pad + (uint32_t)i * 32u;  // k-block i: 32 columns = 64 fp16 per lane
-          if (lead) {
+        const uint32_t at = tmem_base + (uint32_t)p.m_pad + (uint32_t)i * 32u;  // k-block i: 32 columns = 64 fp16 per lane
+        if (lead) {
 #pragma unroll
-            for (int k = 0; k < kBlockK / 16; ++k) umma_f16_ts(tmem_base, at + (uint32_t)(8 * k), bd + (uint64_t)(2 * k), idesc, (i | k) != 0 ? 1u : 0u);
-          }
-        } else {
-          const uint64_t ad = umma_desc(smem_u32(sA + (size_t)s * kWBytes));
-          if (lead) {
-#pragma unroll
-            for (int k = 0; k < kBlockK / 16; ++k)
-              umma_f16(tmem_base, ad + (uint64_t)(2 * k), bd + (uint64_t)(2 * k), idesc, (i | k) != 0 ? 1u : 0u);
-            umma_commit(&aempty[s]);
-          }
+          for (int k = 0; k < kBlockK / 16; ++k) umma_f16_ts(tmem_base, at + (uint32_t)(8 * k), bd + (uint64_t)(2 * k), idesc, (i | k) != 0 ? 1u : 0u);
         }
         if (lead && i + XS < nkb) umma_commit(&xempty[xs]);
         if (++xs == XS) { xs = 0; xph ^= 1u; }
-        if (!TS && ++s == NA) { s = 0; aph ^= 1u; }
       }
       if (lead) umma_commit(tmem_full);
     }
@@ -311,10 +282,9 @@ tc_skinny_q_kernel(const __grid_constant__ CUtensorMap tmP, const __grid_constan
     float* my_sb = sb_s + row;  // [2 * group + (0: scale, 1: bias)][128 rows]
     {
       const size_t g_first = srow + (size_t)g_lo;
-      const bool live = row_ok && !(p.q_dbg & 2);
-      if (p.q_sdt == Q3TTS_F32) fill_sb_table<2>(my_sb, p.q_scales, p.q_biases, g_first, ng, live);
-      else if (p.q_sdt == Q3TTS_F16) fill_sb_table<1>(my_sb, p.q_scales, p.q_biases, g_first, ng, live);
-      else fill_sb_table<0>(my_sb, p.q_scales, p.q_biases, g_first, ng, live);
+      if (p.q_sdt == Q3TTS_F32) fill_sb_table<2>(my_sb, p.q_scales, p.q_biases, g_first, ng, row_ok);
+      else if (p.q_sdt == Q3TTS_F16) fill_sb_table<1>(my_sb, p.q_scales, p.q_biases, g_first, ng, row_ok);
+      else fill_sb_table<0>(my_sb, p.q_scales, p.q_biases, g_first, ng, row_ok);
     }
     auto load_sb = [&](int kb, float (&sc)[2], float (&bi)[2]) {  // this thread's own table column: no barrier needed
       const int gi = (kb * gpk) / gdiv - g_lo;
@@ -336,65 +306,36 @@ tc_skinny_q_kernel(const __grid_constant__ CUtensorMap tmP, const __grid_constan
       }
       asm volatile("bar.sync 1, 128;" ::: "memory");
     }
-    const uint32_t arow0 = smem_u32(sA) + (uint32_t)row * 128u;
     const uint32_t prow0 = smem_u32(sP) + (uint32_t)prow * (uint32_t)(PS * kPRow);  // row pitch = the whole slice: PS k-blocks
-    // Every k-block is dequantised NOW, ahead of the dependency on the predecessor kernel: the first AS blocks straight into the A
-    // ring, the rest PARKED in spare TMEM columns (thread = TMEM lane, 32 columns of packed fp16 pairs per block; written and read
-    // back by the same thread with tcgen05.st / tcgen05.ld, so no operand layout is involved).  Once the MMAs release an A stage,
-    // re-staging a parked block is one TMEM load + eight shared-memory stores instead of a dequantisation on the critical path.
-    const uint32_t park0 = tmem_base + ((uint32_t)(q * 32) << 16) + (uint32_t)p.m_pad;
-    const int n_direct = TS ? 0 : AS;  // k-blocks written straight into the shared-memory A ring
+    // Every k-block is dequantised NOW, ahead of the dependency on the predecessor kernel, into its own 32 TMEM columns (thread = TMEM
+    // lane, packed fp16 pairs): k-block i is columns [m_pad + 32 i, +32) of this warp's lanes, the A operand of its MMAs.
+    const uint32_t a0 = tmem_base + ((uint32_t)(q * 32) << 16) + (uint32_t)p.m_pad;
     for (int i = 0; i < nkb; ++i) {
       float sc[2], bi[2];
       load_sb(kb0 + i, sc, bi);
-      if (i == 0) {
-        if (threadIdx.x == 96 && (p.q_dbg & 1)) SK_STAMP(10);
-        mbar_wait(&pfull[0], 0);
-        if (threadIdx.x == 96 && (p.q_dbg & 1)) SK_STAMP(11);
-      }
+      if (i == 0) mbar_wait(&pfull[0], 0);
       uint32_t v[32];
       const float* fold = p.q_fold ? fold_s + i * kBlockK : nullptr;
       if (p.q_sdt == Q3TTS_F32) dequant_row<BITS, true>(prow0 + (uint32_t)i * (uint32_t)kPRow, sc, bi, fold, v);
       else dequant_row<BITS, false>(prow0 + (uint32_t)i * (uint32_t)kPRow, sc, bi, fold, v);
-      if (i < n_direct) {
-        store_row_swizzled(arow0 + (uint32_t)i * (uint32_t)kWBytes, row & 7, v);
-        asm volatile("fence.proxy.async.shared::cta;" ::: "memory");  // generic-proxy stores -> visible to the tensor core's reads
-        __syncwarp();
-        if (lane == 0) mbar_arrive(&afull[i]);
-      } else {
-        tmem_st32(park0 + (uint32_t)(i - n_direct) * 32u, v);  // TS: column block i; SS: parked block i - AS
-      }
-      if (threadIdx.x == 96 && (p.q_dbg & 1) && i < 2) SK_STAMP(12 + i);
+      tmem_st32(a0 + (uint32_t)i * 32u, v);
     }
-    if (nkb > n_direct) tmem_st_wait();
-    if (TS) tc_fence_before();  // the tensor-memory writes are ordered before the barrier the MMA thread waits on
+    if (nkb > 0) tmem_st_wait();
+    tc_fence_before();  // the tensor-memory writes are ordered before the barrier the MMA thread waits on
     __syncwarp();
     if (lane == 0) {
       mbar_arrive(pdone);  // this warp has read its last packed byte
-      if (TS) mbar_arrive(&afull[0]);
+      mbar_arrive(afull);
     }
     if (threadIdx.x == 96) SK_STAMP(14);
-    if (!TS) {
-      for (int i = AS; i < nkb; ++i) {
-        const int s = i % NA;
-        uint32_t v[32];
-        tmem_ld32_issue(park0 + (uint32_t)(i - AS) * 32u, v);
-        mbar_wait(&aempty[s], (uint32_t)(((i / AS) - 1) & 1));  // the MMAs of k-block i - AS have read A[s]
-        tmem_ld_wait32(v);
-        store_row_swizzled(arow0 + (uint32_t)s * (uint32_t)kWBytes, row & 7, v);
-        asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-        __syncwarp();
-        if (lane == 0) mbar_arrive(&afull[s]);
-      }
-    }
-    sk_wait_dependency_warp(p);  // residual rows and the activation rows were written by earlier kernels
+    pdl_wait();  // residual rows and the activation rows were written by earlier kernels
     if (threadIdx.x == 96) SK_STAMP(15);
     if (p.rms_x) sk_row_factors(p, rowscale_s, rank);
     if (p.split > 1) cluster_wait_acquire();  // A: every peer CTA is resident, its mbarriers initialised
     mbar_wait(tmem_full, 0);
     tc_fence_after();
     if (threadIdx.x == 64) SK_STAMP(4);
-    // the A / X rings are free (every MMA of this CTA has completed): they hold the outgoing partial sums
+    // the X ring and the packed region are free (every MMA of this CTA has completed): they hold the outgoing partial sums
     sk_reduce_epilogue<TC_ACT_NONE, SWIGLU>(p, reinterpret_cast<float*>(smem), red, red_full, ack, rowscale_s, tmem_base, rank, n0);
   }
   if (p.split > 1 && warp < 2) cluster_wait_acquire();  // A (the epilogue warps passed it above)
@@ -410,51 +351,32 @@ tc_skinny_q_kernel(const __grid_constant__ CUtensorMap tmP, const __grid_constan
   }
 }
 
-int env_int(const char* name, int dflt) {
-  const char* e = getenv(name);
-  return e ? atoi(e) : dflt;
-}
-
 struct SkqPlan {
-  int m_pad, split, tiles, num_kb, nkb_max, a_stages, x_own, x_stages, tmem_cols, ngm;
+  int m_pad, split, tiles, num_kb, nkb_max, x_own, x_stages, tmem_cols, ngm;
   size_t smem;
   bool ok;
 };
 
-bool ts_mode() {
-  static const bool on = env_int("Q3TTS_SKQ_TS", 1) != 0;
-  return on;
-}
-
 SkqPlan plan(const TcGemm& g) {
-  static const int max_split = std::max(1, std::min(16, env_int("Q3TTS_SK_MAX_SPLIT", 8)));
-  static const int cta_target = env_int("Q3TTS_SK_CTAS", 200);
   SkqPlan s{};
   const int M = g.Bt * g.T;
   s.m_pad = M <= 32 ? 32 : (M <= 64 ? 64 : 128);
   s.tiles = (g.N + kRowsW - 1) / kRowsW;
   s.num_kb = (g.cin + kBlockK - 1) / kBlockK;
-  s.split = 1;  // the SAME rule as gemm_skinny.cu: the K split (= the fp32 summation order) depends on the weight shape only
-  while (s.split * 2 <= max_split && s.tiles * s.split * 2 <= cta_target && s.split * 2 <= s.num_kb && s.m_pad / (s.split * 2) >= 4) s.split *= 2;
+  s.split = k_split(s.tiles, s.num_kb, s.m_pad);
   s.nkb_max = (s.num_kb + s.split - 1) / s.split;
   const int x_bytes = s.m_pad * kBlockK * 2, red_bytes = kRowsW * s.m_pad * 4;
   const int p_bytes = kRowsW * kBlockK * g.q_bits / 8;
   // quantisation groups a CTA's K slice can touch (scale / bias table rows)
   s.ngm = g.q_group == 32 ? 2 * s.nkb_max : (g.q_group == 64 ? s.nkb_max : s.nkb_max / 2 + 1);
-  if (ts_mode()) {  // A from tensor memory: no A ring; the activation stages + the (dead) packed region double as the outgoing staging buffer
-    s.a_stages = 0;
-    s.x_own = 2;
-    while (s.x_own * x_bytes + s.nkb_max * p_bytes < red_bytes) ++s.x_own;
-  } else {
-    s.a_stages = std::min(s.nkb_max, s.m_pad <= 32 ? 3 : 2);
-    while (s.a_stages * (kWBytes + x_bytes) < red_bytes) ++s.a_stages;  // the rings double as the outgoing staging buffer
-    s.x_own = s.a_stages;                                                                // activation stages of their own ...
-  }
+  // the activation stages + the (dead) packed region double as the outgoing staging buffer
+  s.x_own = 2;                                                                             // activation stages of their own ...
+  while (s.x_own * x_bytes + s.nkb_max * p_bytes < red_bytes) ++s.x_own;
   s.x_stages = std::min(s.nkb_max, s.x_own + (s.nkb_max * p_bytes) / x_bytes);           // ... plus those that alias the packed region
-  s.smem = (size_t)s.a_stages * kWBytes + (size_t)s.x_own * x_bytes + (size_t)s.nkb_max * p_bytes + red_bytes + 1024 +
-           (size_t)(2 * std::max(1, s.a_stages) + 2 * s.x_stages + s.nkb_max + 4) * 8 + 16 + kRowsW * 4 + (size_t)s.nkb_max * kBlockK * 4 + (size_t)2 * s.ngm * kRowsW * 4 + 64;
-  // TMEM: the fp32 accumulator [128 lanes x m_pad columns] + 32 columns per k-block parked beyond the A ring
-  int cols = s.m_pad + 32 * std::max(0, s.nkb_max - s.a_stages);  // TS: every k-block lives in tensor memory
+  s.smem = (size_t)s.x_own * x_bytes + (size_t)s.nkb_max * p_bytes + red_bytes + 1024 +
+           (size_t)(1 + 2 * s.x_stages + s.nkb_max + 4) * 8 + 16 + kRowsW * 4 + (size_t)s.nkb_max * kBlockK * 4 + (size_t)2 * s.ngm * kRowsW * 4 + 64;
+  // TMEM: the fp32 accumulator [128 lanes x m_pad columns] + 32 columns per k-block of the dequantised A operand
+  int cols = s.m_pad + 32 * s.nkb_max;
   s.tmem_cols = 32;
   while (s.tmem_cols < cols) s.tmem_cols <<= 1;
   // the packed slice is one TMA box: <= 256 elements in the inner dimension
@@ -463,13 +385,9 @@ SkqPlan plan(const TcGemm& g) {
 }
 
 using SkqKernel = void (*)(const CUtensorMap, const CUtensorMap, const SkParams);
-SkqKernel pick_kernel(int bits, int swiglu, bool ts) {
-  if (ts) {
-    if (bits == 4) return swiglu ? tc_skinny_q_kernel<4, true, true> : tc_skinny_q_kernel<4, false, true>;
-    return swiglu ? tc_skinny_q_kernel<8, true, true> : tc_skinny_q_kernel<8, false, true>;
-  }
-  if (bits == 4) return swiglu ? tc_skinny_q_kernel<4, true, false> : tc_skinny_q_kernel<4, false, false>;
-  return swiglu ? tc_skinny_q_kernel<8, true, false> : tc_skinny_q_kernel<8, false, false>;
+SkqKernel pick_kernel(int bits, int swiglu) {
+  if (bits == 4) return swiglu ? tc_skinny_q_kernel<4, true> : tc_skinny_q_kernel<4, false>;
+  return swiglu ? tc_skinny_q_kernel<8, true> : tc_skinny_q_kernel<8, false>;
 }
 
 CUtensorMap make_packed_map(const void* base, uint64_t words_per_row, uint64_t rows, uint32_t box_words, uint32_t box_rows) {
@@ -491,7 +409,7 @@ bool tc_skinny_q_supported(const TcGemm& g) {
   if (!g.q_w || !(g.q_bits == 4 || g.q_bits == 8)) return false;
   if (!(g.q_group == 32 || g.q_group == 64 || g.q_group == 128)) return false;
   const long long M = (long long)g.Bt * g.T;
-  if (!(tc_skinny_enabled() && g.allow_skinny && !g.res16 && !g.outr16 && g.ntap == 1 && M >= 1 && M <= 128 && !g.snake_ea && !g.pcm)) return false;
+  if (!(g.allow_skinny && !g.res16 && !g.outr16 && g.ntap == 1 && M >= 1 && M <= 128 && !g.snake_ea && !g.pcm)) return false;
   if (g.act != TC_ACT_NONE || g.row_scale) return false;
   if (g.cin % kBlockK != 0 || g.cin % g.q_group != 0 || g.N % 32 != 0) return false;
   if (g.q_halves && (!g.swiglu || (g.N / 2) % (kRowsW / 2) != 0)) return false;
@@ -502,11 +420,10 @@ bool tc_skinny_q_supported(const TcGemm& g) {
 void init_tc_skinny_q() {
   tc_resolve_encode();
   for (int bits : {4, 8})
-    for (int sw : {0, 1})
-      for (bool ts : {false, true}) {
-        Q3_CUDA(cudaFuncSetAttribute(pick_kernel(bits, sw, ts), cudaFuncAttributeMaxDynamicSharedMemorySize, 220 * 1024));
-        Q3_CUDA(cudaFuncSetAttribute(pick_kernel(bits, sw, ts), cudaFuncAttributeNonPortableClusterSizeAllowed, 1));
-      }
+    for (int sw : {0, 1}) {
+      Q3_CUDA(cudaFuncSetAttribute(pick_kernel(bits, sw), cudaFuncAttributeMaxDynamicSharedMemorySize, 220 * 1024));
+      Q3_CUDA(cudaFuncSetAttribute(pick_kernel(bits, sw), cudaFuncAttributeNonPortableClusterSizeAllowed, 1));
+    }
 }
 
 void launch_tc_skinny_q(const LaunchCtx& c, const TcGemm& g) {
@@ -516,7 +433,7 @@ void launch_tc_skinny_q(const LaunchCtx& c, const TcGemm& g) {
   const SkqPlan s = plan(g);
   SkParams p{};
   p.M = g.Bt * g.T; p.N = g.N; p.K = g.cin;
-  p.m_pad = s.m_pad; p.split = s.split; p.mc = s.m_pad / s.split; p.stages = s.a_stages; p.num_kb = s.num_kb;
+  p.m_pad = s.m_pad; p.split = s.split; p.mc = s.m_pad / s.split; p.num_kb = s.num_kb;
   p.mc_shift = 0;
   while ((1 << p.mc_shift) < p.mc) ++p.mc_shift;
   p.split_shift = 0;
@@ -528,15 +445,10 @@ void launch_tc_skinny_q(const LaunchCtx& c, const TcGemm& g) {
   p.rms_x = g.rms_in ? g.a : nullptr;
   p.rms_a = 1.0f / (g.in_scale * g.in_scale * (float)g.cin); p.rms_eps = g.rms_eps; p.rms_mult = 1.0f / g.in_scale;
   p.trace = tc_skinny_trace_buf();
-  p.sig = c.chain_link((unsigned)(s.tiles * s.split));
   p.q_scales = g.q_scales; p.q_biases = g.q_biases; p.q_fold = g.q_fold; p.q_group = g.q_group; p.q_sdt = g.q_sdt;
   p.q_pstages = s.nkb_max;
   p.q_xstages = s.x_stages; p.q_xown = s.x_own;
   p.q_half_rows = g.q_halves ? g.N / 2 : 0;
-  {
-    static const int dbg = [] { const char* e = getenv("Q3TTS_SKQ_DBG"); return e ? atoi(e) : 0; }();
-    p.q_dbg = dbg;
-  }
 
   const uint32_t wpk = (uint32_t)(kBlockK * g.q_bits / 32) * (uint32_t)s.nkb_max;  // one box = the whole K slice of a row
   const CUtensorMap mp = make_packed_map(g.q_w, (uint64_t)g.cin * g.q_bits / 32, (uint64_t)g.N, wpk, (uint32_t)(g.q_halves ? kRowsW / 2 : kRowsW));
@@ -564,8 +476,8 @@ void launch_tc_skinny_q(const LaunchCtx& c, const TcGemm& g) {
   }
   cfg.attrs = attr;
   cfg.numAttrs = na;
-  Q3_CUDA(cudaLaunchKernelEx(&cfg, pick_kernel(g.q_bits, g.swiglu, ts_mode()), mp, mx, p));
-  c.tick_chained();
+  Q3_CUDA(cudaLaunchKernelEx(&cfg, pick_kernel(g.q_bits, g.swiglu), mp, mx, p));
+  c.tick();
 }
 
 }  // namespace q3

@@ -23,10 +23,9 @@ using namespace tcptx;
 constexpr int kTileM = 128;
 constexpr int kBlockK = 64;                       // fp16 elements per k-block = one 128-byte swizzle row
 constexpr int kABytes = kTileM * kBlockK * 2;     // 16 KB per stage
-constexpr int kHaloRowsMax = 192;                 // halo mode: 128 + (ntap - 1) * dil rows <= 192
-constexpr int kHaloBytes = kHaloRowsMax * kBlockK * 2;  // 24 KB per activation stage
-constexpr int kThreads = 192;      // warps 0-1 + one set of 4 epilogue warps
-constexpr int kMaxThreads = 448;   // ... up to three sets (persistent schedule)
+constexpr int kMaxEpiSets = 3;                            // sets of 4 epilogue warps (persistent schedule)
+constexpr int kMaxThreads = 64 + 128 * kMaxEpiSets;       // warps 0-1 + the epilogue sets
+constexpr int kPersistMinTiles = 4;                       // tiles per resident CTA from which the schedule is persistent
 
 // Ring position as counters that wrap (stage, parity of the round) instead of `it % stages` / `(it / stages) & 1`: a runtime integer
 // division is ~35 dependent instructions, and one or two per k-block in the single MMA-issuing (or TMA-issuing) thread cost more than
@@ -71,10 +70,6 @@ struct TcParams {
   const __half* res16;
   __half* outr16;
   int epi_sets;  // sets of 4 epilogue warps; set e handles the 32-column chunks e, e + epi_sets, ... of every tile
-  // halo mode (ntap > 1): ONE activation tile of 128 + (ntap-1)*dil rows per channel block feeds all taps -- tap t reads rows
-  // [t*dil, t*dil + 128) of it through a UMMA descriptor whose start address is shifted by whole 128-byte rows -- instead of one
-  // shifted 128-row TMA box per tap (ntap x the L2 -> SM traffic for the activations).
-  int halo, a_stages, b_stages, halo_rows;
   // residual ring (fp16 residual stream, classic schedule): the [128 rows x bn] residual tile of a tile is fetched by the TMA producer
   // res_stages tiles ahead of the epilogue that adds it.  Per-thread residual loads kept ONE 2 KB batch per epilogue warp in flight
   // (12 warps x 2 KB / ~1.2 us of DRAM latency = 20 GB/s per SM -- exactly what the 1x1 convolutions of the vocoder ran at, 30-45 %
@@ -94,15 +89,13 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~(uintptr_t)1023);  // SWIZZLE_128B: 1024-B aligned
   const int b_bytes = p.bn * kBlockK * 2;
-  const int a_stage_bytes = p.halo ? kHaloBytes : kABytes;
-  const int a_st = p.halo ? p.a_stages : p.stages, b_st = p.halo ? p.b_stages : p.stages;
   uint8_t* sA = smem;
-  uint8_t* sB = smem + (size_t)a_st * a_stage_bytes;
-  // classic: full[s] / empty[s] guard stage s of both rings.  halo: full/empty[0, a_st) guard the A ring, [a_st, a_st + b_st) the B ring
-  uint8_t* sR = sB + (size_t)b_st * b_bytes;   // [res_stages][128 rows][bn] fp16 residual tiles (dense rows, no swizzle)
+  uint8_t* sB = smem + (size_t)p.stages * kABytes;
+  // full[s] / empty[s] guard stage s of both rings
+  uint8_t* sR = sB + (size_t)p.stages * b_bytes;   // [res_stages][128 rows][bn] fp16 residual tiles (dense rows, no swizzle)
   uint64_t* full = reinterpret_cast<uint64_t*>(sR + (size_t)p.res_stages * p.res_bytes);
-  uint64_t* empty = full + (p.halo ? a_st + b_st : p.stages);
-  uint64_t* tmem_full = empty + (p.halo ? a_st + b_st : p.stages);   // [2]
+  uint64_t* empty = full + p.stages;
+  uint64_t* tmem_full = empty + p.stages;   // [2]
   uint64_t* tmem_empty = tmem_full + 2;     // [2]
   uint64_t* rfull = tmem_empty + 2;         // [res_stages]
   uint64_t* rempty = rfull + p.res_stages;  // [res_stages]
@@ -136,7 +129,7 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
   }
   pdl_launch_dependents();  // the next kernel of the stream may start its prologue / weight prefetch now
   if (threadIdx.x == 0) {
-    for (int s = 0; s < (p.halo ? a_st + b_st : p.stages); ++s) { mbar_init(&full[s], 1); mbar_init(&empty[s], 1); }
+    for (int s = 0; s < p.stages; ++s) { mbar_init(&full[s], 1); mbar_init(&empty[s], 1); }
     mbar_init(&tmem_full[0], 1); mbar_init(&tmem_full[1], 1);
     mbar_init(&tmem_empty[0], 4 * p.epi_sets); mbar_init(&tmem_empty[1], 4 * p.epi_sets);  // one arrival per epilogue warp
     for (int s = 0; s < p.res_stages; ++s) { mbar_init(&rfull[s], 1); mbar_init(&rempty[s], 4 * p.epi_sets); }
@@ -160,42 +153,6 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
       // dependency is resolved, so the weight stream overlaps the predecessor's tail; activations (A) follow the wait.
       // Every CTA of a column of the grid reads the SAME activation tiles: walking K from a per-CTA offset keeps the CTAs
       // off each other's L2 lines (same-address storms serialise in one L2 slice and multiply the TMA latency).
-      if (p.halo) {
-        const uint32_t a_tx = (uint32_t)(p.halo_rows * kBlockK * 2);
-        uint64_t *a_full = full, *a_empty = empty, *b_full = full + a_st, *b_empty = empty + a_st;
-        TcRing ra(a_st), rb(b_st);  // activation / weight rings
-        bool waited = false;
-        for (int tile = blockIdx.x; tile < total_tiles; tile += gridDim.x) {
-          const int m_tile = fast_div(tile, p.div_n_mul, p.div_n_shift), n_tile = tile - m_tile * p.tiles_n;
-          const int bidx = fast_div(m_tile, p.div_b_mul, p.div_b_shift), t0 = (m_tile - bidx * p.tiles_per_batch) * kTileM, n0 = n_tile * p.bn;
-          for (int kc = 0; kc < p.kb_per_tap; ++kc) {
-            auto issue_b = [&](int tap) {
-              if (rb.wrapped) mbar_wait(&b_empty[rb.s], rb.ph ^ 1u);
-              if (lead) {
-                mbar_expect_tx(&b_full[rb.s], (uint32_t)b_bytes);
-                tma_load_3d(sB + (size_t)rb.s * b_bytes, &tmB, &b_full[rb.s], kc * kBlockK, tap * p.N + n0, w_rep);
-              }
-              rb.next();
-            };
-            int tap0 = 0;
-            if (!waited) {  // the very first weight tiles are requested before the programmatic dependency resolves
-              const int pre = b_st < p.ntap ? b_st : p.ntap;
-              for (; tap0 < pre; ++tap0) issue_b(tap0);
-              pdl_wait();
-              waited = true;
-            }
-            // the activation tile goes out BEFORE the weight tiles that may have to wait for a free stage (the MMA issuer
-            // releases weight stages only once it also holds the activation tile)
-            if (ra.wrapped) mbar_wait(&a_empty[ra.s], ra.ph ^ 1u);
-            if (lead) {
-              mbar_expect_tx(&a_full[ra.s], a_tx);
-              tma_load_3d(sA + (size_t)ra.s * kHaloBytes, &tmA, &a_full[ra.s], kc * kBlockK, t0 - (p.ntap - 1) * p.dil, bidx);
-            }
-            ra.next();
-            for (int tap = tap0; tap < p.ntap; ++tap) issue_b(tap);
-          }
-        }
-      } else {
       TcRing rg(p.stages);  // the ring does not care about tile boundaries
       int rt = 0;  // residual tiles issued so far (tile sequence numbers of this CTA)
       // residual tiles of this CTA's tiles [rt, upto].  blocking: wait for a stage's previous tenant to be consumed (only ever for the
@@ -257,14 +214,13 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
           if (++kcb == p.kb_per_tap) { kcb = 0; if (++tap == p.ntap) tap = 0; }
         }
       }
-      }  // classic schedule
     }
   } else if (warp == 1) {
     {  // ---------------- MMA issuer: the whole warp walks the loop (uniform registers), one elected lane issues (tc_ptx.cuh elect_one)
       const bool lead = elect_one();
       // instruction descriptor (cute::UMMA::InstrDescriptor): c = F32 (bit 4), a = b = F16 (0), K-major both, N>>3 at bit 17, M>>4 at bit 24
       const uint32_t idesc = (1u << 4) | ((uint32_t)(p.bn >> 3) << 17) | ((uint32_t)(kTileM >> 4) << 24);
-      TcRing rg(p.halo ? a_st : p.stages), rb(b_st);  // classic: rg = the one ring; halo: rg = activation ring, rb = weight ring
+      TcRing rg(p.stages);
       const uint32_t sA0 = smem_u32(sA), sB0 = smem_u32(sB);
       for (int tile = blockIdx.x, ti = 0; tile < total_tiles; tile += gridDim.x, ++ti) {
         const int a = p.n_acc == 2 ? (ti & 1) : 0, use = p.n_acc == 2 ? (ti >> 1) : ti;
@@ -273,32 +229,6 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
           tc_fence_after();
         }
         const uint32_t acc = tmem_base + (uint32_t)(a * p.acc_cols);
-        if (p.halo) {
-          uint64_t *a_full = full, *a_empty = empty, *b_full = full + a_st, *b_empty = empty + a_st;
-          for (int kc = 0; kc < p.kb_per_tap; ++kc) {
-            const int sa = rg.s;
-            // the weight stages of this channel block arrive first (the producer issues them first), then the halo tile
-            for (int tap = 0; tap < p.ntap; ++tap) {
-              const int sb = rb.s;
-              mbar_wait(&b_full[sb], rb.ph);
-              if (tap == 0) mbar_wait(&a_full[sa], rg.ph);
-              tc_fence_after();
-              const uint64_t ad = umma_desc_rows(sA0 + (uint32_t)sa * (uint32_t)kHaloBytes + (uint32_t)(tap * p.dil) * 128u);
-              const uint64_t bd = umma_desc(sB0 + (uint32_t)sb * (uint32_t)b_bytes);
-              if (lead) {
-#pragma unroll
-                for (int k = 0; k < kBlockK / 16; ++k)
-                  umma_f16(acc, ad + (uint64_t)(2 * k), bd + (uint64_t)(2 * k), idesc, (kc | tap | k) != 0 ? 1u : 0u);
-                umma_commit(&b_empty[sb]);
-              }
-              rb.next();
-            }
-            if (lead) umma_commit(&a_empty[sa]);
-            rg.next();
-          }
-          if (lead) umma_commit(&tmem_full[a]);
-          continue;
-        }
         for (int kb = 0; kb < num_kb; ++kb) {
           const int s = rg.s;
           mbar_wait(&full[s], rg.ph);
@@ -626,42 +556,24 @@ void launch_tc_gemm(const LaunchCtx& c, const TcGemm& g) {
   // Persistent schedule for grids of many tiles (the codec's thin-channel stages launch up to 25 000): per-CTA set-up / tear-down
   // and the exposed epilogue of a one-tile CTA (a 128 x 96 tile lived ~14 us for ~2 us of MMA) are paid once per SM instead of
   // once per tile.
-  static const int persist_min = [] { const char* e = getenv("Q3TTS_TC_PERSIST_MIN_TILES"); return e ? atoi(e) : 4; }();
-  static const int persist_two = [] { const char* e = getenv("Q3TTS_TC_PERSIST_2CTA"); return e ? atoi(e) : 0; }();
-  const int ctas_per_sm = (persist_two && 4 * cols <= 512) ? 2 : 1;  // default: one CTA per SM with up to 3 sets of epilogue warps
-  const long long resident = 148LL * ctas_per_sm;
-  const bool persistent = persist_min > 0 && tiles >= persist_min * resident;
+  // A persistent grid is one CTA per SM with up to kMaxEpiSets sets of epilogue warps.
+  const long long resident = 148;
+  const bool persistent = tiles >= kPersistMinTiles * resident;
   p.n_acc = persistent ? 2 : 1;
   p.tmem_cols = cols * p.n_acc;
   // The epilogue (TMEM -> registers -> bias / activation / SnakeBeta / residual -> global) is the latency-bound pipe of the thin
   // stages (ncu: 3 active warps per scheduler, 0.25 eligible): a persistent CTA gets up to three sets of epilogue warps, each
   // taking every third 32-column chunk of a tile.
-  static const int max_sets = [] { const char* e = getenv("Q3TTS_TC_EPI_SETS"); return e ? std::max(1, std::min(3, atoi(e))) : 3; }();
-  p.epi_sets = (persistent && ctas_per_sm == 1) ? std::max(1, std::min(max_sets, p.bn / 32)) : 1;
-  // Bytes in flight per SM bound a latency-limited K loop: big grids run 2 CTAs/SM with ~100 KB rings each, small grids
-  // (one CTA per SM at most) take the whole shared memory for one deep ring.
-  static const bool tio_on = [] { const char* e = getenv("Q3TTS_TC_TIO"); return !(e && atoi(e) == 0); }();
-  p.tio = tio_on && (g.out16 || g.outr16) && !g.swiglu && !g.res && !g.out32 && !g.pcm && g.N % 32 == 0 && g.ld16 % 8 == 0 && (!g.outr16 || g.ld32 % 8 == 0) &&
+  p.epi_sets = persistent ? std::max(1, std::min(kMaxEpiSets, p.bn / 32)) : 1;
+  // Bytes in flight per SM bound a latency-limited K loop: big one-tile-per-CTA grids run 2 CTAs/SM with ~100 KB rings each, small
+  // grids and persistent ones (one CTA per SM at most) take the whole shared memory for one deep ring.
+  p.tio = (g.out16 || g.outr16) && !g.swiglu && !g.res && !g.out32 && !g.pcm && g.N % 32 == 0 && g.ld16 % 8 == 0 && (!g.outr16 || g.ld32 % 8 == 0) &&
           (!g.res16 || g.ld_res % 8 == 0);
   const int tio_bytes = p.tio ? 256 + 4 * p.epi_sets * epiio::kPatchBytes : 0;
-  const int ring_budget = ((persistent ? ctas_per_sm == 2 : tiles > 148) ? 100 * 1024 : 200 * 1024) - tio_bytes;
+  const int ring_budget = ((!persistent && tiles > 148) ? 100 * 1024 : 200 * 1024) - tio_bytes;
   p.stages = std::max(2, std::min(12, ring_budget / stage_bytes));
   if (!persistent) p.stages = std::min(p.stages, std::max(2, g.ntap * p.kb_per_tap));
-  // halo mode for multi-tap convolutions whose 128 + (ntap-1)*dil rows fit a 192-row stage.  Opt-in (Q3TTS_TC_HALO=1): exact on
-  // every multi-tap test shape, but on B200 a 64 x 26-frame codec pass ran 18.6 ms with it against 17.9 ms without -- the
-  // vocoder stages are bound by their epilogues, not by the 7x activation re-read it removes.
-  static const bool halo_on = [] { const char* e = getenv("Q3TTS_TC_HALO"); return e && atoi(e) != 0; }();
-  p.halo_rows = kTileM + (g.ntap - 1) * g.dil;
-  p.halo = halo_on && g.ntap > 1 && p.halo_rows <= kHaloRowsMax;
   int ring_bytes = p.stages * stage_bytes;
-  if (p.halo) {
-    const int b_bytes = p.bn * kBlockK * 2;
-    p.a_stages = std::max(2, std::min(4, p.kb_per_tap * (persistent ? 2 : 1)));
-    p.a_stages = std::min(p.a_stages, std::max(1, (ring_budget / 3) / kHaloBytes));
-    p.b_stages = std::max(2, std::min(16, (ring_budget - p.a_stages * kHaloBytes) / b_bytes));
-    if (!persistent) p.b_stages = std::min(p.b_stages, g.ntap * p.kb_per_tap);
-    ring_bytes = p.a_stages * kHaloBytes + p.b_stages * b_bytes;
-  }
   p.bias = g.bias; p.res = g.res; p.ld_res = g.ld_res; p.scale = g.scale; p.act = g.act; p.swiglu = g.swiglu;
   p.out32 = g.out32; p.ld32 = g.ld32; p.out16 = g.out16; p.ld16 = g.ld16;
   p.snake_ea = g.snake_ea; p.snake_ieb = g.snake_ieb; p.snake_ch = g.snake_ch > 0 ? g.snake_ch : 1;
@@ -670,9 +582,8 @@ void launch_tc_gemm(const LaunchCtx& c, const TcGemm& g) {
   p.k_rotate = g.k_rotate;
   p.res16 = g.res16; p.outr16 = g.outr16;
   // residual ring: persistent classic schedule, fp16 residual stream, no SwiGLU column pairing
-  static const bool res_ring_on = [] { const char* e = getenv("Q3TTS_TC_RES_RING"); return !(e && atoi(e) == 0); }();
   p.res_stages = 0; p.res_bytes = kTileM * p.bn * 2;
-  if (res_ring_on && !p.tio && g.res16 && persistent && !p.halo && !g.swiglu && p.bn % 8 == 0 && g.N % p.bn == 0) {
+  if (!p.tio && g.res16 && persistent && !g.swiglu && p.bn % 8 == 0 && g.N % p.bn == 0) {
     int rs = std::max(1, std::min(4, (ring_budget / 2) / p.res_bytes));
     int st = (ring_budget - rs * p.res_bytes) / stage_bytes;
     if (st >= 2) { p.res_stages = rs; p.stages = std::min(p.stages, st); ring_bytes = p.stages * stage_bytes; }
@@ -681,7 +592,7 @@ void launch_tc_gemm(const LaunchCtx& c, const TcGemm& g) {
 
   const uint64_t adims[3] = {(uint64_t)g.cin, (uint64_t)g.T, (uint64_t)g.Bt};
   const uint64_t astr[2] = {(uint64_t)g.cin * 2, (uint64_t)g.T * g.cin * 2};
-  const uint32_t abox[3] = {(uint32_t)kBlockK, (uint32_t)(p.halo ? p.halo_rows : kTileM), 1};
+  const uint32_t abox[3] = {(uint32_t)kBlockK, (uint32_t)kTileM, 1};
   const CUtensorMap ma = tc_make_map(g.a, 3, adims, astr, abox);
   p.w_reps = std::max(1, g.w_reps);
   const uint64_t bdims[3] = {(uint64_t)g.cin, (uint64_t)g.ntap * g.N, (uint64_t)p.w_reps};
@@ -701,7 +612,7 @@ void launch_tc_gemm(const LaunchCtx& c, const TcGemm& g) {
   }
   const size_t smem = (size_t)ring_bytes + (size_t)p.res_stages * p.res_bytes + 1024 + 64 * 8 + (size_t)tio_bytes;
   Q3_CHECK(smem <= 212 * 1024, Q3TTS_ERR_CAPACITY, "tc_gemm: shared memory request %zu too large", smem);
-  Q3_CHECK(2 * (p.halo ? p.a_stages + p.b_stages : p.stages) + 5 + 2 * p.res_stages <= 64, Q3TTS_ERR_CAPACITY, "tc_gemm: too many ring stages");
+  Q3_CHECK(2 * p.stages + 5 + 2 * p.res_stages <= 64, Q3TTS_ERR_CAPACITY, "tc_gemm: too many ring stages");
   dim3 grid((unsigned)(persistent ? std::min<long long>(tiles, resident) : tiles));
   launch_kernel_pdl(tc_gemm_kernel, grid, dim3(64 + 128 * p.epi_sets), smem, c.stream, pdl_enabled(), ma, mb, mr, p);
   c.tick();

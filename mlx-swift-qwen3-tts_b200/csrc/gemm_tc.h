@@ -107,6 +107,5 @@ void launch_rmsnorm_f16(const LaunchCtx& c, const float* x, int ldx, int m, int 
 void launch_scale_to_f16(const LaunchCtx& c, const float* x, size_t n, float scale, __half* y);
 // rs[m] = (1 / in_scale) * rsqrt(sum(a[m][:]^2) / (in_scale^2 * dim) + eps) for fp16 rows a = fp16(x * in_scale)
 void launch_row_scale(const LaunchCtx& c, const __half* a, int m, int dim, float in_scale, float eps, float* rs);
-bool tc_skinny_enabled();  // Q3TTS_SKINNY != 0
 
 }  // namespace q3

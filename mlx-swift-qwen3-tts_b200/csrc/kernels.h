@@ -9,19 +9,7 @@ namespace q3 {
 struct LaunchCtx {
   cudaStream_t stream = nullptr;
   LaunchCounter* counter = nullptr;
-  ChainState* chain = nullptr;   // non-null while a decode step is being issued with chain signals (common.h)
-  // a launch that does not signal breaks the chain: its successor falls back to griddepcontrol.wait / stream order
-  inline void tick() const { if (counter) counter->tick(); if (chain) chain->prev = nullptr; }
-  // chained launchers: call chain_link BEFORE the launch (grid size in CTAs), tick_chained after it
-  inline ChainSig chain_link(unsigned ctas) const {
-    ChainSig s;
-    if (!chain || chain->next >= chain->capacity) { if (chain) chain->prev = nullptr; return s; }
-    s.in = chain->prev; s.in_target = chain->prev_ctas;
-    s.out = chain->base + chain->next++;
-    chain->prev = s.out; chain->prev_ctas = ctas;
-    return s;
-  }
-  inline void tick_chained() const { if (counter) counter->tick(); }
+  inline void tick() const { if (counter) counter->tick(); }
 };
 
 enum Epilogue { EPI_STORE = 0, EPI_ADD = 1, EPI_SILU = 2, EPI_SWIGLU = 3 };

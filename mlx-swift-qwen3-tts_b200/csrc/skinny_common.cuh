@@ -1,5 +1,5 @@
 // Pieces shared by the two <= 128-row split-K cluster GEMMs (gemm_skinny.cu: fp16 dense weights through TMA; gemm_skinny_q.cu:
-// MLX-packed 4/8-bit weights dequantised inside the kernel): parameter block, trace hooks, epilogue.
+// MLX-packed 4/8-bit weights dequantised inside the kernel): K split, parameter block, trace hooks, epilogue.
 #pragma once
 #include <cuda.h>
 
@@ -15,6 +15,18 @@ constexpr int kRowsW = 128;                     // weight rows per CTA = UMMA M
 constexpr int kBlockK = 64;                     // fp16 elements per k-block = one 128-byte swizzle row
 constexpr int kWBytes = kRowsW * kBlockK * 2;   // 16 KB of fp16 weights per stage
 constexpr int kThreads = 192;
+constexpr int kMaxSplit = 8;                    // K slices = cluster size; > 8 is a non-portable cluster size (B200 allows 16)
+// up to ~1.3 waves: 48 weight tiles (gate|up) take 4 K slices = 192 CTAs of 4 k-blocks (two co-resident per SM on 44 SMs)
+// rather than 96 CTAs of 8 k-blocks; measured 13.5 -> ~9 us per launch at 64 rows
+constexpr int kCtaTarget = 200;
+
+// The K split (= the fp32 summation order of the partial sums) of both kernels: it depends on the weight shape and the row bucket
+// only, so the packed-weight kernel and the fp16-copy kernel produce the same bits.
+inline int k_split(int tiles, int num_kb, int m_pad) {
+  int split = 1;
+  while (split * 2 <= kMaxSplit && tiles * split * 2 <= kCtaTarget && split * 2 <= num_kb && m_pad / (split * 2) >= 4) split *= 2;
+  return split;
+}
 
 struct SkParams {
   int M, N, K;
@@ -32,7 +44,6 @@ struct SkParams {
   const __half* rms_x;      // folded RMSNorm: fp16 activation rows [M][K] (= the B operand), or null
   float rms_a, rms_eps, rms_mult;  // row factor = rms_mult * rsqrt(sum(x16^2) * rms_a + rms_eps)
   unsigned long long* trace;  // measurement hook (q3tts_skinny_trace): 16 stamps per CTA, or null
-  ChainSig sig;               // chain signals (common.h): flag hand-off from / to the neighbouring launches of a decode step
   // ---- packed-weight kernel only (gemm_skinny_q.cu)
   const void* q_scales;     // [N][K / q_group] of q_sdt
   const void* q_biases;
@@ -42,7 +53,6 @@ struct SkParams {
   int q_xstages, q_xown;    // activation stages in total / outside the (dead after dequantisation) packed region
   int q_half_rows;          // SwiGLU over a [gate ; up] matrix: rows of one half (N / 2); tile row 2i = gate i, 2i + 1 = up i.  0: plain rows
   int split_shift;          // log2(split)
-  int q_dbg;                // measurement only (Q3TTS_SKQ_DBG): bit 0 = stamps 10-13 follow the dequantisation instead of the epilogue
 };
 
 __device__ __forceinline__ unsigned long long sk_globaltimer() {
@@ -50,7 +60,6 @@ __device__ __forceinline__ unsigned long long sk_globaltimer() {
   asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
   return t;
 }
-#define SK_STAMP_EPI(slot) do { if (!(p.q_dbg & 1)) SK_STAMP(slot); } while (0)
 #define SK_STAMP(slot)                                                                                        \
   do {                                                                                                        \
     if (p.trace) p.trace[((size_t)blockIdx.y * gridDim.x + blockIdx.x) * 16 + (slot)] = (unsigned long long)clock64(); \
@@ -166,7 +175,7 @@ __device__ __forceinline__ void sk_reduce_epilogue(const SkParams& p, float* sta
     sk_load_res<16>(p, r16, lane_out ? valid0 : 0, m_base, so);
   }
   if (p.split > 1) mbar_wait(red_full, 0);  // the other K slices of MY activation rows have landed
-  if (threadIdx.x == 96) SK_STAMP_EPI(10);
+  if (threadIdx.x == 96) SK_STAMP(10);
   if (threadIdx.x == 64) {
     SK_STAMP(6);
     // tell every peer that its copy into this CTA is complete (it may retire its staging buffer / exit)
@@ -188,40 +197,18 @@ __device__ __forceinline__ void sk_reduce_epilogue(const SkParams& p, float* sta
         }
       }
     }
-    if (threadIdx.x == 96 && cb == 0) SK_STAMP_EPI(11);
+    if (threadIdx.x == 96 && cb == 0) SK_STAMP(11);
     int valid = p.M - (m_base + cb);
     valid = valid < nc ? valid : nc;
     if (!lane_out) valid = 0;
     if (cb > 0) sk_load_res<16>(p, r16, valid, m_base + cb, so);
     sk_finish<16, ACT, SWIGLU>(p, a16, r16, valid, m_base + cb, so, bias, scale, p.rms_x ? rowscale_s + cb : nullptr);
-    if (threadIdx.x == 96 && cb == 0) SK_STAMP_EPI(12);
+    if (threadIdx.x == 96 && cb == 0) SK_STAMP(12);
   }
-  if (threadIdx.x == 96) SK_STAMP_EPI(13);
-  if (p.sig.out) {  // every global store (and every global read) of this CTA is done: hand over to the next launch
-    asm volatile("bar.sync 1, 128;" ::: "memory");
-    if (threadIdx.x == 64) chain_signal(p.sig.out);
-  }
+  if (threadIdx.x == 96) SK_STAMP(13);
   if (threadIdx.x == 64 && p.split > 1) {
     SK_STAMP(7);
     mbar_wait(ack, 0);  // every peer has received my partial sums: my staging buffer is no longer being read
-  }
-}
-
-// the dependency on the predecessor launch: its chain signal when there is one, else programmatic-dependent-launch completion
-__device__ __forceinline__ void sk_wait_dependency_warp(const SkParams& p) {  // a whole warp
-  if (p.sig.in) {
-    if ((threadIdx.x & 31) == 0) chain_wait(p.sig.in, p.sig.in_target);
-    __syncwarp();
-  } else {
-    pdl_wait();
-  }
-}
-__device__ __forceinline__ void sk_wait_dependency_tma(const SkParams& p) {  // the single TMA-issuing thread
-  if (p.sig.in) {
-    chain_wait(p.sig.in, p.sig.in_target);
-    asm volatile("fence.proxy.async;" ::: "memory");  // the tensor loads that follow (async proxy) are ordered after the acquire
-  } else {
-    pdl_wait();
   }
 }
 

@@ -33,11 +33,10 @@ TalkerEngine::TalkerEngine(const std::string& model_dir, const TalkerConfig& cfg
   kv_layer_stride_ = (size_t)T.kv_heads * C * 128;
   kv_slot_stride_ = kv_layer_stride_ * T.layers;
   // decided here (before the tensor-core copies exist) from the same inputs handle_tc_ is decided from below
+  if (const char* e = getenv("Q3TTS_TC_MIN_ROWS")) tc_min_rows_ = atoi(e);
   {
-    int min_rows = 3;
-    if (const char* e = getenv("Q3TTS_TC_MIN_ROWS")) min_rows = atoi(e);
     const char* e16 = getenv("Q3TTS_KV_F16");
-    kv_f16_ = (min_rows > 0 && B >= min_rows && !(e16 && atoi(e16) == 0)) ? 1 : 0;
+    kv_f16_ = (tc_min_rows_ > 0 && B >= tc_min_rows_ && !(e16 && atoi(e16) == 0)) ? 1 : 0;
   }
   const size_t kv_elem = kv_f16_ ? 2 : 4;
   kcache_ = arena_.alloc(kv_slot_stride_ * B * kv_elem);
@@ -84,8 +83,7 @@ TalkerEngine::TalkerEngine(const std::string& model_dir, const TalkerConfig& cfg
   d_ids_ = arena_.alloc_n<int>(max_tp_rows_);
   d_desc_ = arena_.alloc_n<int>((size_t)3 * max_rows_);
   // tensor-core copies: built when the handle can see >= tc_min_rows_ rows at once (batched decode, or any prefill)
-  if (const char* e = getenv("Q3TTS_TC_MIN_ROWS")) tc_min_rows_ = tc_min_rows_step_ = atoi(e);
-  if (tc_min_rows_step_ > 0 && B >= tc_min_rows_step_) {  // batched handle: fp16 copies for prefill, packed weights for decode steps
+  if (tc_min_rows_ > 0 && B >= tc_min_rows_) {  // batched handle: fp16 copies for prefill, packed weights for decode steps
     init_tc_gemm();
     {
       std::lock_guard<std::mutex> lk(shared_->mu);
@@ -98,20 +96,12 @@ TalkerEngine::TalkerEngine(const std::string& model_dir, const TalkerConfig& cfg
     d_tpe16_ = arena_.alloc((size_t)max_tp_rows_ * cfg_.text_hidden_size * 2);
     d_tph16_ = arena_.alloc((size_t)max_tp_rows_ * cfg_.text_hidden_size * 2);
   }
-  handle_tc_ = w_.has_tc && tc_min_rows_step_ > 0 && B >= tc_min_rows_step_;
+  handle_tc_ = w_.has_tc && tc_min_rows_ > 0 && B >= tc_min_rows_;
   {
     const char* e = getenv("Q3TTS_SKINNY_Q");
     packed_gemm_ = opt_.packed_gemm == 1 || (opt_.packed_gemm == 0 && e && atoi(e) != 0);
   }
   Q3_CHECK(!kv_f16_ || handle_tc_ || !w_.has_tc, Q3TTS_ERR_BAD_CONFIG, "internal: fp16 KV rings on a handle without the tensor-core step");
-  chain_.base = arena_.alloc_n<unsigned>(kChainCounters);
-  chain_.capacity = kChainCounters;
-  Q3_CUDA(cudaMemsetAsync(chain_.base, 0, sizeof(unsigned) * kChainCounters, stream_));
-  // Measured on B200 (0.6B 4-bit, 64 utterances): 5.44 ms per frame-step with chain signals against 5.04 ms with plain programmatic
-  // dependent launches -- the spinning consumers and the gpu-scope fences cost more than the earlier hand-over saves.  Opt-in only.
-  chain_enabled_ = false;
-  if (const char* e = getenv("Q3TTS_CHAIN")) chain_enabled_ = atoi(e) != 0;
-  if (!pdl_enabled()) chain_enabled_ = false;  // a consumer may only spin on its producer when it was launched as its programmatic dependent
   d_probe_logits_ = arena_.alloc_n<float>(4096);
   d_probe_set_ = arena_.alloc_n<unsigned>(128);
   d_probe_out_ = arena_.alloc_n<int>(1);
@@ -470,7 +460,7 @@ void TalkerEngine::forward_stack(const StackWeights& S, float* x, int m, const i
     //   prefill (any row count): the same arithmetic on the 128-row-tile kernel with precomputed factors (launch_row_scale).
     //      Every output row of either kernel depends only on its own input row and on the weight shape, so a request's
     //      result does not depend on which other requests shared its launches (tests: batched == single, bit for bit).
-    const bool fused = decode_step && m <= 128 && tc_skinny_enabled();
+    const bool fused = decode_step && m <= 128;
     // decode step with two rows per slot and no window = code-predictor pass 0: rows (2s, 2s+1) at positions (0, 1)
     const bool pass0_pairs = decode_step && !one_row_per_slot && win_start == nullptr && row_pos == d_cp_pos2_ && (m % 2) == 0;
     const float inv16 = 1.0f / kX16Div;
@@ -509,9 +499,7 @@ void TalkerEngine::forward_stack(const StackWeights& S, float* x, int m, const i
       kv.k = static_cast<char*>(kbase) + l * layer_stride * kv_elem; kv.v = static_cast<char*>(vbase) + l * layer_stride * kv_elem;
       kv.slot_stride = slot_stride; kv.capacity = capacity; kv.f16 = kv_f16;
       consumer(Tc.qkv, d_qkv_, qkv_ld, nullptr, 0, 0);
-      static const int dbg_skip = getenv("Q3TTS_DEBUG_SKIP") ? atoi(getenv("Q3TTS_DEBUG_SKIP")) : 0;  // timing attribution only
-      if (one_row_per_slot && (dbg_skip & 1)) {
-      } else if (one_row_per_slot) {
+      if (one_row_per_slot) {
         launch_rope_attention_f16(c, d_qkv_, qkv_ld, m, S.heads, S.kv_heads, L.q_norm, L.k_norm, S.eps, inv_freq, row_slot, row_pos, win_start, kv,
                                   (__half*)d_attn16_, attn_ld);
       } else if (pass0_pairs) {
@@ -521,9 +509,9 @@ void TalkerEngine::forward_stack(const StackWeights& S, float* x, int m, const i
                                    row_pos, kv);
         launch_attention_f16(c, d_qkv_, qkv_ld, m, S.heads, S.kv_heads, S.head_dim, row_slot, row_pos, win_start, kv, (__half*)d_attn16_, attn_ld);
       }
-      if (!(dbg_skip & 2)) producer(Tc.o, d_attn16_);
-      if (!(dbg_skip & 4)) consumer(Tc.gate_up_il, nullptr, 0, d_act16_, S.inter, 1);
-      if (!(dbg_skip & 8)) producer(Tc.down, d_act16_);
+      producer(Tc.o, d_attn16_);
+      consumer(Tc.gate_up_il, nullptr, 0, d_act16_, S.inter, 1);
+      producer(Tc.down, d_act16_);
     }
     return;
   }
@@ -734,18 +722,6 @@ void TalkerEngine::release(int slot) {
 // One 12.5 Hz frame for slots [0, n_slots): the loop body of Model/Qwen3Talker.swift:464-562 with every decision on device.
 void TalkerEngine::issue_frame(int n_slots) {
   step_tc_ = use_tc_step(n_slots);  // one decision per frame step (by utterances, not by the rows of each launch)
-  // chain signals between the consecutive tensor-core launches of this frame (GEMM -> attention -> GEMM ...): only inside a
-  // captured graph, where consecutive kernel nodes are programmatic dependents of each other
-  struct ChainScope {
-    bool& on;
-    explicit ChainScope(bool& f, bool v) : on(f) { on = v; }
-    ~ChainScope() { on = false; }
-  } chain_scope(chain_on_, step_tc_ && chain_enabled_ && opt_.use_cuda_graph != 0);
-  if (chain_on_) {
-    chain_.next = 0;
-    chain_.prev = nullptr;
-    Q3_CUDA(cudaMemsetAsync(chain_.base, 0, sizeof(unsigned) * kChainCounters, stream_));
-  }
   const LaunchCtx c = ctx();
   const int H = cfg_.hidden_size, Hcp = cfg_.cp.hidden_size, V = cfg_.vocab_size, Vc = cfg_.cp.vocab_size;
   const int B = opt_.max_batch, F = opt_.max_frames;
@@ -778,7 +754,7 @@ void TalkerEngine::issue_frame(int n_slots) {
     forward_stack(w_.cp, x, m, g == 0 ? d_cp_slot2_ : d_iota_, g == 0 ? d_cp_pos2_ : d_cp_pos_ + (size_t)g * B, nullptr,
                   d_cp_inv_freq_, cp_k_, cp_v_, 0, cpkv_slot_stride_, cpkv_layer_stride_, kCpCapacity, g != 0, true, x16_direct);
     // norm + lm_head[g] on the last position of each slot (Qwen3CodePredictor.swift:207-212)
-    if (step_tc_ && g != 0 && n_slots <= 128 && tc_skinny_enabled()) {
+    if (step_tc_ && g != 0 && n_slots <= 128) {
       // the last layer's down GEMM left fp16(x / 16) in d_h16_: lm_head (final norm folded in) takes it as is
       TcGemm hg;
       hg.a = (const __half*)d_h16_; hg.w = (const __half*)w_.lm_head_tc[g].w; hg.Bt = 1; hg.T = n_slots; hg.cin = Hcp; hg.N = Vc;
@@ -898,7 +874,7 @@ double TalkerEngine::profile_linears(int which, int m, int iters, int64_t& launc
   }
   launches = 0;
   bytes_per_iter = 0;
-  const bool tc = handle_tc_ && m >= tc_min_rows_step_ && !S.tc.empty();  // the launches a decode step of this handle issues at m rows
+  const bool tc = handle_tc_ && m >= tc_min_rows_ && !S.tc.empty();  // the launches a decode step of this handle issues at m rows
   auto pass = [&](bool count) {
     for (int l = 0; l < S.layers; ++l) {
       const LayerWeights& L = S.layer[l];
@@ -929,22 +905,11 @@ double TalkerEngine::profile_linears(int which, int m, int iters, int64_t& launc
     if (count) { launches += 1; bytes_per_iter += (int64_t)head.weight_bytes(); }
   };
   pass(true);  // warm-up (and the per-iteration accounting)
-  // the captured pass hands over between its GEMMs exactly like a frame step does (chain signals)
-  struct ChainScope {
-    bool& on;
-    explicit ChainScope(bool& f, bool v) : on(f) { on = v; }
-    ~ChainScope() { on = false; }
-  } chain_scope(chain_on_, tc && chain_enabled_);
   // One pass as a CUDA graph, replayed `iters` times: the same submission path as the frame step (stream launches would add a
   // host-side tensor-map encode + launch per kernel and measure the CPU instead of the kernels).
   cudaGraph_t graph = nullptr;
   cudaGraphExec_t exec = nullptr;
   Q3_CUDA(cudaStreamBeginCapture(stream_, cudaStreamCaptureModeThreadLocal));
-  if (chain_on_) {
-    chain_.next = 0;
-    chain_.prev = nullptr;
-    Q3_CUDA(cudaMemsetAsync(chain_.base, 0, sizeof(unsigned) * kChainCounters, stream_));
-  }
   pass(false);
   Q3_CUDA(cudaStreamEndCapture(stream_, &graph));
   Q3_CUDA(cudaGraphInstantiate(&exec, graph, 0));

@@ -548,17 +548,12 @@ __global__ void __launch_bounds__(128, 4) rope_attention_kernel(const float* __r
                                                              const float* __restrict__ q_norm, const float* __restrict__ k_norm, float eps,
                                                              const float* __restrict__ inv_freq, const int* __restrict__ row_slot,
                                                              const int* __restrict__ row_pos, const int* __restrict__ win_start, KVLayout kv,
-                                                             OutT* __restrict__ out, int ldo, float scale, const ChainSig sig) {
+                                                             OutT* __restrict__ out, int ldo, float scale) {
   __shared__ __align__(16) float q[G * 128];
   __shared__ __align__(16) float part_o[4][G][128];
   __shared__ float part_m[4][G], part_l[4][G];
   pdl_launch_dependents();
-  if (sig.in) {  // chain signal of the qkv GEMM (common.h) instead of its grid completion
-    if (threadIdx.x == 0) chain_wait(sig.in, sig.in_target);
-    __syncthreads();
-  } else {
-    pdl_wait();
-  }
+  pdl_wait();
   const int row = blockIdx.x, kvh = blockIdx.y, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   const int slot = row_slot[row], pos = row_pos[row];
   const int w0 = win_start ? win_start[slot] : 0;
@@ -686,10 +681,6 @@ __global__ void __launch_bounds__(128, 4) rope_attention_kernel(const float* __r
     }
     store_act(out + (size_t)row * ldo + (size_t)(kvh * G + g) * 128 + tid, num / den);
   }
-  if (sig.out) {  // K / V appended, outputs stored, every read of qkv done: hand over to the o projection
-    __syncthreads();
-    if (threadIdx.x == 0) chain_signal(sig.out);
-  }
 }
 // Code-predictor pass 0 (Qwen3CodePredictor.swift:183-212 with L = 2): rows (2s, 2s+1) of slot s sit at positions 0 and 1 of a
 // cache that is reset every frame, so norm + RoPE + append + causal attention of BOTH rows is one small CTA per (slot, kv head):
@@ -699,18 +690,13 @@ template <int G>
 __global__ void __launch_bounds__(128) cp_pass0_attention_kernel(const float* __restrict__ qkv, int ld, int heads, int kv_heads,
                                                                  const float* __restrict__ q_norm, const float* __restrict__ k_norm, float eps,
                                                                  const float* __restrict__ inv_freq, KVLayout kv, __half* __restrict__ out,
-                                                                 int ldo, float scale, const ChainSig sig) {
+                                                                 int ldo, float scale) {
   __shared__ __align__(16) float q1[G * 128];   // roped query heads of position 1
   __shared__ __align__(16) float kk[2][128];    // roped keys of positions 0 and 1
   __shared__ __align__(16) float vv[2][128];
   __shared__ float w0[G], w1[G];                // softmax weights of position 1 over keys {0, 1}
   pdl_launch_dependents();
-  if (sig.in) {
-    if (threadIdx.x == 0) chain_wait(sig.in, sig.in_target);
-    __syncthreads();
-  } else {
-    pdl_wait();
-  }
+  pdl_wait();
   const int slot = blockIdx.x, kvh = blockIdx.y, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   float* kb = static_cast<float*>(kv.k) + (size_t)slot * kv.slot_stride + (size_t)kvh * kv.capacity * 128;  // the code predictor's cache is fp32
   float* vb = static_cast<float*>(kv.v) + (size_t)slot * kv.slot_stride + (size_t)kvh * kv.capacity * 128;
@@ -765,10 +751,6 @@ __global__ void __launch_bounds__(128) cp_pass0_attention_kernel(const float* __
     out[(size_t)(2 * slot) * ldo + (size_t)(kvh * G + g) * 128 + tid] = __float2half_rn(vv[0][tid]);
     out[(size_t)(2 * slot + 1) * ldo + (size_t)(kvh * G + g) * 128 + tid] = __float2half_rn(w0[g] * vv[0][tid] + w1[g] * vv[1][tid]);
   }
-  if (sig.out) {
-    __syncthreads();
-    if (threadIdx.x == 0) chain_signal(sig.out);
-  }
 }
 void launch_cp_pass0_attention_f16(const LaunchCtx& c, const float* qkv, int ld, int n_slots, int heads, int kv_heads, const float* q_norm,
                                    const float* k_norm, float eps, const float* inv_freq, const KVLayout& kv, __half* out, int ldo) {
@@ -778,11 +760,10 @@ void launch_cp_pass0_attention_f16(const LaunchCtx& c, const float* qkv, int ld,
   dim3 grid(n_slots, kv_heads);
   const bool pdl = pdl_enabled();
   Q3_CHECK(G == 1 || G == 2 || G == 4, Q3TTS_ERR_BAD_CONFIG, "unsupported GQA group size %d", G);
-  const ChainSig sig = pdl ? c.chain_link((unsigned)(n_slots * kv_heads)) : ChainSig();
-  if (G == 1) launch_kernel_pdl(cp_pass0_attention_kernel<1>, grid, dim3(128), 0, c.stream, pdl, qkv, ld, heads, kv_heads, q_norm, k_norm, eps, inv_freq, kv, out, ldo, scale, sig);
-  else if (G == 2) launch_kernel_pdl(cp_pass0_attention_kernel<2>, grid, dim3(128), 0, c.stream, pdl, qkv, ld, heads, kv_heads, q_norm, k_norm, eps, inv_freq, kv, out, ldo, scale, sig);
-  else launch_kernel_pdl(cp_pass0_attention_kernel<4>, grid, dim3(128), 0, c.stream, pdl, qkv, ld, heads, kv_heads, q_norm, k_norm, eps, inv_freq, kv, out, ldo, scale, sig);
-  if (sig.out) c.tick_chained(); else c.tick();
+  if (G == 1) launch_kernel_pdl(cp_pass0_attention_kernel<1>, grid, dim3(128), 0, c.stream, pdl, qkv, ld, heads, kv_heads, q_norm, k_norm, eps, inv_freq, kv, out, ldo, scale);
+  else if (G == 2) launch_kernel_pdl(cp_pass0_attention_kernel<2>, grid, dim3(128), 0, c.stream, pdl, qkv, ld, heads, kv_heads, q_norm, k_norm, eps, inv_freq, kv, out, ldo, scale);
+  else launch_kernel_pdl(cp_pass0_attention_kernel<4>, grid, dim3(128), 0, c.stream, pdl, qkv, ld, heads, kv_heads, q_norm, k_norm, eps, inv_freq, kv, out, ldo, scale);
+  c.tick();
 }
 
 template <typename OutT>
@@ -796,19 +777,18 @@ static void launch_rope_attention_t(const LaunchCtx& c, const float* qkv, int ld
   dim3 grid(m, kv_heads);
   const bool pdl = pdl_enabled();
   Q3_CHECK(G == 1 || G == 2 || G == 4, Q3TTS_ERR_BAD_CONFIG, "unsupported GQA group size %d", G);
-  const ChainSig sig = pdl ? c.chain_link((unsigned)(m * kv_heads)) : ChainSig();
 #define RA_LAUNCH(GV)                                                                                                                              \
   {                                                                                                                                                \
     if (kv.f16) launch_kernel_pdl(rope_attention_kernel<GV, OutT, __half>, grid, dim3(128), smem, c.stream, pdl, qkv, ld, heads, kv_heads, q_norm, k_norm, eps, \
-                                  inv_freq, row_slot, row_pos, win_start, kv, out, ldo, scale, sig);                                               \
+                                  inv_freq, row_slot, row_pos, win_start, kv, out, ldo, scale);                                                    \
     else launch_kernel_pdl(rope_attention_kernel<GV, OutT, float>, grid, dim3(128), smem, c.stream, pdl, qkv, ld, heads, kv_heads, q_norm, k_norm, eps,         \
-                           inv_freq, row_slot, row_pos, win_start, kv, out, ldo, scale, sig);                                                      \
+                           inv_freq, row_slot, row_pos, win_start, kv, out, ldo, scale);                                                           \
   }
   if (G == 1) RA_LAUNCH(1)
   else if (G == 2) RA_LAUNCH(2)
   else RA_LAUNCH(4)
 #undef RA_LAUNCH
-  if (sig.out) c.tick_chained(); else c.tick();
+  c.tick();
 }
 void launch_rope_attention(const LaunchCtx& c, const float* qkv, int ld, int m, int heads, int kv_heads, const float* q_norm,
                            const float* k_norm, float eps, const float* inv_freq, const int* row_slot, const int* row_pos,

@@ -102,7 +102,6 @@ SYMBOLS = {
     "q3tts_rvq_embed": (i32, [C.c_void_p, p_i32, i32, i32, p_f32, p_f32, p_i32]),
     "q3tts_encode_reference_audio": (i32, [C.c_void_p, p_f32, i64, p_i32, i32, p_i32, p_i32, p_f32]),
     "q3tts_extract_speaker_embedding": (i32, [C.c_void_p, p_f32, i64, p_f32, i32, p_i32, p_f32]),
-    "q3tts_debug_trap": (i32, [C.c_void_p]),
     "q3tts_clone": (i32, [C.c_void_p, C.POINTER(C.c_void_p)]),
     "q3tts_safetensors_check": (i32, [C.c_char_p, p_i32, C.POINTER(i64)]),
 }

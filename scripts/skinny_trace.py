@@ -19,9 +19,7 @@ for name, N, K, swiglu, res in SHAPES:
     s = st[:n].astype(np.int64)
     g0 = s[:, 0].min()
     rel = lambda a: (a - s[:, 1])  # cycles since CTA entry
-    alt = int(os.environ.get("Q3TTS_SKQ_DBG", "0")) & 1  # stamps 10-13 then follow the dequantisation (gemm_skinny_q.cu)
-    names = ("w3_dq_ready", "w3_packed_in", "w3_block0", "w3_block1") if alt else ("w3_peers_in", "w3_reduced", "w3_finished_chunk0", "w3_done")
-    cyc = {k: rel(s[:, i]) for k, i in (("setup", 2), ("first_stage", 3), ("acc_done", 4), ("shipped", 5), ("peers_in", 6), ("epi_done", 7), ("exit", 8), (names[0], 10), (names[1], 11), (names[2], 12), (names[3], 13), ("w3_dequant_done", 14), ("w3_dependency_resolved", 15))}
+    cyc = {k: rel(s[:, i]) for k, i in (("setup", 2), ("first_stage", 3), ("acc_done", 4), ("shipped", 5), ("peers_in", 6), ("epi_done", 7), ("exit", 8), ("w3_peers_in", 10), ("w3_reduced", 11), ("w3_finished_chunk0", 12), ("w3_done", 13), ("w3_dequant_done", 14), ("w3_dependency_resolved", 15))}
     out = {"shape": name, "bits": BITS, "M": M, "N": N, "K": K, "grid": [tiles.value, split.value], "stages": stages.value, "avg_us_per_launch": round(us.value, 2),
            "cta_start_spread_us": round(float(s[:, 0].max() - g0) / 1e3, 2), "kernel_span_us": round(float(s[:, 9].max() - g0) / 1e3, 2)}
     for k, v in cyc.items():
