@@ -33,6 +33,7 @@ extern "C" {
 
 typedef struct q3tts_handle q3tts_handle;
 typedef struct q3tts_stream q3tts_stream;
+typedef struct q3tts_voice q3tts_voice; /* a registered voice: see q3tts_voice_create */
 
 typedef enum q3tts_status {
   Q3TTS_OK = 0,
@@ -133,7 +134,9 @@ typedef struct q3tts_request {
   float* cp_logits_out;       /* [frames][15][cp_vocab]   raw lm_head logits of every code-predictor pass */
   int32_t logits_capacity_frames;
   int32_t keep_invalid_frames; /* 1: skip the final code0 in [0,2048) filter (:571-576) */
-  int32_t reserved[6];
+  const q3tts_voice* voice;     /* a voice of q3tts_voice_create whose prefilled prompt prefix replaces the voice fields, or NULL
+                                   (every field written inline, prefilled with the request).  Rules at q3tts_voice_create */
+  int32_t reserved[4];
 } q3tts_request;
 
 /* decode scheduling of the fused text->PCM calls (Qwen3TTSPipeline.swift) */
@@ -157,7 +160,9 @@ typedef struct q3tts_timing {
   double talker_ms;               /* CUDA-event time of prompt assembly + prefill + all frame steps of the last call */
   int64_t codec_flops;            /* algorithmic flops of the codec passes of the last call (SURVEY.md §8d) */
   int64_t persistent_launches;    /* launches of the persistent frame kernel in the last call (0 = CUDA-graph / eager path) */
-  int64_t reserved[3];
+  int64_t prefill_rows;           /* talker rows the last call's prefill computed (q3tts_stream_begin included): the whole prompt of an
+                                     inline request, 1 of a request with a voice */
+  int64_t reserved[2];
 } q3tts_timing;
 
 /* ------------------------------------------------------------------------------------------------------
@@ -217,6 +222,34 @@ q3tts_status q3tts_stream_next_audio(q3tts_stream* s, float* pcm_out, int32_t ca
                                      int32_t* done_out);
 q3tts_status q3tts_stream_cancel(q3tts_stream* s);
 void q3tts_stream_free(q3tts_stream* s);
+
+/* ------------------------------------------------------------------------------------------------------
+ * registered voices (no reference counterpart: the reference prefills every prompt whole).  Every prompt row before the
+ * first text id depends only on the voice: [instruct | ICL transcript + ICL codes] + role ids + the codec rows with the speaker
+ * (Model/Qwen3Talker.swift:344-433).  q3tts_voice_create prefills those P - 1 rows once and keeps their talker K / V (every layer
+ * and kv head, in the handle's ring element type: fp16 on handles of >= 3 slots, fp32 otherwise); a request with `voice` set
+ * installs them into its slot's KV ring and prefills its one remaining row.
+ *
+ *   - Input: `voice` is read for instruct_ids, speaker_id / speaker_embedding, ref_text_ids + ref_codes / ref_frames (the same
+ *     precedence rules as a request) and text_ids[0..2] (the role ids; n_text_ids >= 3).  Sampling and diagnostic fields are ignored.
+ *     Ids and codes are validated with the same checks and errors as a request.  P - 1 prefix positions: P + 16 <= kv_capacity, or
+ *     Q3TTS_ERR_CAPACITY.  Not while a stream is open on the handle (Q3TTS_ERR_INVALID_ARG, as q3tts_generate_*).
+ *   - Output contract: a request with voice = v gives the same codes, code0_logits_out / cp_logits_out and PCM, bit for bit, as the
+ *     same request with v's fields written inline and voice = NULL -- on every decode path, greedy, sampled and teacher-forced.
+ *   - Exclusive fields: a request with a voice leaves instruct_ids, ref_text_ids, ref_codes and speaker_embedding NULL and
+ *     speaker_id at -1, and its text_ids[0..2] equal the voice's role ids; otherwise the call returns Q3TTS_ERR_INVALID_ARG before
+ *     any device work.  A request with fewer than 9 text ids still returns 0 frames with Q3TTS_OK (its text is not read).
+ *   - Handles: a voice is accepted by the handle that created it and by that handle's clones (the same weights and options, so the
+ *     same numeric path and KV element type); any other handle returns Q3TTS_ERR_INVALID_ARG.  Streams (q3tts_stream_begin), batches
+ *     and q3tts_options.lanes accept voices; requests with and without voices, and with different voices, mix in one call.
+ *   - Lifetime and threads: a voice is immutable once created and may be used from several threads at once by the handles that
+ *     accept it.  It holds a reference on the shared weights: a voice, its handle and the handle's clones may be freed in any order.
+ *     Freeing a voice while a call that uses it is running is a caller error.
+ * ---------------------------------------------------------------------------------------------------- */
+q3tts_status q3tts_voice_create(q3tts_handle* h, const q3tts_request* voice, q3tts_voice** out);
+/* prefix positions (P - 1) and the device bytes the voice holds (P - 1 positions x 2 x layers x kv_heads x 128 elements) */
+q3tts_status q3tts_voice_info(const q3tts_voice* v, int32_t* prefix_positions_out, int64_t* device_bytes_out);
+void q3tts_voice_free(q3tts_voice* v);
 
 /* ------------------------------------------------------------------------------------------------------
  * codec — replaces AudioDecoder.mlxDecode / decode / chunkedDecode (Vocoder/AudioDecoder.swift:157-182) and

@@ -94,7 +94,10 @@ struct CallTimer {
   explicit CallTimer(q3tts_handle* hh) : h(hh) {
     h->timing = q3tts_timing{};
     launches0 = h->counter.n;
-    if (h->talker) { replays0 = h->talker->graph_replays; mega0 = h->talker->mega_launches; h->talker->last_prefill_ms = 0; }
+    if (h->talker) {
+      replays0 = h->talker->graph_replays; mega0 = h->talker->mega_launches;
+      h->talker->last_prefill_ms = 0; h->talker->last_prefill_rows = 0;
+    }
     cudaEventRecord(h->ev_start, h->stream);
   }
   void finish() {
@@ -108,6 +111,7 @@ struct CallTimer {
       h->timing.graph_replays = h->talker->graph_replays - replays0;
       h->timing.persistent_launches = h->talker->mega_launches - mega0;
       h->timing.prefill_ms = h->talker->last_prefill_ms;
+      h->timing.prefill_rows = h->talker->last_prefill_rows;
       h->timing.weight_bytes_per_frame = (int64_t)h->talker->weight_bytes_per_frame();
     }
   }
@@ -116,6 +120,11 @@ struct CallTimer {
 void require_no_open_stream(q3tts_handle* h) {
   Q3_CHECK(h->open_stream == nullptr, Q3TTS_ERR_INVALID_ARG,
            "a stream is open on this handle (it owns talker slot 0): finish or free it before another talker call");
+}
+
+// the voice rules of every request of a call, before any device work (the engine checks them again at admission)
+void check_voices(q3tts_handle* h, const q3tts_request* reqs, int n) {
+  for (int i = 0; i < n; ++i) h->talker->check_voice_request(reqs[i]);
 }
 
 bool frame_valid(const int32_t* f) { return f[0] >= 0 && f[0] < 2048; }  // Model/Qwen3Talker.swift:571-576
@@ -637,6 +646,7 @@ q3tts_status q3tts_generate_codes(q3tts_handle* h, const q3tts_request* req, int
     Q3_CHECK(req && frames_out, Q3TTS_ERR_INVALID_ARG, "NULL argument");
     Q3_CHECK(h->talker != nullptr, Q3TTS_ERR_MODEL_NOT_LOADED, "Model is not loaded");
     require_no_open_stream(h);
+    check_voices(h, req, 1);
     *frames_out = 0;
     CallTimer tm(h);
     std::vector<int32_t> raw;
@@ -704,6 +714,7 @@ static q3tts_status over_lanes(q3tts_handle* h, int32_t n, F&& run) {
     a.decode_ms = std::max(a.decode_ms, t.decode_ms); a.talker_ms = std::max(a.talker_ms, t.talker_ms);
     a.kernel_launches += t.kernel_launches; a.graph_replays += t.graph_replays; a.frames += t.frames;
     a.h2d_bytes += t.h2d_bytes; a.d2h_bytes += t.d2h_bytes; a.codec_flops += t.codec_flops; a.persistent_launches += t.persistent_launches;
+    a.prefill_rows += t.prefill_rows;
     if (result == Q3TTS_OK && st[l] != Q3TTS_OK) {
       result = st[l];
       h->last_error = "lane " + std::to_string(l) + ": " + lane->last_error;
@@ -720,6 +731,7 @@ static q3tts_status generate_codes_batch_one(q3tts_handle* h, const q3tts_reques
     Q3_CHECK(reqs && frames_out && n >= 0, Q3TTS_ERR_INVALID_ARG, "NULL argument");
     Q3_CHECK(h->talker != nullptr, Q3TTS_ERR_MODEL_NOT_LOADED, "Model is not loaded");
     require_no_open_stream(h);
+    check_voices(h, reqs, n);
     CallTimer tm(h);
     std::vector<std::vector<int32_t>> raw;
     std::vector<int> n_raw;
@@ -736,6 +748,8 @@ static q3tts_status generate_codes_batch_one(q3tts_handle* h, const q3tts_reques
 q3tts_status q3tts_generate_codes_batch(q3tts_handle* h, const q3tts_request* reqs, int32_t n, int32_t* const* codes_out,
                                         int32_t capacity_frames, int32_t* frames_out) {
   if (!use_lanes(h, reqs, n) || !frames_out) return generate_codes_batch_one(h, reqs, n, codes_out, capacity_frames, frames_out);
+  const q3tts_status st = guarded(h, [&] { check_voices(h, reqs, n); });  // every lane's share, before any lane starts
+  if (st != Q3TTS_OK) return st;
   return over_lanes(h, n, [&](q3tts_handle* lane, int off, int cnt) {
     return generate_codes_batch_one(lane, reqs + off, cnt, codes_out ? codes_out + off : nullptr, capacity_frames, frames_out + off);
   });
@@ -792,13 +806,18 @@ q3tts_status q3tts_stream_begin(q3tts_handle* h, const q3tts_request* req, int32
     Q3_CHECK(req && out, Q3TTS_ERR_INVALID_ARG, "NULL argument");
     Q3_CHECK(h->talker != nullptr, Q3TTS_ERR_MODEL_NOT_LOADED, "Model is not loaded");
     require_no_open_stream(h);
+    check_voices(h, req, 1);
     h->timing = q3tts_timing{};
     std::unique_ptr<q3tts_stream> s(new q3tts_stream());
     s->h = h;
     s->chunk_size = chunk_size > 0 ? chunk_size : 12;  // defaultStreamingChunkSize (Qwen3TTSPipeline.swift:43)
     q3tts_request r = *req;
     r.stream_variant = 1;
+    h->talker->last_prefill_ms = 0;
+    h->talker->last_prefill_rows = 0;
     Admission a = h->talker->admit(0, r);
+    h->timing.prefill_ms = h->talker->last_prefill_ms;
+    h->timing.prefill_rows = h->talker->last_prefill_rows;
     s->too_short = a.too_short;
     s->limit = std::min(std::max(r.max_tokens, 0), h->talker->max_frames());
     h->open_stream = s.get();
@@ -886,6 +905,29 @@ void q3tts_stream_free(q3tts_stream* s) {
   }
   delete s;
 }
+
+// =================================================================================================== registered voices
+q3tts_status q3tts_voice_create(q3tts_handle* h, const q3tts_request* voice, q3tts_voice** out) {
+  if (out) *out = nullptr;
+  if (!h || !voice || !out) return Q3TTS_ERR_INVALID_ARG;
+  return guarded(h, [&] {
+    Q3_CHECK(h->talker != nullptr, Q3TTS_ERR_MODEL_NOT_LOADED, "Model is not loaded");
+    require_no_open_stream(h);  // the stream owns slot 0, the scratch slot of the prefix prefill
+    std::unique_ptr<q3tts_voice> v(new q3tts_voice());
+    v->device = h->opt.device;
+    h->talker->create_voice(*voice, *v);
+    *out = v.release();
+  });
+}
+
+q3tts_status q3tts_voice_info(const q3tts_voice* v, int32_t* prefix_positions_out, int64_t* device_bytes_out) {
+  if (!v) return Q3TTS_ERR_INVALID_ARG;
+  if (prefix_positions_out) *prefix_positions_out = v->prefix_len;
+  if (device_bytes_out) *device_bytes_out = (int64_t)v->bytes;
+  return Q3TTS_OK;
+}
+
+void q3tts_voice_free(q3tts_voice* v) { delete v; }
 
 // =================================================================================================== codec
 q3tts_status q3tts_decode(q3tts_handle* h, const int32_t* codes, int32_t batch, int32_t frames, float* pcm_out) {
@@ -977,6 +1019,7 @@ q3tts_status q3tts_generate_pcm(q3tts_handle* h, const q3tts_request* req, int32
     Q3_CHECK(h->talker != nullptr, Q3TTS_ERR_MODEL_NOT_LOADED, "Model is not loaded");
     require_no_open_stream(h);
     Q3_CHECK(h->codec != nullptr, Q3TTS_ERR_DECODER_LOAD_FAILED, "Failed to load MLX audio decoder");
+    check_voices(h, req, 1);
     *samples_out = 0;
     if (frames_out) *frames_out = 0;
     CallTimer tm(h);
@@ -1004,6 +1047,7 @@ static q3tts_status generate_pcm_batch_one(q3tts_handle* h, const q3tts_request*
     Q3_CHECK(h->talker != nullptr, Q3TTS_ERR_MODEL_NOT_LOADED, "Model is not loaded");
     require_no_open_stream(h);
     Q3_CHECK(h->codec != nullptr, Q3TTS_ERR_DECODER_LOAD_FAILED, "Failed to load MLX audio decoder");
+    check_voices(h, reqs, n);
     CallTimer tm(h);
     static const bool host_trace = getenv("Q3TTS_HOST_TRACE") != nullptr;  // wall-clock phases of this call on stderr
     const auto w0 = std::chrono::steady_clock::now();
@@ -1039,6 +1083,8 @@ static q3tts_status generate_pcm_batch_one(q3tts_handle* h, const q3tts_request*
 q3tts_status q3tts_generate_pcm_batch(q3tts_handle* h, const q3tts_request* reqs, int32_t n, int32_t mode, float* const* pcm_out,
                                       int64_t capacity_samples, int64_t* samples_out, int32_t* frames_out) {
   if (!use_lanes(h, reqs, n) || !pcm_out || !samples_out) return generate_pcm_batch_one(h, reqs, n, mode, pcm_out, capacity_samples, samples_out, frames_out);
+  const q3tts_status st = guarded(h, [&] { check_voices(h, reqs, n); });
+  if (st != Q3TTS_OK) return st;
   return over_lanes(h, n, [&](q3tts_handle* lane, int off, int cnt) {
     return generate_pcm_batch_one(lane, reqs + off, cnt, mode, pcm_out + off, capacity_samples, samples_out + off, frames_out ? frames_out + off : nullptr);
   });

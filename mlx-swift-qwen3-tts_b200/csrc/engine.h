@@ -32,6 +32,21 @@ struct Admission {
   int prefill_len = 0;
 };
 
+struct TalkerShared;
+
+// q3tts_voice: the talker K / V of a voice's prompt prefix (positions [0, prefix_len)), prefilled once on the handle that created it.
+// Immutable; holds a reference on the weights, so it may outlive that handle.  Accepted by every handle with the same weights and
+// options (the creator and its clones): same numeric path, same ring element type.
+struct VoicePrefix {
+  std::shared_ptr<TalkerShared> shared;
+  int device = 0, max_batch = 0, kv_capacity = 0, kv_f16 = 0, handle_tc = 0;
+  int prefix_len = 0;  // P - 1 of every request in this voice
+  int role[3] = {0, 0, 0};
+  void* kv = nullptr;  // [2 (K, V)][layers][kv_heads][prefix_len][128], fp16 when kv_f16 else fp32 (cudaMalloc: outlives arenas)
+  size_t bytes = 0;
+  ~VoicePrefix();
+};
+
 // Immutable after load: the checkpoint's tensors (packed / dense, runtime-quantised when asked) and the fp16 tensor-core copies.  Shared
 // by a handle and its clones (q3tts_clone): every handle owns its stream, KV rings, slot state and activation buffers, none owns the weights.
 struct TalkerShared {
@@ -52,6 +67,10 @@ class TalkerEngine {
   struct AdmitItem { int slot; const q3tts_request* req; };
   // Several utterances at once: one concatenated prefill pass (rows carry their own slot / position).
   void admit_batch(const std::vector<AdmitItem>& items, std::vector<Admission>& out);
+  // q3tts_voice_create: prefills the voice part of `r` (rows [0, P-1)) in a scratch slot and copies its K / V out into v.kv
+  void create_voice(const q3tts_request& r, VoicePrefix& v);
+  // the voice rules of a request (q3tts_request::voice): exclusive fields, role ids, a voice this handle accepts; host only
+  void check_voice_request(const q3tts_request& r) const;
   int max_prefill_rows() const { return max_rows_; }
   // slot count a frame step is issued for when `hi` slots are in use: the row bucket of the tensor-core GEMMs (32 / 64 / 128 ...)
   // on batched handles, `hi` itself on the <= 2-slot handles of the persistent frame kernel
@@ -86,6 +105,7 @@ class TalkerEngine {
   int64_t graph_replays = 0, graph_nodes_replayed = 0, mega_launches = 0;
   bool megakernel_enabled() const { return mega_.ok; }
   double last_prefill_ms = 0;
+  int64_t last_prefill_rows = 0;
 
   // measurement hook (q3tts_profile_linear)
   double profile_linears(int which, int m, int iters, int64_t& launches, int64_t& bytes_per_iter);
@@ -100,6 +120,21 @@ class TalkerEngine {
                      const float* inv_freq, void* kbase, void* vbase, int kv_f16, size_t slot_stride, size_t layer_stride, int capacity,
                      bool one_row_per_slot, bool decode_step, bool x16_ready);
   void issue_frame(int n_slots);
+  // Prompt assembly (Model/Qwen3Talker.swift:338-433), ONE copy for admission and voice creation.  A PromptBatch collects the rows of
+  // several prompts: text ids to project ([0, 3) = tts bos / eos / pad), one (tp, codec, speaker) descriptor per prefill row with its
+  // (slot, position), and the speaker vectors.
+  struct PromptBatch {
+    std::vector<int> ids, desc, row_slot, row_pos;
+    std::vector<float> spk;
+  };
+  PromptBatch new_prompt_batch() const;
+  // the voice rows [0, P-1) of `r` at positions 0.. of `slot` (validated as admission validates them); returns P - 1
+  int voice_rows(PromptBatch& b, int slot, const q3tts_request& r);
+  // firstText row of `r` at position `pos` (codec bos + text_ids[3]) and its trailing text ids; returns the first trailing id's index
+  int text_rows(PromptBatch& b, int slot, int pos, const q3tts_request& r);
+  // uploads a PromptBatch, runs text_projection over its ids and assembles its rows into d_x_ (d_tp_ keeps the projected ids)
+  void assemble_prompt(const PromptBatch& b);
+  KvPrefixEntry* d_voice_tab_ = nullptr;  // [max_batch] voice prefixes to install in one admission round
   void build_tc_weights();
   void build_mega_plan();
   TcLinear make_tc(const Linear& L, bool interleave_halves, const float* fold = nullptr);
@@ -217,3 +252,5 @@ struct Handle {
 };
 
 }  // namespace q3
+
+struct q3tts_voice : q3::VoicePrefix {};

@@ -85,6 +85,17 @@ void launch_gather_rows(const LaunchCtx& c, const Embedding& e, const int* ids, 
 void launch_assemble_rows(const LaunchCtx& c, const float* tp_rows, int H, const Embedding& codec, const float* spk,
                           const int* desc /*[n][3] = tp, codec, spk*/, int n, float* y);
 
+// Voice prefixes (q3tts_voice): the K / V of positions [0, n_pos) of one slot's talker rings <-> a compact buffer
+// [2 (K, V)][layers][kv_heads][n_pos][128] of the rings' element type (elem_bytes 2 = fp16, 4 = fp32).  Ring index = position
+// (a prefix is shorter than the ring).  One launch covers every entry of the device table, every layer and every kv head.
+struct KvPrefixEntry {
+  void* compact;
+  int slot;
+  int n_pos;
+};
+void launch_kv_prefix_copy(const LaunchCtx& c, const KvPrefixEntry* table, int n_entries, int max_pos, void* k, void* v, size_t slot_stride,
+                           size_t layer_stride, int layers, int kv_heads, int capacity, int elem_bytes, bool to_ring);
+
 // ---- per-slot generation state living in HBM (read / written only by kernels during graph replay) ----------
 struct SlotState {
   int active;           // slot holds a running utterance

@@ -82,6 +82,7 @@ TalkerEngine::TalkerEngine(const std::string& model_dir, const TalkerConfig& cfg
   d_spk_ = arena_.alloc_n<float>((size_t)B * H);
   d_ids_ = arena_.alloc_n<int>(max_tp_rows_);
   d_desc_ = arena_.alloc_n<int>((size_t)3 * max_rows_);
+  d_voice_tab_ = arena_.alloc_n<KvPrefixEntry>(B);
   // tensor-core copies: built when the handle can see >= tc_min_rows_ rows at once (batched decode, or any prefill)
   if (tc_min_rows_ > 0 && B >= tc_min_rows_) {  // batched handle: fp16 copies for prefill, packed weights for decode steps
     init_tc_gemm();
@@ -542,101 +543,103 @@ Admission TalkerEngine::admit(int slot, const q3tts_request& r) {
   return out[0];
 }
 
-// Prompt assembly + prefill of several utterances at once (Model/Qwen3Talker.swift:344-462 for each): their prefill rows
-// are concatenated into one [R, H] activation matrix so the 28-layer prefill is ONE pass of (tensor-core) GEMMs; rows carry
-// (slot, position) so RoPE / KV append / causal attention stay per utterance.
-void TalkerEngine::admit_batch(const std::vector<AdmitItem>& items, std::vector<Admission>& out) {
-  const int H = cfg_.hidden_size, C = opt_.kv_capacity, F = opt_.max_frames, TH = cfg_.text_hidden_size;
-  out.assign(items.size(), Admission{});
-  std::vector<int> ids{cfg_.tts_bos_token_id, cfg_.tts_eos_token_id, cfg_.tts_pad_token_id};
-  const int TP_BOS = 0, TP_EOS = 1, TP_PAD = 2;
-  std::vector<int> desc, meta_slot, meta_pos;
-  std::vector<float> spk_host;
-  struct Plan { int slot, row0, P, tp_trailing, n_trailing; const q3tts_request* r; };
-  std::vector<Plan> plans;
-  auto check_text = [&](const int32_t* p, int n, const char* what) {
-    for (int i = 0; i < n; ++i)
-      Q3_CHECK(p[i] >= 0 && p[i] < cfg_.text_vocab_size, Q3TTS_ERR_INVALID_ARG, "%s id %d outside the text vocabulary", what, p[i]);
-  };
-  for (size_t it = 0; it < items.size(); ++it) {
-    const int slot = items[it].slot;
-    const q3tts_request& r = *items[it].req;
-    Q3_CHECK(slot >= 0 && slot < opt_.max_batch, Q3TTS_ERR_INVALID_ARG, "slot %d out of range", slot);
-    Q3_CHECK(r.text_ids != nullptr || r.n_text_ids == 0, Q3TTS_ERR_INVALID_ARG, "text_ids is NULL");
-    if (r.n_text_ids < 9) {  // minTokens (Model/Qwen3Talker.swift:348-352)
-      out[it].too_short = true;
-      continue;
-    }
-    check_text(r.text_ids, r.n_text_ids, "text");
-    const bool has_instruct = r.instruct_ids != nullptr && r.n_instruct_ids > 0;
-    const bool use_icl = !has_instruct && r.ref_codes != nullptr && r.ref_text_ids != nullptr && r.n_ref_text_ids > 0;  // :338, 395
-    if (has_instruct) check_text(r.instruct_ids, r.n_instruct_ids, "instruct");
-    if (use_icl) check_text(r.ref_text_ids, r.n_ref_text_ids, "reference transcript");
-    const bool spk_by_id = r.speaker_id >= 0;
-    const bool spk_by_vec = !spk_by_id && r.speaker_embedding != nullptr;
-    if (spk_by_id) Q3_CHECK(r.speaker_id < cfg_.vocab_size, Q3TTS_ERR_INVALID_ARG, "speaker_id %d outside codec vocabulary", r.speaker_id);
-    if (spk_by_vec) Q3_CHECK(r.speaker_embedding_dim == H, Q3TTS_ERR_INVALID_ARG, "speaker embedding has %d dims, model hidden size is %d", r.speaker_embedding_dim, H);
-    const int n_front_text = has_instruct ? r.n_instruct_ids : (use_icl ? r.n_ref_text_ids : 0);
-    const int n_ref_audio = (use_icl && r.ref_frames > 0) ? r.ref_frames : 0;
-    const int trailing_len = r.n_text_ids - 4 - 5;  // :426
-    const int n_trailing = trailing_len > 0 ? trailing_len : 0;
-    Q3_CHECK(n_trailing + 1 <= opt_.max_trailing, Q3TTS_ERR_CAPACITY, "text too long: %d trailing tokens > %d", n_trailing + 1, opt_.max_trailing);
-    const int n_codec = 5 + ((spk_by_id || spk_by_vec) ? 1 : 0);
-    const int P = n_front_text + n_ref_audio + 3 + (n_codec - 1) + 1;
-    Q3_CHECK(P <= C - 16, Q3TTS_ERR_CAPACITY, "prefill of %d positions exceeds kv_capacity %d - 16; raise q3tts_options.kv_capacity", P, C);
-    Q3_CHECK((int)ids.size() + n_front_text + 4 + n_trailing <= max_tp_rows_ && (int)meta_slot.size() + P <= max_rows_, Q3TTS_ERR_CAPACITY,
-             "prompt batch too large for this handle");
-    // text rows to project: [instruct | ref-text ..., role(3), first text, trailing ...]
-    const int tp_front = (int)ids.size();
-    for (int i = 0; i < n_front_text; ++i) ids.push_back(has_instruct ? r.instruct_ids[i] : r.ref_text_ids[i]);
-    const int tp_role = (int)ids.size();
-    for (int i = 0; i < 3; ++i) ids.push_back(r.text_ids[i]);
-    const int tp_first = (int)ids.size();
-    ids.push_back(r.text_ids[3]);
-    const int tp_trailing = (int)ids.size();
-    for (int i = 0; i < n_trailing; ++i) ids.push_back(r.text_ids[4 + i]);
-    // prefill row descriptors (tp index, codec row, speaker-vector index + 1)
-    int spk_ref = 0;
-    if (spk_by_vec) {
-      spk_host.insert(spk_host.end(), r.speaker_embedding, r.speaker_embedding + H);
-      spk_ref = (int)(spk_host.size() / H);
-    }
-    const int row0 = (int)meta_slot.size();
-    auto row = [&](int tp, int codec, int spk) {
-      desc.push_back(tp); desc.push_back(codec); desc.push_back(spk);
-      meta_slot.push_back(slot); meta_pos.push_back((int)meta_slot.size() - 1 - row0);
-    };
-    for (int i = 0; i < n_front_text; ++i) row(tp_front + i, -1, 0);
-    for (int i = 0; i < n_ref_audio; ++i) {  // codec_embedding(refCodes[0]) — first codebook only (:402-403)
-      const int code = r.ref_codes[i];
-      Q3_CHECK(code >= 0 && code < cfg_.vocab_size, Q3TTS_ERR_INVALID_ARG, "reference code %d outside codec vocabulary", code);
-      row(-1, code, 0);
-    }
-    for (int i = 0; i < 3; ++i) row(tp_role + i, -1, 0);
-    // codecEmbed = [nothink, think_bos, think_eos, (speaker), pad, bos] (:360-379);
-    // combined = [tts_pad x (n-2), tts_bos] + codecEmbed[0 ..< n-1] (:383-386)
-    int codec_ids[6], codec_spk[6] = {0, 0, 0, 0, 0, 0};
-    int k = 0;
-    codec_ids[k++] = cfg_.codec_nothink_id; codec_ids[k++] = cfg_.codec_think_bos_id; codec_ids[k++] = cfg_.codec_think_eos_id;
-    if (spk_by_id) codec_ids[k++] = r.speaker_id;
-    else if (spk_by_vec) { codec_ids[k] = -1; codec_spk[k] = spk_ref; ++k; }
-    codec_ids[k++] = cfg_.codec_pad_id; codec_ids[k++] = cfg_.codec_bos_id;
-    for (int i = 0; i < n_codec - 1; ++i) row(i < n_codec - 2 ? TP_PAD : TP_BOS, codec_ids[i], codec_spk[i]);
-    row(tp_first, codec_ids[n_codec - 1], 0);  // firstTextEmbed (:423)
-    out[it].prefill_len = P;
-    plans.push_back({slot, row0, P, tp_trailing, n_trailing, &r});
-  }
-  if (plans.empty()) return;
-  const int n_tp = (int)ids.size(), R = (int)meta_slot.size();
-  Q3_CHECK((int)(spk_host.size() / H) <= opt_.max_batch, Q3TTS_ERR_CAPACITY, "too many speaker embeddings in one admission batch");
+namespace {
+constexpr int TP_BOS = 0, TP_EOS = 1, TP_PAD = 2;  // rows of PromptBatch::ids
+void check_text(const int32_t* p, int n, int vocab, const char* what) {
+  for (int i = 0; i < n; ++i)
+    Q3_CHECK(p[i] >= 0 && p[i] < vocab, Q3TTS_ERR_INVALID_ARG, "%s id %d outside the text vocabulary", what, p[i]);
+}
+}  // namespace
 
+VoicePrefix::~VoicePrefix() {
+  int prev = 0;
+  cudaGetDevice(&prev);
+  cudaSetDevice(device);
+  if (kv) cudaFree(kv);
+  shared.reset();  // may be the last reference on the weights
+  cudaSetDevice(prev);
+}
+
+TalkerEngine::PromptBatch TalkerEngine::new_prompt_batch() const {
+  PromptBatch b;
+  b.ids = {cfg_.tts_bos_token_id, cfg_.tts_eos_token_id, cfg_.tts_pad_token_id};
+  return b;
+}
+
+int TalkerEngine::voice_rows(PromptBatch& b, int slot, const q3tts_request& r) {
+  const int H = cfg_.hidden_size, C = opt_.kv_capacity;
+  const bool has_instruct = r.instruct_ids != nullptr && r.n_instruct_ids > 0;
+  const bool use_icl = !has_instruct && r.ref_codes != nullptr && r.ref_text_ids != nullptr && r.n_ref_text_ids > 0;  // :338, 395
+  if (has_instruct) check_text(r.instruct_ids, r.n_instruct_ids, cfg_.text_vocab_size, "instruct");
+  if (use_icl) check_text(r.ref_text_ids, r.n_ref_text_ids, cfg_.text_vocab_size, "reference transcript");
+  const bool spk_by_id = r.speaker_id >= 0;
+  const bool spk_by_vec = !spk_by_id && r.speaker_embedding != nullptr;
+  if (spk_by_id) Q3_CHECK(r.speaker_id < cfg_.vocab_size, Q3TTS_ERR_INVALID_ARG, "speaker_id %d outside codec vocabulary", r.speaker_id);
+  if (spk_by_vec) Q3_CHECK(r.speaker_embedding_dim == H, Q3TTS_ERR_INVALID_ARG, "speaker embedding has %d dims, model hidden size is %d", r.speaker_embedding_dim, H);
+  const int n_front_text = has_instruct ? r.n_instruct_ids : (use_icl ? r.n_ref_text_ids : 0);
+  const int n_ref_audio = (use_icl && r.ref_frames > 0) ? r.ref_frames : 0;
+  const int n_codec = 5 + ((spk_by_id || spk_by_vec) ? 1 : 0);
+  const int n = n_front_text + n_ref_audio + 3 + (n_codec - 1);  // every prompt row before firstText
+  Q3_CHECK(n + 1 <= C - 16, Q3TTS_ERR_CAPACITY, "prefill of %d positions exceeds kv_capacity %d - 16; raise q3tts_options.kv_capacity", n + 1, C);
+  Q3_CHECK((int)b.ids.size() + n_front_text + 3 <= max_tp_rows_ && (int)b.row_slot.size() + n <= max_rows_, Q3TTS_ERR_CAPACITY,
+           "prompt batch too large for this handle");
+  // text rows to project: [instruct | ref-text ..., role(3)]
+  const int tp_front = (int)b.ids.size();
+  for (int i = 0; i < n_front_text; ++i) b.ids.push_back(has_instruct ? r.instruct_ids[i] : r.ref_text_ids[i]);
+  const int tp_role = (int)b.ids.size();
+  for (int i = 0; i < 3; ++i) b.ids.push_back(r.text_ids[i]);
+  int spk_ref = 0;  // speaker-vector index + 1
+  if (spk_by_vec) {
+    b.spk.insert(b.spk.end(), r.speaker_embedding, r.speaker_embedding + H);
+    spk_ref = (int)(b.spk.size() / H);
+  }
+  int pos = 0;
+  auto row = [&](int tp, int codec, int spk) {  // prefill row descriptor (tp index, codec row, speaker-vector index + 1)
+    b.desc.push_back(tp); b.desc.push_back(codec); b.desc.push_back(spk);
+    b.row_slot.push_back(slot); b.row_pos.push_back(pos++);
+  };
+  for (int i = 0; i < n_front_text; ++i) row(tp_front + i, -1, 0);
+  for (int i = 0; i < n_ref_audio; ++i) {  // codec_embedding(refCodes[0]) — first codebook only (:402-403)
+    const int code = r.ref_codes[i];
+    Q3_CHECK(code >= 0 && code < cfg_.vocab_size, Q3TTS_ERR_INVALID_ARG, "reference code %d outside codec vocabulary", code);
+    row(-1, code, 0);
+  }
+  for (int i = 0; i < 3; ++i) row(tp_role + i, -1, 0);
+  // codecEmbed = [nothink, think_bos, think_eos, (speaker), pad, bos] (:360-379);
+  // combined = [tts_pad x (n-2), tts_bos] + codecEmbed[0 ..< n-1] (:383-386); its last row, bos, goes with firstText (text_rows)
+  int codec_ids[5], codec_spk[5] = {0, 0, 0, 0, 0};
+  int k = 0;
+  codec_ids[k++] = cfg_.codec_nothink_id; codec_ids[k++] = cfg_.codec_think_bos_id; codec_ids[k++] = cfg_.codec_think_eos_id;
+  if (spk_by_id) codec_ids[k++] = r.speaker_id;
+  else if (spk_by_vec) { codec_ids[k] = -1; codec_spk[k] = spk_ref; ++k; }
+  codec_ids[k++] = cfg_.codec_pad_id;
+  for (int i = 0; i < n_codec - 1; ++i) row(i < n_codec - 2 ? TP_PAD : TP_BOS, codec_ids[i], codec_spk[i]);
+  return n;
+}
+
+int TalkerEngine::text_rows(PromptBatch& b, int slot, int pos, const q3tts_request& r) {
+  const int n_trailing = std::max(r.n_text_ids - 4 - 5, 0);  // :426
+  Q3_CHECK((int)b.ids.size() + 1 + n_trailing <= max_tp_rows_ && (int)b.row_slot.size() + 1 <= max_rows_, Q3TTS_ERR_CAPACITY,
+           "prompt batch too large for this handle");
+  const int tp_first = (int)b.ids.size();
+  b.ids.push_back(r.text_ids[3]);
+  const int tp_trailing = (int)b.ids.size();
+  for (int i = 0; i < n_trailing; ++i) b.ids.push_back(r.text_ids[4 + i]);
+  b.desc.push_back(tp_first); b.desc.push_back(cfg_.codec_bos_id); b.desc.push_back(0);  // firstTextEmbed (:423)
+  b.row_slot.push_back(slot); b.row_pos.push_back(pos);
+  return tp_trailing;
+}
+
+void TalkerEngine::assemble_prompt(const PromptBatch& b) {
+  const int H = cfg_.hidden_size, TH = cfg_.text_hidden_size;
+  const int n_tp = (int)b.ids.size(), R = (int)b.row_slot.size();
+  Q3_CHECK((int)(b.spk.size() / H) <= opt_.max_batch, Q3TTS_ERR_CAPACITY, "too many speaker embeddings in one admission batch");
   const LaunchCtx c = ctx();
-  Q3_CUDA(cudaEventRecord(ev_a_, stream_));
-  Q3_CUDA(cudaMemcpyAsync(d_ids_, ids.data(), sizeof(int) * n_tp, cudaMemcpyHostToDevice, stream_));
-  Q3_CUDA(cudaMemcpyAsync(d_desc_, desc.data(), sizeof(int) * 3 * R, cudaMemcpyHostToDevice, stream_));
-  Q3_CUDA(cudaMemcpyAsync(d_pf_slot_, meta_slot.data(), sizeof(int) * R, cudaMemcpyHostToDevice, stream_));
-  Q3_CUDA(cudaMemcpyAsync(d_pf_pos_, meta_pos.data(), sizeof(int) * R, cudaMemcpyHostToDevice, stream_));
-  if (!spk_host.empty()) Q3_CUDA(cudaMemcpyAsync(d_spk_, spk_host.data(), sizeof(float) * spk_host.size(), cudaMemcpyHostToDevice, stream_));
+  Q3_CUDA(cudaMemcpyAsync(d_ids_, b.ids.data(), sizeof(int) * n_tp, cudaMemcpyHostToDevice, stream_));
+  Q3_CUDA(cudaMemcpyAsync(d_desc_, b.desc.data(), sizeof(int) * 3 * R, cudaMemcpyHostToDevice, stream_));
+  Q3_CUDA(cudaMemcpyAsync(d_pf_slot_, b.row_slot.data(), sizeof(int) * R, cudaMemcpyHostToDevice, stream_));
+  Q3_CUDA(cudaMemcpyAsync(d_pf_pos_, b.row_pos.data(), sizeof(int) * R, cudaMemcpyHostToDevice, stream_));
+  if (!b.spk.empty()) Q3_CUDA(cudaMemcpyAsync(d_spk_, b.spk.data(), sizeof(float) * b.spk.size(), cudaMemcpyHostToDevice, stream_));
   // text_projection(text_embedding(ids)) (Model/Qwen3Talker.swift:103-106; Qwen3Layers.swift:276-279)
   if (use_tc(n_tp)) {
     launch_gather_rows_f16(c, w_.text_embedding, d_ids_, n_tp, (__half*)d_tpe16_, TH);
@@ -648,6 +651,99 @@ void TalkerEngine::admit_batch(const std::vector<AdmitItem>& items, std::vector<
     launch_linear(c, w_.fc2, d_tph_, TH, n_tp, d_tp_, H, nullptr, 0.f, EPI_STORE);
   }
   launch_assemble_rows(c, d_tp_, H, w_.codec_embedding, d_spk_, d_desc_, R, d_x_);
+}
+
+void TalkerEngine::check_voice_request(const q3tts_request& r) const {
+  const VoicePrefix* v = r.voice;
+  if (!v) return;
+  Q3_CHECK(v->shared == shared_ && v->max_batch == opt_.max_batch && v->kv_capacity == opt_.kv_capacity && v->kv_f16 == kv_f16_ &&
+               v->handle_tc == (handle_tc_ ? 1 : 0),
+           Q3TTS_ERR_INVALID_ARG,
+           "the request's voice was created on a handle with other weights or options: a voice is accepted only by the handle that created "
+           "it and that handle's clones");
+  Q3_CHECK(r.instruct_ids == nullptr && r.ref_text_ids == nullptr && r.ref_codes == nullptr && r.speaker_embedding == nullptr && r.speaker_id == -1,
+           Q3TTS_ERR_INVALID_ARG, "a request with a voice leaves instruct_ids, ref_text_ids, ref_codes and speaker_embedding NULL and speaker_id at -1");
+  if (r.n_text_ids < 9) return;  // too short: 0 frames, the text is never read (Model/Qwen3Talker.swift:348-352)
+  Q3_CHECK(r.text_ids != nullptr, Q3TTS_ERR_INVALID_ARG, "text_ids is NULL");
+  Q3_CHECK(r.text_ids[0] == v->role[0] && r.text_ids[1] == v->role[1] && r.text_ids[2] == v->role[2], Q3TTS_ERR_INVALID_ARG,
+           "text_ids[0..2] = (%d, %d, %d) differ from the voice's role ids (%d, %d, %d)", r.text_ids[0], r.text_ids[1], r.text_ids[2], v->role[0],
+           v->role[1], v->role[2]);
+}
+
+// The voice part of a prompt, prefilled alone: with causal attention, row i's K / V depend on rows <= i only, and every prefill GEMM
+// gives a row the same bits whatever the row count (forward_stack), so positions [0, P-1) hold what a whole-prompt prefill leaves there.
+void TalkerEngine::create_voice(const q3tts_request& r, VoicePrefix& v) {
+  Q3_CHECK(r.voice == nullptr, Q3TTS_ERR_INVALID_ARG, "a voice is created from inline voice fields, not from another voice");
+  Q3_CHECK(r.text_ids != nullptr && r.n_text_ids >= 3, Q3TTS_ERR_INVALID_ARG, "a voice needs its role ids: text_ids[0..2] (n_text_ids >= 3)");
+  check_text(r.text_ids, 3, cfg_.text_vocab_size, "role");
+  const int slot = 0;  // scratch: between calls no slot holds an utterance (an open stream, which owns slot 0, refuses the call)
+  PromptBatch b = new_prompt_batch();
+  const int n = voice_rows(b, slot, r);
+  const StackWeights& T = w_.talker;
+  v.shared = shared_;
+  v.max_batch = opt_.max_batch; v.kv_capacity = opt_.kv_capacity; v.kv_f16 = kv_f16_; v.handle_tc = handle_tc_ ? 1 : 0;
+  v.prefix_len = n;
+  for (int i = 0; i < 3; ++i) v.role[i] = r.text_ids[i];
+  v.bytes = (size_t)2 * T.layers * T.kv_heads * n * 128 * (kv_f16_ ? 2 : 4);
+  Q3_CUDA(cudaMalloc(&v.kv, v.bytes));
+  assemble_prompt(b);
+  forward_stack(T, d_x_, n, d_pf_slot_, d_pf_pos_, d_pf_win_, d_inv_freq_, kcache_, vcache_, kv_f16_, kv_slot_stride_, kv_layer_stride_,
+                opt_.kv_capacity, false, false, false);
+  const KvPrefixEntry e{v.kv, slot, n};
+  Q3_CUDA(cudaMemcpyAsync(d_voice_tab_, &e, sizeof e, cudaMemcpyHostToDevice, stream_));
+  launch_kv_prefix_copy(ctx(), d_voice_tab_, 1, n, kcache_, vcache_, kv_slot_stride_, kv_layer_stride_, T.layers, T.kv_heads, opt_.kv_capacity,
+                        kv_f16_ ? 2 : 4, false);
+  Q3_CUDA(cudaStreamSynchronize(stream_));
+}
+
+// Prompt assembly + prefill of several utterances at once (Model/Qwen3Talker.swift:344-462 for each): their prefill rows
+// are concatenated into one [R, H] activation matrix so the 28-layer prefill is ONE pass of (tensor-core) GEMMs; rows carry
+// (slot, position) so RoPE / KV append / causal attention stay per utterance.  An item with a voice contributes its firstText row
+// only: one launch first installs every such item's prefix K / V into its slot's rings.
+void TalkerEngine::admit_batch(const std::vector<AdmitItem>& items, std::vector<Admission>& out) {
+  const int H = cfg_.hidden_size, C = opt_.kv_capacity, F = opt_.max_frames;
+  out.assign(items.size(), Admission{});
+  PromptBatch b = new_prompt_batch();
+  struct Plan { int slot, last_row, P, tp_trailing, n_trailing; const q3tts_request* r; };
+  std::vector<Plan> plans;
+  std::vector<KvPrefixEntry> installs;
+  int max_install = 0;
+  for (size_t it = 0; it < items.size(); ++it) {
+    const int slot = items[it].slot;
+    const q3tts_request& r = *items[it].req;
+    Q3_CHECK(slot >= 0 && slot < opt_.max_batch, Q3TTS_ERR_INVALID_ARG, "slot %d out of range", slot);
+    Q3_CHECK(r.text_ids != nullptr || r.n_text_ids == 0, Q3TTS_ERR_INVALID_ARG, "text_ids is NULL");
+    check_voice_request(r);
+    if (r.n_text_ids < 9) {  // minTokens (Model/Qwen3Talker.swift:348-352)
+      out[it].too_short = true;
+      continue;
+    }
+    check_text(r.text_ids, r.n_text_ids, cfg_.text_vocab_size, "text");
+    const int n_trailing = std::max(r.n_text_ids - 4 - 5, 0);  // :426
+    Q3_CHECK(n_trailing + 1 <= opt_.max_trailing, Q3TTS_ERR_CAPACITY, "text too long: %d trailing tokens > %d", n_trailing + 1, opt_.max_trailing);
+    int n_prefix = 0;
+    if (r.voice) {
+      n_prefix = r.voice->prefix_len;
+      installs.push_back({r.voice->kv, slot, n_prefix});
+      max_install = std::max(max_install, n_prefix);
+    } else {
+      n_prefix = voice_rows(b, slot, r);
+    }
+    const int tp_trailing = text_rows(b, slot, n_prefix, r);
+    out[it].prefill_len = n_prefix + 1;
+    plans.push_back({slot, (int)b.row_slot.size() - 1, n_prefix + 1, tp_trailing, n_trailing, &r});
+  }
+  if (plans.empty()) return;
+  const int R = (int)b.row_slot.size();
+
+  const LaunchCtx c = ctx();
+  Q3_CUDA(cudaEventRecord(ev_a_, stream_));
+  if (!installs.empty()) {  // ring index = position: a prefix is shorter than kv_capacity - 16
+    Q3_CUDA(cudaMemcpyAsync(d_voice_tab_, installs.data(), sizeof(KvPrefixEntry) * installs.size(), cudaMemcpyHostToDevice, stream_));
+    launch_kv_prefix_copy(c, d_voice_tab_, (int)installs.size(), max_install, kcache_, vcache_, kv_slot_stride_, kv_layer_stride_, w_.talker.layers,
+                          w_.talker.kv_heads, C, kv_f16_ ? 2 : 4, true);
+  }
+  assemble_prompt(b);
   for (const Plan& p : plans) {  // trailingTextHidden = textproj(ids[4 ..< len-5]) ++ tts_eos (:426-433)
     float* tr = d_trailing_ + (size_t)p.slot * opt_.max_trailing * H;
     if (p.n_trailing > 0)
@@ -656,9 +752,10 @@ void TalkerEngine::admit_batch(const std::vector<AdmitItem>& items, std::vector<
   }
   // prefill: every row at its own (slot, position) (Model/Qwen3Talker.swift:437)
   forward_stack(w_.talker, d_x_, R, d_pf_slot_, d_pf_pos_, d_pf_win_, d_inv_freq_, kcache_, vcache_, kv_f16_, kv_slot_stride_, kv_layer_stride_, C, false, false, false);
+  last_prefill_rows += R;
   // final norm + codec_head on the last position only (the reference computes all, :449, and samples the last, :284-286)
   for (const Plan& p : plans) {
-    launch_rmsnorm(c, d_x_ + (size_t)(p.row0 + p.P - 1) * H, H, 1, H, w_.talker.final_norm, w_.talker.eps, d_hlast_ + (size_t)p.slot * H, H);
+    launch_rmsnorm(c, d_x_ + (size_t)p.last_row * H, H, 1, H, w_.talker.final_norm, w_.talker.eps, d_hlast_ + (size_t)p.slot * H, H);
     launch_linear(c, w_.codec_head, d_hlast_ + (size_t)p.slot * H, H, 1, d_logits0_ + (size_t)p.slot * cfg_.vocab_size, cfg_.vocab_size, nullptr, 0.f, EPI_STORE);
   }
   for (const Plan& p : plans) {

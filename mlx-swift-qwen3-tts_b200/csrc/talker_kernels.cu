@@ -898,6 +898,38 @@ void launch_assemble_rows(const LaunchCtx& c, const float* tp_rows, int H, const
   c.tick();
 }
 
+// ------------------------------------------------------------------------------------------------ voice prefix <-> KV rings
+// grid (x: 16-byte vectors of one run, y: run = (K|V, layer, kv head), z: table entry).  A run is n_pos consecutive ring rows of one
+// (layer, kv head) and the matching contiguous block of the compact buffer; the copy is a bit copy whatever the element type.
+__global__ void __launch_bounds__(256) kv_prefix_copy_kernel(const KvPrefixEntry* __restrict__ table, char* k, char* v, size_t slot_bytes,
+                                                             size_t layer_bytes, size_t head_bytes, int layers, int kv_heads, int row_bytes,
+                                                             int to_ring) {
+  const KvPrefixEntry e = table[blockIdx.z];
+  const int run = blockIdx.y, per_kind = layers * kv_heads;
+  const int kind = run / per_kind, layer = (run - kind * per_kind) / kv_heads, head = run - kind * per_kind - layer * kv_heads;
+  uint4* ring = reinterpret_cast<uint4*>((kind ? v : k) + (size_t)e.slot * slot_bytes + (size_t)layer * layer_bytes + (size_t)head * head_bytes);
+  uint4* comp = reinterpret_cast<uint4*>(static_cast<char*>(e.compact) + (size_t)run * e.n_pos * row_bytes);
+  const int n_vec = e.n_pos * (row_bytes / 16);
+  for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n_vec; i += gridDim.x * blockDim.x) {
+    if (to_ring) ring[i] = comp[i];
+    else comp[i] = ring[i];
+  }
+}
+
+void launch_kv_prefix_copy(const LaunchCtx& c, const KvPrefixEntry* table, int n_entries, int max_pos, void* k, void* v, size_t slot_stride,
+                           size_t layer_stride, int layers, int kv_heads, int capacity, int elem_bytes, bool to_ring) {
+  if (n_entries <= 0 || max_pos <= 0) return;
+  Q3_CHECK(elem_bytes == 2 || elem_bytes == 4, Q3TTS_ERR_INVALID_ARG, "kv prefix copy: element size %d", elem_bytes);
+  Q3_CHECK(max_pos <= capacity && n_entries <= 65535 && 2 * layers * kv_heads <= 65535, Q3TTS_ERR_INVALID_ARG, "kv prefix copy: bad shape");
+  const int row_bytes = 128 * elem_bytes;
+  const int n_vec = max_pos * (row_bytes / 16);
+  dim3 grid((n_vec + 255) / 256, 2 * layers * kv_heads, n_entries);
+  kv_prefix_copy_kernel<<<grid, 256, 0, c.stream>>>(table, static_cast<char*>(k), static_cast<char*>(v), slot_stride * elem_bytes,
+                                                    layer_stride * elem_bytes, (size_t)capacity * row_bytes, layers, kv_heads, row_bytes,
+                                                    to_ring ? 1 : 0);
+  c.tick();
+}
+
 // ------------------------------------------------------------------------------------------------ sampler
 // (device code in sampler.cuh, shared with the frame megakernel)
 // After the group's token is known the same CTA writes the code predictor's NEXT input rows (Qwen3Talker.swift:501-523:

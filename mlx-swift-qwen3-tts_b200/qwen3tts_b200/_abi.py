@@ -45,13 +45,13 @@ class Request(C.Structure):
                 ("n_ref_text_ids", i32), ("ref_codes", p_i32), ("ref_frames", i32), ("temperature", f32), ("top_k", i32),
                 ("top_p", f32), ("repetition_penalty", f32), ("max_tokens", i32), ("seed", u64), ("stream_variant", i32),
                 ("forced_codes", p_i32), ("n_forced_frames", i32), ("code0_logits_out", p_f32), ("cp_logits_out", p_f32),
-                ("logits_capacity_frames", i32), ("keep_invalid_frames", i32), ("reserved", i32 * 6)]
+                ("logits_capacity_frames", i32), ("keep_invalid_frames", i32), ("voice", C.c_void_p), ("reserved", i32 * 4)]
 
 
 class Timing(C.Structure):
     _fields_ = [("device_ms", C.c_double), ("prefill_ms", C.c_double), ("decode_ms", C.c_double), ("kernel_launches", i64),
                 ("graph_replays", i64), ("frames", i64), ("h2d_bytes", i64), ("d2h_bytes", i64), ("weight_bytes_per_frame", i64),
-                ("talker_ms", C.c_double), ("codec_flops", i64), ("persistent_launches", i64), ("reserved", i64 * 3)]
+                ("talker_ms", C.c_double), ("codec_flops", i64), ("persistent_launches", i64), ("prefill_rows", i64), ("reserved", i64 * 2)]
 
 
 # every symbol include/qwen3tts_b200.h declares: name -> (restype, argtypes)
@@ -104,6 +104,9 @@ SYMBOLS = {
     "q3tts_extract_speaker_embedding": (i32, [C.c_void_p, p_f32, i64, p_f32, i32, p_i32, p_f32]),
     "q3tts_clone": (i32, [C.c_void_p, C.POINTER(C.c_void_p)]),
     "q3tts_safetensors_check": (i32, [C.c_char_p, p_i32, C.POINTER(i64)]),
+    "q3tts_voice_create": (i32, [C.c_void_p, C.POINTER(Request), C.POINTER(C.c_void_p)]),
+    "q3tts_voice_info": (i32, [C.c_void_p, p_i32, C.POINTER(i64)]),
+    "q3tts_voice_free": (None, [C.c_void_p]),
 }
 
 _lib = None

@@ -33,6 +33,7 @@ class GenRequest:
     forced_codes: np.ndarray | None = None  # [F][16]
     keep_invalid_frames: bool = False
     want_logits: int = 0  # frames of logits to capture (one request per call)
+    voice: "Voice | None" = None  # a registered voice (Engine.create_voice): leave the voice fields above at their defaults
 
     def to_c(self) -> A.Request:
         """-> q3tts_request whose pointers reference numpy buffers kept alive by the returned struct itself (`r._keep`): the
@@ -77,6 +78,9 @@ class GenRequest:
             r.forced_codes = fc.ctypes.data_as(A.p_i32)
             r.n_forced_frames = int(fc.shape[0])
         r.keep_invalid_frames = 1 if self.keep_invalid_frames else 0
+        if self.voice is not None:
+            r.voice = self.voice.ptr
+            keep.append(self.voice)  # a voice is not freed while a struct that names it lives
         return r
 
 
@@ -88,6 +92,40 @@ def _attach_logits(r: "A.Request", frames: int, info) -> dict:
     r.logits_capacity_frames = frames
     r._keep.extend([l0, lc])
     return {"code0_logits": l0, "cp_logits": lc}
+
+
+class Voice:
+    """`q3tts_voice`: the prefilled prompt prefix of one voice (Engine.create_voice).  Requests that set `voice=` give the bits of the
+    same requests with the voice fields written inline; the handle that made it and its clones accept it."""
+
+    def __init__(self, ptr):
+        self._p = ptr
+        n, b = A.i32(0), A.i64(0)
+        A.check(A.lib().q3tts_voice_info(self._p, C.byref(n), C.byref(b)), None)
+        self.prefix_positions, self.device_bytes = n.value, b.value
+
+    @property
+    def ptr(self):
+        if not self._p:
+            raise ValueError("the voice is closed")
+        return self._p
+
+    def close(self):
+        if getattr(self, "_p", None):
+            A.lib().q3tts_voice_free(self._p)
+            self._p = None
+
+    def __enter__(self):
+        return self
+
+    def __exit__(self, *exc):
+        self.close()
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
 
 
 class CodeStream:
@@ -194,6 +232,15 @@ class Engine:
         A.check(A.lib().q3tts_clear_cache(self._h), self._h)
 
     # ---- talker
+    def create_voice(self, req: GenRequest) -> Voice:
+        """q3tts_voice_create: prefill the voice part of `req` (instruct / speaker / ICL fields and the role ids text_ids[:3]) once."""
+        r = req.to_c()
+        p = C.c_void_p()
+        A.check(A.lib().q3tts_voice_create(self._h, C.byref(r), C.byref(p)), self._h)
+        v = Voice(p)
+        v.role_ids = [int(i) for i in req.text_ids[:3]]
+        return v
+
     def generate_codes(self, req: GenRequest, capacity: int | None = None):
         """-> frames int32 [F,16]  (+ dict of logits when req.want_logits)."""
         cap = capacity or max(req.max_tokens, 0 if req.forced_codes is None else len(req.forced_codes), 1)

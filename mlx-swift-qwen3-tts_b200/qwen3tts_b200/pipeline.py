@@ -10,6 +10,7 @@ Mapping (reference file:line -> here)
     generateVoiceDesign / generateCustomVoice (+Stream)        :355-480
     generateToFile(...) async throws -> Int                    :644  -> generate_to_file(...)
     generateBatch(...) async -> [Float]                        :774  -> generate_batch(...)
+    (no counterpart: a registered voice, q3tts_voice)                -> prepare_voice(...) -> Voice; voice= on every generate*
     clearCache()                                               :951
     availableSpeakers / supports* / modelType / sampleRate     :65-104
     AudioChunk :6-19, Qwen3TTSPipelineConfiguration :22-54, Qwen3TTSError :985-1000
@@ -25,7 +26,7 @@ from dataclasses import dataclass
 import numpy as np
 
 from . import _abi as A
-from .engine import Engine, GenRequest
+from .engine import Engine, GenRequest, Voice
 
 
 @dataclass
@@ -249,9 +250,16 @@ class Qwen3TTSPipeline:
 
     # ---- request assembly (host string side of Model/Qwen3Talker.swift:338-414)
     def _request(self, text, speaker="", instruct=None, speaker_embedding=None, reference_transcript=None, reference_audio_codes=None,
-                 temperature=None, max_tokens=None, stream_variant=False) -> GenRequest:
+                 temperature=None, max_tokens=None, stream_variant=False, voice=None) -> GenRequest:
         enc = self.tokenizer.encode
         chat = f"<|im_start|>assistant\n{text}<|im_end|>\n<|im_start|>assistant\n"  # :344
+        if voice is not None:  # the voice's prefilled prefix stands for every voice field
+            if speaker or instruct or speaker_embedding is not None or reference_transcript or reference_audio_codes is not None:
+                raise ValueError("voice= replaces speaker, instruct, speaker_embedding and the reference fields: pass one or the other")
+            return GenRequest(text_ids=enc(chat), voice=voice,
+                              temperature=self.config.default_temperature if temperature is None else temperature,
+                              max_tokens=self.config.default_max_tokens if max_tokens is None else max_tokens,
+                              seed=self.config.seed, stream_variant=stream_variant)
         spk_id = self._speakers.get(speaker.lower(), -1) if speaker else -1  # :339-340
         instruct_ids = None
         ref_ids = None
@@ -271,23 +279,48 @@ class Qwen3TTSPipeline:
             max_tokens=self.config.default_max_tokens if max_tokens is None else max_tokens,
             seed=self.config.seed, stream_variant=stream_variant)
 
+    # ---- registered voices (no reference counterpart)
+    def prepare_voice(self, speaker="", instruct=None, speaker_embedding=None, reference_transcript=None, reference_audio_codes=None) -> Voice:
+        """Prefill the voice part of the prompt once (q3tts_voice_create), from the same fields and rules as a request.  Pass the result
+        as `voice=` to any generate* call of this pipeline: the output is bit for bit what the fields written inline give, without
+        prefilling them again.  Free it with close() (or a `with` block); it may outlive the pipeline."""
+        return self.engine.create_voice(self._request("", speaker=speaker, instruct=instruct, speaker_embedding=speaker_embedding,
+                                                      reference_transcript=reference_transcript, reference_audio_codes=reference_audio_codes))
+
+    def _call_voice(self, n_chunks, voice, **fields):
+        """(voice to use, voice to free at the end) of a call that runs n_chunks generations with the same voice fields."""
+        if voice is not None or n_chunks <= 1:
+            return voice, None
+        own = self.prepare_voice(**fields)
+        return own, own
+
+    def _chunk_request(self, text, voice, own, fields, **kw) -> GenRequest:
+        """The request of one chunk: with the call's voice, unless the chunk's role ids differ from a voice the call made itself
+        (a tokenizer may merge the role's last id into the text), which then runs with its fields inline."""
+        if voice is not None:
+            req = self._request(text, voice=voice, **kw)
+            if voice is not own or list(req.text_ids[:3]) == voice.role_ids:
+                return req
+        return self._request(text, **fields, **kw)
+
     # ---- simple generation (:244-306, 355-381, 424-451)
-    def generate(self, text, speaker="", speaker_embedding=None, temperature=None, max_tokens=None, instruct=None):
+    def generate(self, text, speaker="", speaker_embedding=None, temperature=None, max_tokens=None, instruct=None, voice=None):
         req = self._request(text, speaker=speaker, instruct=instruct, speaker_embedding=speaker_embedding, temperature=temperature,
-                            max_tokens=max_tokens)
+                            max_tokens=max_tokens, voice=voice)
         pcm, _ = self.engine.generate_pcm(req, A.DECODE_WHOLE)
         return pcm
 
-    def generate_voice_design(self, text, voice_description, temperature=None, max_tokens=None):
-        return self.generate(text, speaker="", instruct=voice_description, temperature=temperature, max_tokens=max_tokens)
+    def generate_voice_design(self, text, voice_description=None, temperature=None, max_tokens=None, voice=None):
+        return self.generate(text, speaker="", instruct=voice_description, temperature=temperature, max_tokens=max_tokens, voice=voice)
 
-    def generate_custom_voice(self, text, speaker, instruct, temperature=None, max_tokens=None):
-        return self.generate(text, speaker=speaker, instruct=instruct, temperature=temperature, max_tokens=max_tokens)
+    def generate_custom_voice(self, text, speaker="", instruct=None, temperature=None, max_tokens=None, voice=None):
+        return self.generate(text, speaker=speaker, instruct=instruct, temperature=temperature, max_tokens=max_tokens, voice=voice)
 
     # ---- streaming (:323-340, 392-408, 463-480, 484-624)
-    def generate_stream(self, text, speaker="", speaker_embedding=None, temperature=None, max_tokens=None, chunk_size=None, instruct=None):
+    def generate_stream(self, text, speaker="", speaker_embedding=None, temperature=None, max_tokens=None, chunk_size=None, instruct=None,
+                        voice=None):
         req = self._request(text, speaker=speaker, instruct=instruct, speaker_embedding=speaker_embedding, temperature=temperature,
-                            max_tokens=max_tokens, stream_variant=True)
+                            max_tokens=max_tokens, stream_variant=True, voice=voice)
         st = self.engine.stream(req, chunk_size or self.config.default_streaming_chunk_size)
         try:
             while True:
@@ -298,18 +331,29 @@ class Qwen3TTSPipeline:
         finally:
             st.close()
 
-    def generate_stream_voice_design(self, text, voice_description, **kw):
+    def generate_stream_voice_design(self, text, voice_description=None, **kw):
         return self.generate_stream(text, speaker="", instruct=voice_description, **kw)
 
-    def generate_stream_custom_voice(self, text, speaker, instruct, **kw):
+    def generate_stream_custom_voice(self, text, speaker="", instruct=None, **kw):
         return self.generate_stream(text, speaker=speaker, instruct=instruct, **kw)
 
     # ---- file output (:644-757)
     def generate_to_file(self, text, output_url, speaker="", instruct=None, speaker_embedding=None, reference_transcript=None,
-                         reference_audio_codes=None, temperature=None, on_progress=None) -> int:
+                         reference_audio_codes=None, temperature=None, on_progress=None, voice=None) -> int:
         chunks = TextChunker.chunk(text, TextChunker.default_max_words)
         if not chunks:
             return 0
+        fields = dict(speaker=speaker, instruct=instruct, speaker_embedding=speaker_embedding, reference_transcript=reference_transcript,
+                      reference_audio_codes=reference_audio_codes)
+        # every chunk repeats the same voice: a call of several chunks prefills it once (a voice of its own, freed before returning)
+        voice, own = self._call_voice(len(chunks), voice, **fields)
+        try:
+            return self._generate_to_file(chunks, output_url, voice, own, fields, temperature, on_progress)
+        finally:
+            if own is not None:
+                own.close()
+
+    def _generate_to_file(self, chunks, output_url, voice, own, fields, temperature, on_progress) -> int:
         writer = StreamingWAVWriter(output_url)
         # Every text chunk is an independent generation with a fresh KV cache (Qwen3TTSPipeline.swift:668-691), so a handle with
         # several slots runs `max_batch` chunks at a time through the batched path; a handle's numeric path is fixed at creation,
@@ -319,9 +363,7 @@ class Qwen3TTSPipeline:
             part = chunks[g0: g0 + group]
             if on_progress:
                 on_progress(g0 / len(chunks))
-            reqs = [self._request(tc, speaker=speaker, instruct=instruct, speaker_embedding=speaker_embedding,
-                                  reference_transcript=reference_transcript, reference_audio_codes=reference_audio_codes,
-                                  temperature=temperature, max_tokens=600) for tc in part]  # :690
+            reqs = [self._chunk_request(tc, voice, own, fields, temperature=temperature, max_tokens=600) for tc in part]  # :690
             if len(reqs) == 1:
                 outs = [self.engine.generate_pcm(reqs[0], A.DECODE_FILE)]
             else:
@@ -337,17 +379,27 @@ class Qwen3TTSPipeline:
 
     # ---- batch (:774-898)
     def generate_batch(self, text, speaker="", instruct=None, speaker_embedding=None, reference_transcript=None, temperature=None,
-                       on_progress=None):
+                       on_progress=None, voice=None):
         chunks = TextChunker.chunk(text, TextChunker.default_max_words)
         if not chunks:
             return np.zeros(0, np.float32)
         if len(chunks) == 1:  # single-chunk shortcut drops speakerEmbedding / instruct, as the reference does (:791-796)
             if on_progress:
                 on_progress(0.0)
-            out = self.generate(chunks[0], speaker=speaker, temperature=temperature)
+            out = self.generate(chunks[0], speaker=speaker if voice is None else "", temperature=temperature, voice=voice)
             if on_progress:
                 on_progress(1.0)
             return out
+        # generateBatch forwards the transcript but not the codes, so ICL stays off (:813-822)
+        fields = dict(speaker=speaker, instruct=instruct, speaker_embedding=speaker_embedding)
+        voice, own = self._call_voice(len(chunks), voice, **fields)
+        try:
+            return self._generate_batch(chunks, voice, own, fields, temperature, on_progress)
+        finally:
+            if own is not None:
+                own.close()
+
+    def _generate_batch(self, chunks, voice, own, fields, temperature, on_progress):
         cf = self.config.crossfade_samples
         all_s, tail = [], np.zeros(0, np.float32)
         # chunks are independent generations (:813-864): a handle with several slots runs `max_batch` of them per batched call, the
@@ -358,9 +410,7 @@ class Qwen3TTSPipeline:
             if on_progress:
                 on_progress(i / len(chunks))
             if i not in done:
-                # generateBatch forwards the transcript but not the codes, so ICL stays off (:813-822)
-                reqs = [self._request(c, speaker=speaker, instruct=instruct, speaker_embedding=speaker_embedding, temperature=temperature, max_tokens=600)
-                        for c in chunks[i: i + group]]
+                reqs = [self._chunk_request(c, voice, own, fields, temperature=temperature, max_tokens=600) for c in chunks[i: i + group]]
                 if len(reqs) == 1:
                     done[i] = self.engine.generate_pcm(reqs[0], A.DECODE_BATCHAPI)
                 else:

@@ -52,6 +52,26 @@ public enum Qwen3TTSError: LocalizedError {
     }
 }
 
+/// A registered voice (q3tts_voice): the prompt prefix of one speaker / instruct / ICL reference, prefilled once by
+/// `Qwen3TTSPipeline.prepareVoice`.  Requests made with it give the bits of the same requests with the fields written inline.
+/// Immutable; usable from several threads; may outlive the pipeline.  Freed when the last reference goes.
+public final class Qwen3TTSVoice: @unchecked Sendable {
+    let pointer: OpaquePointer
+    let roleIds: [Int32]
+    public let prefixPositions: Int
+    public let deviceBytes: Int64
+    init(pointer: OpaquePointer, roleIds: [Int32]) {
+        self.pointer = pointer
+        self.roleIds = roleIds
+        var n: Int32 = 0
+        var b: Int64 = 0
+        _ = q3tts_voice_info(pointer, &n, &b)
+        prefixPositions = Int(n)
+        deviceBytes = b
+    }
+    deinit { q3tts_voice_free(pointer) }
+}
+
 public final class Qwen3TTSPipeline: @unchecked Sendable {
     public static let sampleRate: Int = 24000
 
@@ -103,6 +123,14 @@ public final class Qwen3TTSPipeline: @unchecked Sendable {
     private struct Ids {
         var text: [Int32]; var instruct: [Int32] = []; var refText: [Int32] = []; var refCodes: [Int32] = []; var refFrames: Int32 = 0
         var speakerId: Int32 = -1; var embedding: [Float] = []
+        var voice: Qwen3TTSVoice? = nil   // replaces every voice field above
+    }
+    /// the ids of `text` in a voice; nil when a voice made by the call itself does not match the chunk's role ids
+    private func voiceIds(text: String, voice: Qwen3TTSVoice, strict: Bool) -> Ids? {
+        var ids = Ids(text: tokenizer.encode(text: "<|im_start|>assistant\n\(text)<|im_end|>\n<|im_start|>assistant\n"))
+        if !strict && Array(ids.text.prefix(3)) != voice.roleIds { return nil }
+        ids.voice = voice
+        return ids
     }
     private func makeIds(text: String, speaker: String, instruct: String?, speakerEmbedding: [Float]?, referenceTranscript: String?,
                          referenceAudioCodes: [[Int32]]?) -> Ids {
@@ -139,6 +167,7 @@ public final class Qwen3TTSPipeline: @unchecked Sendable {
                             req.max_tokens = Int32(maxTokens)
                             req.seed = pipelineConfig.seed
                             req.stream_variant = streamVariant ? 1 : 0
+                            req.voice = ids.voice?.pointer
                             return body(&req)
                         }
                     }
@@ -159,7 +188,32 @@ public final class Qwen3TTSPipeline: @unchecked Sendable {
         return Array(out.prefix(Int(n)))
     }
 
+    // MARK: registered voices (no reference counterpart)
+    /// Prefill the voice part of the prompt once (q3tts_voice_create), from the same fields and rules as a request.
+    public func prepareVoice(speaker: String = "", instruct: String? = nil, speakerEmbedding: [Float]? = nil, referenceTranscript: String? = nil,
+                             referenceAudioCodes: [[Int32]]? = nil) throws -> Qwen3TTSVoice {
+        guard let h = handle else { throw Qwen3TTSError.modelNotLoaded }
+        let ids = makeIds(text: "", speaker: speaker, instruct: instruct, speakerEmbedding: speakerEmbedding, referenceTranscript: referenceTranscript,
+                          referenceAudioCodes: referenceAudioCodes)
+        var v: OpaquePointer?
+        let st = withRequest(ids, temperature: 0, maxTokens: 0, streamVariant: false) { req in q3tts_voice_create(h, &req, &v) }
+        guard st == Q3TTS_OK, let vv = v else { throw Qwen3TTSError.engine(st.rawValue, String(cString: q3tts_last_error(h))) }
+        return Qwen3TTSVoice(pointer: vv, roleIds: Array(ids.text.prefix(3)))
+    }
+    /// a voice for a call of several chunks that repeat the same fields (nil: run them inline)
+    private func callVoice(chunks: Int, voice: Qwen3TTSVoice?, speaker: String, instruct: String?, speakerEmbedding: [Float]?,
+                           referenceTranscript: String?, referenceAudioCodes: [[Int32]]?) -> (Qwen3TTSVoice?, Bool) {
+        if let v = voice { return (v, true) }
+        guard chunks > 1 else { return (nil, false) }
+        return ((try? prepareVoice(speaker: speaker, instruct: instruct, speakerEmbedding: speakerEmbedding, referenceTranscript: referenceTranscript,
+                                   referenceAudioCodes: referenceAudioCodes)), false)
+    }
+
     // MARK: simple generation (:244-306)
+    public func generate(text: String, voice: Qwen3TTSVoice, temperature: Float? = nil, maxTokens: Int? = nil) -> [Float] {
+        guard let ids = voiceIds(text: text, voice: voice, strict: true) else { return [] }
+        return pcm(ids, mode: Q3TTS_DECODE_WHOLE, temperature: temperature ?? pipelineConfig.defaultTemperature, maxTokens: maxTokens ?? pipelineConfig.defaultMaxTokens)
+    }
     public func generate(text: String, speaker: String, temperature: Float? = nil, maxTokens: Int? = nil) -> [Float] {
         pcm(makeIds(text: text, speaker: speaker, instruct: nil, speakerEmbedding: nil, referenceTranscript: nil, referenceAudioCodes: nil),
             mode: Q3TTS_DECODE_WHOLE, temperature: temperature ?? pipelineConfig.defaultTemperature, maxTokens: maxTokens ?? pipelineConfig.defaultMaxTokens)
@@ -190,9 +244,15 @@ public final class Qwen3TTSPipeline: @unchecked Sendable {
                                           chunkSize: Int? = nil) -> AsyncThrowingStream<AudioChunk, Error> {
         streamImpl(text: text, speaker: speaker, instruct: instruct, speakerEmbedding: nil, temperature: temperature, maxTokens: maxTokens, chunkSize: chunkSize)
     }
+    public func generateStream(text: String, voice: Qwen3TTSVoice, temperature: Float? = nil, maxTokens: Int? = nil,
+                               chunkSize: Int? = nil) -> AsyncThrowingStream<AudioChunk, Error> {
+        streamImpl(text: text, speaker: "", instruct: nil, speakerEmbedding: nil, temperature: temperature, maxTokens: maxTokens, chunkSize: chunkSize,
+                   voice: voice)
+    }
     private func streamImpl(text: String, speaker: String, instruct: String?, speakerEmbedding: [Float]?, temperature: Float?, maxTokens: Int?,
-                            chunkSize: Int?) -> AsyncThrowingStream<AudioChunk, Error> {
-        let ids = makeIds(text: text, speaker: speaker, instruct: instruct, speakerEmbedding: speakerEmbedding, referenceTranscript: nil, referenceAudioCodes: nil)
+                            chunkSize: Int?, voice: Qwen3TTSVoice? = nil) -> AsyncThrowingStream<AudioChunk, Error> {
+        let ids = voice.flatMap { voiceIds(text: text, voice: $0, strict: true) }
+            ?? makeIds(text: text, speaker: speaker, instruct: instruct, speakerEmbedding: speakerEmbedding, referenceTranscript: nil, referenceAudioCodes: nil)
         let temp = temperature ?? pipelineConfig.defaultTemperature
         let tokens = maxTokens ?? pipelineConfig.defaultMaxTokens
         let chunk = Int32(chunkSize ?? pipelineConfig.defaultStreamingChunkSize)
@@ -223,16 +283,20 @@ public final class Qwen3TTSPipeline: @unchecked Sendable {
     // MARK: file output (:644-757): TextChunker + StreamingWAVWriter are the reference's own Swift sources
     public func generateToFile(text: String, speaker: String = "", instruct: String? = nil, speakerEmbedding: [Float]? = nil,
                                referenceTranscript: String? = nil, referenceAudioCodes: [[Int32]]? = nil, outputURL: URL,
-                               temperature: Float? = nil, onProgress: ((Float) -> Void)? = nil) async throws -> Int {
+                               temperature: Float? = nil, onProgress: ((Float) -> Void)? = nil, voice: Qwen3TTSVoice? = nil) async throws -> Int {
         let temp = temperature ?? pipelineConfig.defaultTemperature
         let chunks = TextChunker.chunk(text, maxWords: TextChunker.defaultMaxWords)
         guard !chunks.isEmpty else { return 0 }
+        // every chunk repeats the same voice: several chunks prefill it once (a voice of the call's own, freed when the call returns)
+        let (v, strict) = callVoice(chunks: chunks.count, voice: voice, speaker: speaker, instruct: instruct, speakerEmbedding: speakerEmbedding,
+                                    referenceTranscript: referenceTranscript, referenceAudioCodes: referenceAudioCodes)
         let writer = try StreamingWAVWriter(to: outputURL)
         for (i, c) in chunks.enumerated() {
             if Task.isCancelled { break }
             onProgress?(Float(i) / Float(chunks.count))
-            let ids = makeIds(text: c, speaker: speaker, instruct: instruct, speakerEmbedding: speakerEmbedding,
-                              referenceTranscript: referenceTranscript, referenceAudioCodes: referenceAudioCodes)
+            let ids = v.flatMap { voiceIds(text: c, voice: $0, strict: strict) }
+                ?? makeIds(text: c, speaker: speaker, instruct: instruct, speakerEmbedding: speakerEmbedding,
+                           referenceTranscript: referenceTranscript, referenceAudioCodes: referenceAudioCodes)
             let samples = pcm(ids, mode: Q3TTS_DECODE_FILE, temperature: temp, maxTokens: 600)
             if !samples.isEmpty { try writer.write(samples: samples) }
         }
@@ -242,17 +306,26 @@ public final class Qwen3TTSPipeline: @unchecked Sendable {
 
     // MARK: batch (:774-898)
     public func generateBatch(text: String, speaker: String = "", instruct: String? = nil, speakerEmbedding: [Float]? = nil,
-                              referenceTranscript: String? = nil, temperature: Float? = nil, onProgress: ((Float) -> Void)? = nil) async -> [Float] {
+                              referenceTranscript: String? = nil, temperature: Float? = nil, onProgress: ((Float) -> Void)? = nil,
+                              voice: Qwen3TTSVoice? = nil) async -> [Float] {
         let temp = temperature ?? pipelineConfig.defaultTemperature
         let crossfade = pipelineConfig.crossfadeSamples
         let chunks = TextChunker.chunk(text, maxWords: TextChunker.defaultMaxWords)
         guard !chunks.isEmpty else { return [] }
-        if chunks.count == 1 { onProgress?(0); let s = generate(text: chunks[0], speaker: speaker, temperature: temp); onProgress?(1); return s }
+        if chunks.count == 1 {
+            onProgress?(0)
+            let s = voice.map { generate(text: chunks[0], voice: $0, temperature: temp) } ?? generate(text: chunks[0], speaker: speaker, temperature: temp)
+            onProgress?(1)
+            return s
+        }
+        let (v, strict) = callVoice(chunks: chunks.count, voice: voice, speaker: speaker, instruct: instruct, speakerEmbedding: speakerEmbedding,
+                                    referenceTranscript: nil, referenceAudioCodes: nil)
         var all: [Float] = [], tail: [Float] = []
         for (i, c) in chunks.enumerated() {
             if Task.isCancelled { return all }
             onProgress?(Float(i) / Float(chunks.count))
-            let ids = makeIds(text: c, speaker: speaker, instruct: instruct, speakerEmbedding: speakerEmbedding, referenceTranscript: nil, referenceAudioCodes: nil)
+            let ids = v.flatMap { voiceIds(text: c, voice: $0, strict: strict) }
+                ?? makeIds(text: c, speaker: speaker, instruct: instruct, speakerEmbedding: speakerEmbedding, referenceTranscript: nil, referenceAudioCodes: nil)
             var s = pcm(ids, mode: Q3TTS_DECODE_BATCHAPI, temperature: temp, maxTokens: 600)
             if s.isEmpty { continue }
             if !tail.isEmpty && crossfade > 0 {
