@@ -75,7 +75,8 @@ typedef struct q3tts_options {
                                without a `quantization` block is MLX-quantised at load, group 64, 6 bits for embeddings / q,k,v projections /
                                heads, 4 bits for the rest (codes held in an 8-bit container).  0 = run the checkpoint as stored.
                                Checkpoints with a `quantization` block are never re-quantised; MLX affine checkpoints of 2, 3, 4, 5, 6
-                               and 8 bits with group_size 32, 64 or 128 load as stored (q3tts_info.checkpoint_quant_bits) */
+                               and 8 bits with group_size 32, 64 or 128 load as stored (q3tts_info.checkpoint_quant_bits), and MLX mxfp4
+                               checkpoints (mode "mxfp4", bits 4, group_size 32) load as exact 8-bit affine groups of 32 */
   int32_t lanes;            /* > 1: q3tts_generate_pcm_batch / q3tts_generate_codes_batch calls with more than max_batch requests are split over
                                `lanes` handles (this one + lazily created q3tts_clone()s sharing its weights), each served by a worker thread
                                of the call: several latency-bound launch chains overlap on the device (see q3tts_clone).  The threads live
@@ -102,7 +103,10 @@ typedef struct q3tts_info {
   int32_t checkpoint_quant_bits; /* width of the MLX-packed leaves on disk (2, 3, 4, 5, 6 or 8); 0 = dense checkpoint, runtime-quantised
                                     or not.  quant_bits is the width the kernels stream: 2 / 3-bit codes are held in 4-bit words and 5 / 6-bit
                                     codes in 8-bit words, unchanged (DESIGN.md §1) */
-  int32_t reserved[3];
+  int32_t checkpoint_quant_mode; /* 0 = MLX affine leaves or a dense checkpoint, 1 = MLX mxfp4 leaves (E2M1 codes, one E8M0 scale byte per
+                                    32): held as exact 8-bit affine groups of 32 with bf16 scales and biases, so checkpoint_quant_bits is 4,
+                                    quant_bits 8 and quant_group_size 32 (DESIGN.md §1; q3tts_mxfp4_to_affine) */
+  int32_t reserved[2];
 } q3tts_info;
 
 /* ---- one utterance; replaces the argument list of Qwen3Talker.generateCodes / generateStream
@@ -311,6 +315,16 @@ q3tts_status q3tts_mlx_quantize(int32_t device, const void* w, int32_t w_dtype, 
 q3tts_status q3tts_dequantize(int32_t device, const uint32_t* packed, const void* scales, const void* biases,
                               int32_t scale_dtype, int32_t out_features, int32_t in_features, int32_t group_size,
                               int32_t bits, int32_t out_dtype, void* out);
+/* The load-time conversion of an MLX mxfp4 leaf (config `mode` "mxfp4") on host buffers.  packed [out][in/8] uint32, E2M1 code j of a
+ * word at bits 4j (LSB first); scales [out][in/32] E8M0 bytes, element = lut[code] * 2^(byte - 127) with
+ * lut = {0, .5, 1, 1.5, 2, 3, 4, 6, -0, -.5, -1, -1.5, -2, -3, -4, -6}.  Output: the same values as an 8-bit affine group of 32:
+ * codes8_out [out][in/4] uint32 (q = 2 * lut[code] + 12, the 8-bit word layout of q3tts_dequantize), scales_out / biases_out
+ * [out][in/32] bf16 (2^(byte - 128) and -12 * 2^(byte - 128)).  q3tts_dequantize, q3tts_quantized_matmul and
+ * q3tts_quantized_matmul_tc take them with bits 8, group_size 32 and Q3TTS_BF16 scales and give the E2M1 values exactly (-0 as +0).
+ * NULL pointers, in % 32 != 0 and scale bytes >= 252 (values the container cannot hold; 255 is E8M0's NaN) are refused with
+ * Q3TTS_ERR_INVALID_ARG before any device is touched. */
+q3tts_status q3tts_mxfp4_to_affine(int32_t device, const uint32_t* packed, const uint8_t* scales, int32_t out_features, int32_t in_features,
+                                   uint32_t* codes8_out, void* scales_out, void* biases_out);
 /* MLXNN.QuantizedLinear / quantized_matmul (Model/QuantizedLayerFactory.swift:56): y[m][out] = x[m][in] . W^T,
  * fp32 activations, the same kernels the talker uses for m rows. */
 q3tts_status q3tts_quantized_matmul(int32_t device, const float* x, int32_t m, const uint32_t* packed,

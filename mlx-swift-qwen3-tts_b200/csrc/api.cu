@@ -577,6 +577,7 @@ q3tts_status q3tts_get_info(const q3tts_handle* hc, q3tts_info* out) {
     out->num_code_groups = c.cp.num_code_groups;
     out->quant_bits = hc->talker->quant_bits(); out->quant_group_size = hc->talker->quant_group();
     out->checkpoint_quant_bits = hc->talker->checkpoint_quant_bits();
+    out->checkpoint_quant_mode = hc->talker->checkpoint_quant_mode();
     out->weight_dtype = hc->talker->weight_dtype();
     out->num_speakers = (int32_t)c.spk_id.size();
     out->model_type = c.tts_model_type == "voice_design" ? 1 : (c.tts_model_type == "custom_voice" ? 2 : 0);
@@ -1175,6 +1176,45 @@ q3tts_status q3tts_mlx_quantize(int32_t device, const void* w, int32_t w_dtype, 
     cudaFree(dw); cudaFree(ds); cudaFree(db); cudaFree(dc);
     return Q3TTS_OK;
   } catch (const Error& e) {
+    g_create_error = e.what();
+    cudaGetLastError();
+    return e.status;
+  }
+}
+
+q3tts_status q3tts_mxfp4_to_affine(int32_t device, const uint32_t* packed, const uint8_t* scales, int32_t out_f, int32_t in_f, uint32_t* codes8_out,
+                                   void* scales_out, void* biases_out) {
+  std::vector<void*> allocs;
+  try {
+    Q3_CHECK(packed && scales && codes8_out && scales_out && biases_out, Q3TTS_ERR_INVALID_ARG, "NULL argument");
+    Q3_CHECK(out_f > 0 && in_f > 0 && in_f % 32 == 0, Q3TTS_ERR_INVALID_ARG, "unsupported shape %d x %d (in_features a multiple of 32)", out_f, in_f);
+    const size_t wbytes = (size_t)out_f * in_f / 2, groups = (size_t)out_f * (in_f / 32), cbytes = (size_t)out_f * in_f;
+    for (size_t k = 0; k < groups; ++k)
+      Q3_CHECK(scales[k] <= kMxfp4MaxScaleByte, Q3TTS_ERR_INVALID_ARG, "scale byte %d at index %zu: bytes 0..%d fit the container", (int)scales[k], k,
+               kMxfp4MaxScaleByte);
+    require_device(device);
+    auto dev = [&](const void* src, size_t bytes) -> void* {
+      void* d = nullptr;
+      Q3_CUDA(cudaMalloc(&d, bytes));
+      allocs.push_back(d);
+      if (src) Q3_CUDA(cudaMemcpy(d, src, bytes, cudaMemcpyHostToDevice));
+      return d;
+    };
+    const uint32_t* dw = (const uint32_t*)dev(packed, wbytes);
+    const uint8_t* ds = (const uint8_t*)dev(scales, groups);
+    uint32_t* dc = (uint32_t*)dev(nullptr, cbytes);
+    uint16_t* dsc = (uint16_t*)dev(nullptr, groups * 2);
+    uint16_t* dbi = (uint16_t*)dev(nullptr, groups * 2);
+    LaunchCtx c{nullptr, nullptr};
+    launch_mxfp4_to_affine(c, dw, ds, out_f, in_f, dc, dsc, dbi);
+    Q3_CUDA(cudaDeviceSynchronize());
+    Q3_CUDA(cudaMemcpy(codes8_out, dc, cbytes, cudaMemcpyDeviceToHost));
+    Q3_CUDA(cudaMemcpy(scales_out, dsc, groups * 2, cudaMemcpyDeviceToHost));
+    Q3_CUDA(cudaMemcpy(biases_out, dbi, groups * 2, cudaMemcpyDeviceToHost));
+    for (void* d : allocs) cudaFree(d);
+    return Q3TTS_OK;
+  } catch (const Error& e) {
+    for (void* d : allocs) cudaFree(d);
     g_create_error = e.what();
     cudaGetLastError();
     return e.status;

@@ -98,6 +98,7 @@ class TalkerEngine {
   int weight_dtype() const { return shared_->weight_dtype; }
   int quant_bits() const { return shared_->eff_bits; }
   int checkpoint_quant_bits() const { return w_.checkpoint_bits; }
+  int checkpoint_quant_mode() const { return w_.checkpoint_mode; }
   int quant_group() const { return shared_->eff_group; }
   size_t device_bytes() const { return arena_.total() + (owns_weights_ ? shared_->arena.total() : 0); }  // a clone reports its own state only
   const std::shared_ptr<TalkerShared>& shared() const { return shared_; }

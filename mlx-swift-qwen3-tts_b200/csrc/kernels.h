@@ -30,6 +30,15 @@ inline int container_bits(int bits) {
 // container_bits(bits) = cb word layout of launch_dequantize / launch_linear.  Scales and biases are untouched.
 void launch_widen_bits(const LaunchCtx& c, const uint32_t* src, int rows, int in, int bits, uint32_t* dst);
 
+// MLX mxfp4 leaves -> the exact 8-bit affine container of group 32 with bf16 scales / biases that launch_dequantize / launch_linear
+// read.  packed: [rows][in / 8] uint32, E2M1 code j of a word at bits 4j; scale_bytes: [rows][in / 32] E8M0 bytes, each < 252 (the
+// caller checks: larger exponents do not fit the container).  Element (c, e) = lut[c] * 2^(e - 127) becomes q = 2 lut[c] + 12 with
+// scale 2^(e - 128) and bias -12 * 2^(e - 128): both are powers of two times small integers, so scale * q + bias is exact in fp32 and
+// equals the E2M1 value (-0 becomes +0).  codes8_out: [rows][in / 4] uint32; scales_out / biases_out: [rows][in / 32] bf16.
+constexpr int kMxfp4MaxScaleByte = 251;
+void launch_mxfp4_to_affine(const LaunchCtx& c, const uint32_t* packed, const uint8_t* scale_bytes, int rows, int in, uint32_t* codes8_out,
+                            uint16_t* scales_out, uint16_t* biases_out);
+
 // y[m][*] (op)= epilogue( rmsnorm?(x[m][:]) . W^T + bias ).   x, y fp32 with row strides ldx / ldy.
 // norm_w != null fuses Qwen3RMSNorm (Model/Qwen3Layers.swift:18-25) into the prologue.
 // EPI_SWIGLU: W rows are [gate ; up]; y[m][r] = silu(gate_r) * up_r, r < out/2 (Model/Qwen3Layers.swift:236).

@@ -17,6 +17,9 @@ struct CPConfig {  // Model/Qwen3Config.swift:21-33
   float rms_norm_eps = 1e-6f, rope_theta = 1000000.0f;
 };
 
+// `mode` of an MLX quantisation block; the values are those of q3tts_info.checkpoint_quant_mode
+enum QuantMode { QMODE_AFFINE = 0, QMODE_MXFP4 = 1 };
+
 struct TalkerConfig {  // Model/Qwen3Config.swift:65-128
   int hidden_size = 0, num_hidden_layers = 0, vocab_size = 0, text_vocab_size = 0, text_hidden_size = 2048;
   int num_attention_heads = 0, num_key_value_heads = 8, head_dim = 128, intermediate_size = 0;
@@ -32,6 +35,7 @@ struct TalkerConfig {  // Model/Qwen3Config.swift:65-128
   bool has_quantization = false, has_quantization_config = false;
   int q_bits = 0, q_group = 64;      // from `quantization`
   int qc_bits = 0, qc_group = 64;    // from `quantization_config`
+  int q_mode = QMODE_AFFINE, qc_mode = QMODE_AFFINE;  // `mode` of each block (absent = affine)
 };
 
 TalkerConfig parse_talker_config(const Json& root);
@@ -105,6 +109,7 @@ struct TalkerWeights {
   bool has_tc = false;
   size_t talker_step_bytes = 0, cp_pass_bytes = 0;  // algorithmic weight bytes per invocation
   int checkpoint_bits = 0;  // width of the packed leaves on disk (2..8), 0 = dense; the kernels read 4 / 8-bit words (Linear::bits)
+  int checkpoint_mode = QMODE_AFFINE;  // QMODE_MXFP4: E2M1 leaves held as exact 8-bit affine groups of 32 (launch_mxfp4_to_affine)
 };
 
 // Loads `model.safetensors` with the key remap of Qwen3Talker.load (Model/Qwen3Talker.swift:117-137).

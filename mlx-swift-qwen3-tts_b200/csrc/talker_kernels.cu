@@ -83,6 +83,42 @@ void launch_widen_bits(const LaunchCtx& c, const uint32_t* src, int rows, int in
   c.tick();
 }
 
+// ------------------------------------------------------------------------------------------------ mxfp4 -> exact 8-bit affine container
+// One thread builds one 8-bit container word: 4 E2M1 codes, the low or high half of one source word.  Rows are whole groups of 32
+// (in % 32 == 0), so the flat indices line up across rows: container word wi takes source word wi / 2 and lies in group wi / 8, and the
+// first thread of each group writes its scale and bias.  The loop never indexes past rows * in / 4 words.  Scale and bias are built
+// from bit patterns: 2^(e - 128) is a bf16 subnormal for e < 2 (0x20 << e) and normal otherwise (exponent field e - 1);
+// -12 * 2^(e - 128) = -1.5 * 2^(e - 125) has exponent field e + 2 and mantissa 0x40.
+__global__ void mxfp4_to_affine_kernel(const uint32_t* __restrict__ packed, const uint8_t* __restrict__ scale_bytes, size_t words,
+                                       uint32_t* __restrict__ codes8, uint16_t* __restrict__ scales, uint16_t* __restrict__ biases) {
+  // q = 2 * lut[c] + 12 by code c, one byte each: codes 0..7 {12,13,14,15,16,18,20,24}, codes 8..15 {12,11,10,9,8,6,4,0}
+  constexpr uint64_t kLo = 0x181412100F0E0D0Cull, kHi = 0x00040608090A0B0Cull;
+  for (size_t wi = (size_t)blockIdx.x * blockDim.x + threadIdx.x; wi < words; wi += (size_t)gridDim.x * blockDim.x) {
+    const uint32_t src = packed[wi >> 1] >> ((wi & 1) * 16);
+    uint32_t out = 0;
+#pragma unroll
+    for (int j = 0; j < 4; ++j) {
+      const uint32_t code = (src >> (4 * j)) & 0xFu;
+      out |= (uint32_t)(((code < 8 ? kLo : kHi) >> (8 * (code & 7))) & 0xFFu) << (8 * j);
+    }
+    codes8[wi] = out;
+    if ((wi & 7) == 0) {
+      const uint32_t e = scale_bytes[wi >> 3];
+      scales[wi >> 3] = (uint16_t)(e < 2 ? 0x20u << e : (e - 1) << 7);
+      biases[wi >> 3] = (uint16_t)(0x8000u | ((e + 2) << 7) | 0x40u);
+    }
+  }
+}
+
+void launch_mxfp4_to_affine(const LaunchCtx& c, const uint32_t* packed, const uint8_t* scale_bytes, int rows, int in, uint32_t* codes8_out,
+                            uint16_t* scales_out, uint16_t* biases_out) {
+  Q3_CHECK(rows > 0 && in > 0 && in % 32 == 0, Q3TTS_ERR_INVALID_ARG, "mxfp4_to_affine: %d x %d unsupported (in a multiple of 32)", rows, in);
+  const size_t words = (size_t)rows * in / 4;
+  const int blocks = (int)std::max<size_t>(1, std::min<size_t>((words + 255) / 256, 148 * 16));
+  mxfp4_to_affine_kernel<<<blocks, 256, 0, c.stream>>>(packed, scale_bytes, words, codes8_out, scales_out, biases_out);
+  c.tick();
+}
+
 // ------------------------------------------------------------------------------------------------ runtime quantisation
 // MLX `quantize(w, group_size: 64, bits)` (affine), one thread per group of 64 weights, restated operation for operation from
 // oracle/mlx_quant.py:quantize (every fp32 step rounded on its own: no FMA contraction, IEEE division, round-half-even):

@@ -95,19 +95,27 @@ TalkerConfig parse_talker_config(const Json& root) {
   if (const Json* rs = src.find("rope_scaling"))
     c.has_mrope = rs->type == Json::Obj && rs->has("mrope_section") && rs->at("mrope_section").type == Json::Arr;
   c.tts_model_type = root.string_or("tts_model_type", "");
+  // MLX's `mode` of a quantisation block: "affine" (the default) or "mxfp4", whose bits and group_size default to 4 and 32 and must be
+  // those.  nvfp4, mxfp8 and every other mode are refused here, before any weight is read (DESIGN.md §8).
+  auto quant_block = [](const Json& q, const char* key, int& bits, int& group, int& mode) {
+    const std::string m = q.string_or("mode", "affine");
+    Q3_CHECK(m == "affine" || m == "mxfp4", Q3TTS_ERR_BAD_CONFIG, "%s.mode \"%s\" is not supported (affine or mxfp4)", key, m.c_str());
+    mode = m == "mxfp4" ? QMODE_MXFP4 : QMODE_AFFINE;
+    bits = q.integer_or("bits", mode == QMODE_MXFP4 ? 4 : 0);
+    group = q.integer_or("group_size", mode == QMODE_MXFP4 ? 32 : 64);
+    if (mode == QMODE_MXFP4)
+      Q3_CHECK(bits == 4 && group == 32, Q3TTS_ERR_BAD_CONFIG, "%s: mode mxfp4 needs bits 4 and group_size 32 (got %d / %d)", key, bits, group);
+  };
   if (const Json* q = root.find("quantization")) {
     if (q->type == Json::Obj) {
       c.has_quantization = true;
-      c.q_bits = q->integer_or("bits", 0);
-      c.q_group = q->integer_or("group_size", 64);
+      quant_block(*q, "quantization", c.q_bits, c.q_group, c.q_mode);
     }
   }
   if (const Json* q = root.find("quantization_config")) {
     if (q->type == Json::Obj) {
       c.has_quantization_config = true;
-      c.qc_bits = q->integer_or("bits", 0);
-      c.qc_group = q->integer_or("group_size", 64);
-      Q3_CHECK(q->string_or("mode", "affine") != "mxfp4", Q3TTS_ERR_BAD_CONFIG, "quantization_config.mode mxfp4 is out of scope (affine only)");
+      quant_block(*q, "quantization_config", c.qc_bits, c.qc_group, c.qc_mode);
     }
   }
   Q3_CHECK(c.hidden_size > 0 && c.num_hidden_layers > 0 && c.num_attention_heads > 0 && c.intermediate_size > 0,
@@ -128,6 +136,7 @@ struct Loader {
   bool packed;          // use uint32 leaves as they are
   bool offline_dequant; // uint32 leaves -> fp16 dense at load (Qwen3Talker.swift:139-175)
   int bits, group;
+  bool mxfp4;           // packed leaves are MLX mxfp4 (E2M1 codes + E8M0 scale bytes), converted to 8-bit affine groups of 32 at load
   // Qwen3TTSPipeline.applyMixedQuantization (:961-980): every dense Linear / Embedding is MLX-quantised at load, group 64, 6 bits for
   // embeddings, q/k/v projections and the heads, 4 bits for the rest; the codes live in an 8-bit container (launch_mlx_quantize)
   bool runtime_quant = false;
@@ -185,6 +194,23 @@ struct Loader {
     return e;
   }
 
+  // The packed words (cbits-bit container), scales and biases of a linear in the arena -> L, used as they are (`quantization`), or
+  // dequantised offline to fp16 (`quantization_config` only).
+  void packed_result(Linear& L, int in, int cbits, int grp, int sdt, const uint32_t* qw, const void* sc, const void* bi) {
+    if (weight_dtype < 0) weight_dtype = sdt;
+    if (packed) {
+      L.bits = cbits; L.group = grp; L.sdt = sdt; L.qw = qw; L.scales = sc; L.biases = bi;
+    } else {
+      // offline `dequantized(..., dtype: .float16)` (Qwen3Talker.swift:156-164) with the bit-exact kernel
+      Q3_CHECK(offline_dequant, Q3TTS_ERR_BAD_CONFIG, "packed weights found but config.json has neither `quantization` nor `quantization_config`");
+      __half* dense = (__half*)arena.alloc((size_t)L.out * in * 2);
+      LaunchCtx lc{stream, nullptr};
+      launch_dequantize(lc, qw, sc, bi, sdt, L.out, in, grp, cbits, Q3TTS_F16, dense);
+      L.bits = 0; L.sdt = Q3TTS_F16; L.w = dense;
+      weight_dtype = Q3TTS_F16;  // what the handle computes with after the load (q3tts_info.weight_dtype)
+    }
+  }
+
   // One or several reference leaves concatenated along `out` (q|k|v, gate|up).
   Linear linear(const std::vector<std::string>& prefixes, int in, const std::vector<int>& outs, bool with_bias) {
     Linear L;
@@ -192,7 +218,46 @@ struct Loader {
     for (int o : outs) L.out += o;
     const STensor& w0 = get(prefixes[0] + ".weight");
     const bool is_packed = (w0.dtype == "U32" || w0.dtype == "I32") && has(prefixes[0] + ".scales");
-    if (is_packed) {
+    if (is_packed && mxfp4) {
+      // .weight [out, in / 8] uint32 + .scales [out, in / 32] uint8, no .biases; the raw leaves go into temporaries and are converted
+      // into the arena.  Every scale byte is checked here, so a leaf the container cannot hold fails q3tts_create.
+      Q3_CHECK(in % 32 == 0, Q3TTS_ERR_BAD_WEIGHTS, "mxfp4 leaf '%s': in_features %d is not a multiple of 32", prefixes[0].c_str(), in);
+      ckpt_bits = 4;
+      const size_t row_words = (size_t)in / 8, row_groups = (size_t)in / 32;
+      uint32_t* qw = (uint32_t*)arena.alloc((size_t)L.out * in);
+      uint16_t* sc = (uint16_t*)arena.alloc((size_t)L.out * row_groups * 2);
+      uint16_t* bi = (uint16_t*)arena.alloc((size_t)L.out * row_groups * 2);
+      std::unique_ptr<void, cudaError_t (*)(void*)> raw_w(nullptr, cudaFree), raw_s(nullptr, cudaFree);
+      void *pw = nullptr, *ps = nullptr;
+      Q3_CUDA(cudaMalloc(&pw, (size_t)L.out * row_words * 4));
+      raw_w.reset(pw);
+      Q3_CUDA(cudaMalloc(&ps, (size_t)L.out * row_groups));
+      raw_s.reset(ps);
+      size_t r0 = 0;
+      for (size_t i = 0; i < prefixes.size(); ++i) {
+        const char* name = prefixes[i].c_str();
+        const STensor& w = get(prefixes[i] + ".weight");
+        const STensor& s = get(prefixes[i] + ".scales");
+        Q3_CHECK(!has(prefixes[i] + ".biases"), Q3TTS_ERR_BAD_WEIGHTS, "mxfp4 leaf '%s' has a .biases tensor (an affine leaf?)", name);
+        const size_t wbytes = (size_t)outs[i] * row_words * 4, sbytes = (size_t)outs[i] * row_groups;
+        Q3_CHECK((w.dtype == "U32" || w.dtype == "I32") && w.shape.size() == 2 && w.shape[0] == outs[i] && (size_t)w.shape[1] == row_words &&
+                     w.nbytes == wbytes,
+                 Q3TTS_ERR_BAD_WEIGHTS, "mxfp4 weight '%s' must be uint32 [%d, %zu]", name, outs[i], row_words);
+        Q3_CHECK(s.dtype == "U8" && s.shape.size() == 2 && s.shape[0] == outs[i] && (size_t)s.shape[1] == row_groups && s.nbytes == sbytes,
+                 Q3TTS_ERR_BAD_WEIGHTS, "mxfp4 scales of '%s' must be uint8 [%d, %zu]", name, outs[i], row_groups);
+        for (size_t k = 0; k < sbytes; ++k)
+          Q3_CHECK(s.data[k] <= kMxfp4MaxScaleByte, Q3TTS_ERR_BAD_WEIGHTS,
+                   "mxfp4 leaf '%s': scale byte %d at index %zu (2^%d) is beyond the 8-bit affine container (bytes 0..%d)", name, (int)s.data[k], k,
+                   (int)s.data[k] - 127, kMxfp4MaxScaleByte);
+        Q3_CUDA(cudaMemcpyAsync((uint32_t*)pw + r0 * row_words, w.data, wbytes, cudaMemcpyHostToDevice, stream));
+        Q3_CUDA(cudaMemcpyAsync((uint8_t*)ps + r0 * row_groups, s.data, sbytes, cudaMemcpyHostToDevice, stream));
+        r0 += outs[i];
+      }
+      LaunchCtx lc{stream, nullptr};
+      launch_mxfp4_to_affine(lc, (const uint32_t*)pw, (const uint8_t*)ps, L.out, in, qw, sc, bi);
+      Q3_CUDA(cudaStreamSynchronize(stream));  // the temporaries are freed when they leave scope
+      packed_result(L, in, 8, 32, Q3TTS_BF16, qw, sc, bi);
+    } else if (is_packed) {
       const int cbits = container_bits(bits);
       Q3_CHECK(cbits != 0, Q3TTS_ERR_BAD_CONFIG, "packed weights with bits=%d: MLX affine checkpoints of 2, 3, 4, 5, 6 or 8 bits are supported", bits);
       const bool widen = cbits != bits;  // 2/3/5/6-bit rows are re-laid into the 4/8-bit words every kernel reads
@@ -244,18 +309,7 @@ struct Loader {
         launch_widen_bits(lc, raw, L.out, in, bits, qw);
         Q3_CUDA(cudaStreamSynchronize(stream));  // raw_tmp is freed when it leaves scope
       }
-      if (weight_dtype < 0) weight_dtype = sdt;
-      if (packed) {
-        L.bits = cbits; L.group = group; L.sdt = sdt; L.qw = qw; L.scales = sc; L.biases = bi;
-      } else {
-        // offline `dequantized(..., dtype: .float16)` (Qwen3Talker.swift:156-164) with the bit-exact kernel
-        Q3_CHECK(offline_dequant, Q3TTS_ERR_BAD_CONFIG, "packed weights found but config.json has neither `quantization` nor `quantization_config`");
-        __half* dense = (__half*)arena.alloc((size_t)L.out * in * 2);
-        LaunchCtx lc{stream, nullptr};
-        launch_dequantize(lc, qw, sc, bi, sdt, L.out, in, group, cbits, Q3TTS_F16, dense);
-        L.bits = 0; L.sdt = Q3TTS_F16; L.w = dense;
-        weight_dtype = Q3TTS_F16;  // what the handle computes with after the load (q3tts_info.weight_dtype)
-      }
+      packed_result(L, in, cbits, group, sdt, qw, sc, bi);
     } else {
       const int sdt = w0.q3_dtype();
       const size_t esz = dtype_size(sdt);
@@ -341,11 +395,11 @@ void load_talker_weights(const std::string& model_dir, const TalkerConfig& cfg, 
   // quantizationSettings prefers quantization_config over quantization (Qwen3Config.swift:275-280);
   // pre-quantised use of the packed leaves requires `quantization` (Qwen3Talker.swift:139)
   const bool packed = cfg.has_quantization;
-  int bits = 0, group = 64;
-  if (cfg.has_quantization_config && cfg.qc_bits) { bits = cfg.qc_bits; group = cfg.qc_group; }
-  else if (cfg.has_quantization && cfg.q_bits) { bits = cfg.q_bits; group = cfg.q_group; }
+  int bits = 0, group = 64, mode = QMODE_AFFINE;
+  if (cfg.has_quantization_config && cfg.qc_bits) { bits = cfg.qc_bits; group = cfg.qc_group; mode = cfg.qc_mode; }
+  else if (cfg.has_quantization && cfg.q_bits) { bits = cfg.q_bits; group = cfg.q_group; mode = cfg.q_mode; }
   else if (!packed) { bits = 8; group = 64; }  // defaults of the offline path (:142-143)
-  Loader L{t, arena, stream, packed, !packed, bits, group};
+  Loader L{t, arena, stream, packed, !packed, bits, group, mode == QMODE_MXFP4};
   L.runtime_quant = runtime_quantization && !cfg.has_quantization;  // `modelConfig.quantization == nil && applyRuntimeQuantization` (:184)
 
   out.talker.hidden = cfg.hidden_size; out.talker.layers = cfg.num_hidden_layers; out.talker.heads = cfg.num_attention_heads;
@@ -375,6 +429,7 @@ void load_talker_weights(const std::string& model_dir, const TalkerConfig& cfg, 
   out.talker_step_bytes = stack_bytes(out.talker) + out.codec_head.weight_bytes();
   out.cp_pass_bytes = stack_bytes(out.cp) + out.lm_head[0].weight_bytes() + (out.has_mtp ? out.small_to_mtp.weight_bytes() : 0);
   out.checkpoint_bits = L.ckpt_bits;
+  out.checkpoint_mode = L.ckpt_bits && L.mxfp4 ? QMODE_MXFP4 : QMODE_AFFINE;
   weight_dtype = L.weight_dtype < 0 ? Q3TTS_BF16 : L.weight_dtype;
   eff_bits = out.talker.layer[0].qkv.bits;
   eff_group = group;

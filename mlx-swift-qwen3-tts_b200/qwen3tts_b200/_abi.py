@@ -36,7 +36,7 @@ class Info(C.Structure):
                                    "num_speakers", "has_codec", "codec_num_quantizers", "codec_total_upsample", "model_type",
                                    "codec_eos_id", "codec_pad_id", "max_batch", "kv_capacity", "max_frames")] + \
                [("device_bytes", i64), ("has_audio_encoder", i32), ("audio_encoder_hidden", i32), ("has_speaker_encoder", i32), ("speaker_embedding_dim", i32),
-                ("checkpoint_quant_bits", i32), ("reserved", i32 * 3)]
+                ("checkpoint_quant_bits", i32), ("checkpoint_quant_mode", i32), ("reserved", i32 * 2)]
 
 
 class Request(C.Structure):
@@ -80,6 +80,7 @@ SYMBOLS = {
     "q3tts_generate_pcm_batch": (i32, [C.c_void_p, C.POINTER(Request), i32, i32, C.POINTER(p_f32), i64, C.POINTER(i64), p_i32]),
     "q3tts_mlx_quantize": (i32, [i32, C.c_void_p, i32, i32, i32, i32, C.c_void_p, C.c_void_p, C.c_void_p]),
     "q3tts_dequantize": (i32, [i32, C.c_void_p, C.c_void_p, C.c_void_p, i32, i32, i32, i32, i32, i32, C.c_void_p]),
+    "q3tts_mxfp4_to_affine": (i32, [i32, C.c_void_p, C.c_void_p, i32, i32, C.c_void_p, C.c_void_p, C.c_void_p]),
     "q3tts_quantized_matmul": (i32, [i32, p_f32, i32, C.c_void_p, C.c_void_p, C.c_void_p, i32, i32, i32, i32, i32, p_f32]),
     "q3tts_quantized_matmul_tc": (i32, [i32, p_f32, i32, C.c_void_p, C.c_void_p, C.c_void_p, i32, i32, i32, i32, i32, p_f32, i32, p_f32, p_f32]),
     "q3tts_conv_probe": (i32, [i32, p_f32, i32, i32, i32, p_f32, p_f32, i32, i32, i32, i32, i32, p_f32, p_f32, p_f32, p_f32, i32, i32, p_f32, p_f32]),

@@ -442,6 +442,22 @@ def mlx_quantize(w, bits=4, dtype="bf16", device=0):
     return codes, s, b
 
 
+def mxfp4_to_affine(packed, scales, device=0):
+    """`q3tts_mxfp4_to_affine` probe: MLX mxfp4 leaves (packed uint32 [out, in/8], E8M0 scale bytes uint8 [out, in/32]) -> the exact 8-bit
+    affine container the loader keeps: (codes uint32 [out, in/4] in 8-bit words, scales, biases as fp32 numpy holding the bf16 values).
+    `dequantize` / `quantized_matmul` / `quantized_matmul_tc` take them with group_size=32, bits=8, scale_dtype="bf16"."""
+    packed = np.ascontiguousarray(packed, dtype=np.uint32)
+    scales = np.ascontiguousarray(scales, dtype=np.uint8)
+    out_f, words = packed.shape
+    in_f = words * 8
+    codes = np.zeros((out_f, in_f // 4), dtype=np.uint32)
+    s = np.zeros((out_f, in_f // 32), dtype=np.uint16)
+    b = np.zeros_like(s)
+    A.check(A.lib().q3tts_mxfp4_to_affine(device, packed.ctypes.data, scales.ctypes.data, out_f, in_f, codes.ctypes.data, s.ctypes.data,
+                                          b.ctypes.data), None)
+    return codes, (s.astype(np.uint32) << 16).view(np.float32), (b.astype(np.uint32) << 16).view(np.float32)
+
+
 def quantized_matmul(x, packed, scales, biases, group_size=64, bits=4, scale_dtype="bf16", device=0) -> np.ndarray:
     """`q3tts_quantized_matmul` probe: y = x @ dequant(W)^T with the talker's GEMV kernels.  bits=0: `packed` is a dense
     fp32-valued weight matrix stored as `scale_dtype`."""

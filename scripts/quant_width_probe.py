@@ -1,11 +1,12 @@
-"""Cost of the 4/8-bit container for 0.6B MLX checkpoints of 3, 4, 5, 6 and 8 bits (group 64).
+"""Cost of the 4/8-bit container for 0.6B MLX checkpoints of 3, 4, 5, 6 and 8 bits (group 64) and for an mxfp4 checkpoint (held as 8-bit
+affine groups of 32 with bf16 scales and biases).
 
 For each width: handle load time, batch-1 ms per frame on the persistent frame kernel (device time of >= 100 teacher-forced frames, prefill
 excluded), ms per frame step of a 64-row handle, and q3tts_timing.weight_bytes_per_frame (container bytes).  2/3-bit checkpoints stream 4-bit
 words and 5/6-bit ones 8-bit words, so the expectation is 3 == 4 and 5 == 6 == 8 at batch 1 within run-to-run spread, and all widths equal
 at 64 rows (the batched step reads the same fp16 copies).  Each width is measured `--reps` times, alternating widths inside a repetition.
 
-    python scripts/quant_width_probe.py [--out results.json] [--bits 3 4 5 6 8] [--reps 3]
+    python scripts/quant_width_probe.py [--out results.json] [--bits 3 4 5 6 8 mxfp4] [--reps 3]
 Needs a B200; the checkpoints go to a temporary directory."""
 import argparse
 import json
@@ -21,6 +22,7 @@ sys.path[:0] = [ROOT, os.path.join(ROOT, "mlx-swift-qwen3-tts_b200"), os.path.jo
 import numpy as np  # noqa: E402
 
 import qwen3tts_b200 as q  # noqa: E402
+import mlx_mxfp4  # noqa: E402
 import mlx_widths  # noqa: E402
 from oracle import checkpoint  # noqa: E402
 
@@ -55,7 +57,7 @@ def step_ms(eng, reqs, frames, batch):
 
 def main():
     ap = argparse.ArgumentParser()
-    ap.add_argument("--bits", type=int, nargs="+", default=[3, 4, 5, 6, 8])
+    ap.add_argument("--bits", nargs="+", default=["3", "4", "5", "6", "8"], help="widths, or mxfp4")
     ap.add_argument("--reps", type=int, default=3)
     ap.add_argument("--out", default=None)
     a = ap.parse_args()
@@ -66,10 +68,12 @@ def main():
         dirs = {}
         for b in a.bits:
             t0 = time.time()
-            if b in (4, 8):
-                dirs[b] = checkpoint.write_checkpoint(os.path.join(tmp, f"b{b}"), "0.6b", bits=b, with_codec=False)
+            if b in ("4", "8"):
+                dirs[b] = checkpoint.write_checkpoint(os.path.join(tmp, f"b{b}"), "0.6b", bits=int(b), with_codec=False)
+            elif b == "mxfp4":  # E2M1 leaves with E8M0 group scales (tests/mlx_mxfp4.py)
+                dirs[b] = mlx_mxfp4.write_mxfp4_checkpoint(os.path.join(tmp, b), "0.6b")[0]
             else:  # 2/3/5/6-bit leaves in MLX's bit-stream layout (tests/mlx_widths.py)
-                dirs[b] = mlx_widths.write_width_checkpoint(os.path.join(tmp, f"b{b}"), "0.6b", bits=b, group=64)[0]
+                dirs[b] = mlx_widths.write_width_checkpoint(os.path.join(tmp, f"b{b}"), "0.6b", bits=int(b), group=64)[0]
             print(f"{b}-bit checkpoint written in {time.time() - t0:.0f} s", flush=True)
         r1, r64 = requests(1, FRAMES_B1, 1), requests(ROWS, FRAMES_B64, 2)
         for rep in range(a.reps):
@@ -83,6 +87,7 @@ def main():
                 res[b]["b1_ms_per_frame"].append(ms)
                 res[b]["weight_bytes_per_frame"] = int(t.weight_bytes_per_frame)
                 res[b]["quant_bits"], res[b]["checkpoint_quant_bits"] = e1.info.quant_bits, e1.info.checkpoint_quant_bits
+                res[b]["quant_group_size"], res[b]["checkpoint_quant_mode"] = e1.info.quant_group_size, e1.info.checkpoint_quant_mode
                 e1.close()
                 e64 = q.Engine(dirs[b], max_batch=ROWS, max_frames=FRAMES_B64 + 8, load_codec=False)
                 step_ms(e64, r64, FRAMES_B64, True)
@@ -92,7 +97,7 @@ def main():
                 e64.close()
                 print(json.dumps({"rep": rep, "bits": b, "load_s": round(res[b]["load_s"][-1], 2), "b1_ms_per_frame": round(ms, 4),
                                   "b64_ms_per_step": round(ms64, 4)}), flush=True)
-    summary = {"card": card, "model": "0.6b g64 bf16 scales", "frames_b1": FRAMES_B1, "rows_b64": ROWS, "results": {}}
+    summary = {"card": card, "model": "0.6b bf16 scales, g64 (mxfp4: g32)", "frames_b1": FRAMES_B1, "rows_b64": ROWS, "results": {}}
     for b in a.bits:
         r = res[b]
         summary["results"][b] = {k: (round(float(np.median(v)), 4) if isinstance(v, list) else v) for k, v in r.items()}
